@@ -55,7 +55,13 @@ def parse():
     ap.add_argument("--no-sustained", action="store_true")
     ap.add_argument("--step-series", type=int, default=0, help="diagnostic: print the device time of each of N steps")
     ap.add_argument("--burst-ab", action="store_true", help="diagnostic: the timed burst under several launch-queue depths")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float32 / float64, at "
+                         "most 64 MB in all), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the outputs of --impl b200")
+    return args
 
 
 class Ctx:
@@ -125,6 +131,49 @@ class Ctx:
     def close(self):
         if self.world > 1 and self.dev is not None:
             torch.distributed.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def snapshot(arrays):
+    """Host copies of the named device tensors, taken right after a timed region (later regions keep training the same
+    table).  Floating-point tensors keep float64 or become float32, integer ones become float64 (exact).  A tensor
+    larger than its share of DUMP_BYTES is cut to a sample of its flattened elements: the positions are drawn with a
+    fixed seed from its size alone, so two runs with the same arguments sample the same elements."""
+    share = (DUMP_BYTES - 4096 * len(arrays)) // len(arrays)   # 4 KB per file for the .npy header
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        dt = torch.float64 if (t.dtype == torch.float64 or not t.is_floating_point()) else torch.float32
+        k = share // dt.itemsize
+        if t.numel() > k:
+            pos = np.sort(np.random.default_rng(0).choice(t.numel(), size=k, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(pos).to(t.device)]
+        out[name] = t.to(dt).cpu().numpy()
+    return out
+
+
+def restarter(eng, initial, moments):
+    """With --dump-outputs the last timed step starts from the seeded initial state: the step sums its gradients with
+    float atomics in no fixed order, and over many steps the hinge thresholds turn those last-bit differences into
+    different trajectories, so only a step from a fixed state computes the same outputs in every run.  Returns the
+    reset: each (parameter, initial device copy) pair is copied back, optimizer moments and step count restart, and the
+    engine re-derives its rows from the table (one copy and one extra launch inside the timed region)."""
+    def restart():
+        for dst, src in initial:
+            dst.copy_(src, non_blocking=True)
+        for m in moments:
+            m.zero_()
+        eng.opt_step = 0
+        eng.invalidate_rows()
+    return restart
+
+
+def write_dump(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def hbm_peak():
@@ -323,7 +372,7 @@ def run_label_reference(args, ctx, wl):
             "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
 
 
-def run_label(args, ctx, wl, steps, warmup, headline=False):
+def run_label(args, ctx, wl, steps, warmup, headline=False, dump=None):
     from learning_embeddings_b200 import _native
     from learning_embeddings_b200.engine import ConeStep, index_dtype_for, pack_index_block
     from learning_embeddings_b200 import sharding
@@ -367,6 +416,10 @@ def run_label(args, ctx, wl, steps, warmup, headline=False):
     sampler.start()
     kev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     ctx.warm(dev_step, eng, kev, warmup)
+    restart = None
+    if args.dump_outputs:
+        restart = restarter(eng, [(table, table0.to(dev))], [m for m in (eng.opt_m, eng.opt_v) if m is not None])
+        cfg["dump_outputs"] = "the last timed step starts from the seeded initial table"
 
     # timed region: inputs resident in HBM
     launches0 = _native.launch_count()
@@ -381,6 +434,8 @@ def run_label(args, ctx, wl, steps, warmup, headline=False):
         # the pair kernel is bracketed by CUDA events on every 4th step only: two event records per step sit between
         # back-to-back launches and cost more than they measure
         eng.kernel_events = kev[i] if i % 4 == 0 else None
+        if restart is not None and i == steps - 1:
+            restart()
         dev_step(i)
     t1.record()
     ctx.sync_all()
@@ -389,7 +444,11 @@ def run_label(args, ctx, wl, steps, warmup, headline=False):
     lec_launches = _native.launch_count() - launches0
     elapsed_ms = ctx.max_ranks(t0.elapsed_time(t1))
     kernel_ms = float(np.mean([a.elapsed_time(b) for i, (a, b) in enumerate(kev) if i % 4 == 0]))
-    final_loss = float(eng.global_loss().item())
+    last_loss = eng.global_loss()
+    final_loss = float(last_loss.item())
+    if dump is not None:
+        # the step's loss, the table it updated in place, and the pair energies of this rank's share of the batch
+        dump.update(snapshot({"loss": last_loss, "table": table, "E_pos": eng.E_pos[:groups], "E_neg": eng.E_neg[:groups]}))
     value = world * pairs_per_step * steps / (elapsed_ms * 1e-3)
     clocks = sampler.summary()
 
@@ -714,6 +773,7 @@ def cfg2_setup(ctx):
     idx_dt = index_dtype_for(h.n + c["m"])
     g = torch.Generator().manual_seed(0)
     table0 = torch.randn(h.n, c["D"], generator=g)
+    torch.manual_seed(0)   # fc1's default init draws from the global generator: the same weights in every run
     lin = torch.nn.Linear(c["F"], c["D"])
     with torch.no_grad():
         fw0, fb0 = lin.weight.detach().clone(), lin.bias.detach().clone()
@@ -756,7 +816,7 @@ def run_cfg2_reference(args, ctx):
             "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
 
 
-def run_cfg2(args, ctx, steps, warmup):
+def run_cfg2(args, ctx, steps, warmup, dump=None):
     from learning_embeddings_b200 import _native
     from learning_embeddings_b200.engine import JointConeStep
     c, h, idx_dt, g, table0, fw0, fb0, rng, leaf_of_img = cfg2_setup(ctx)
@@ -794,6 +854,11 @@ def run_cfg2(args, ctx, steps, warmup):
     sampler.start()
     kev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     ctx.warm(dev_step, eng, kev, warmup)
+    restart = None
+    if args.dump_outputs:
+        restart = restarter(eng, [(table, table0.to(dev)), (eng.fc_w, fw0.to(dev)), (eng.fc_b, fb0.to(dev))],
+                            list(eng.opt.values()) + list(eng.opt_fc.values()))
+        cfg["dump_outputs"] = "the last timed step starts from the seeded initial table and fc1"
     launches0 = _native.launch_count()
     t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     sampler.active.set()
@@ -804,6 +869,8 @@ def run_cfg2(args, ctx, steps, warmup):
     t0.record()
     for i in range(steps):
         eng.kernel_events = kev[i] if i % 4 == 0 else None
+        if restart is not None and i == steps - 1:
+            restart()
         dev_step(i)
     t1.record()
     ctx.sync_all()
@@ -814,6 +881,9 @@ def run_cfg2(args, ctx, steps, warmup):
     kernel_ms = float(np.mean([a.elapsed_time(b) for i, (a, b) in enumerate(kev) if i % 4 == 0]))
     value = world * pairs_per_step * steps / (elapsed_ms * 1e-3)
     clocks = sampler.summary()
+    if dump is not None:
+        dump.update(snapshot({"loss": eng.loss_global, "table": table, "fc_weight": eng.fc_w, "fc_bias": eng.fc_b,
+                              "E_pos": eng.E_pos[:B], "E_neg": eng.E_neg[:B]}))
     e2e = None
     if not args.no_e2e:
         for i in range(3):
@@ -933,7 +1003,7 @@ def run_cfg3_reference(args, ctx):
             "e2e": {"value": v, "unit": "scores/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
 
 
-def run_cfg3(args, ctx, steps, warmup, dim=None, modes=None, with_e2e=True, with_cpu=True):
+def run_cfg3(args, ctx, steps, warmup, dim=None, modes=None, with_e2e=True, with_cpu=True, dump=None):
     """Returns one record per score mode in `modes` (default: the one --score-mode names), sharing inputs."""
     import ctypes
     from learning_embeddings_b200 import _native, ops
@@ -1021,6 +1091,9 @@ def run_cfg3(args, ctx, steps, warmup, dim=None, modes=None, with_e2e=True, with
         kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in kev]))
         value = world * n_img * L * steps / (elapsed_ms * 1e-3)
         clocks = sampler.summary()
+        if dump is not None:
+            got = {"topk_index": idx, "topk_energy": val, "energy": scores}
+            dump.update(snapshot({name: t for name, t in got.items() if t is not None}))
 
         # end to end: pinned host images -> H2D -> per-level top-5 -> predictions D2H, through ops.ScorePipeline, which
         # cuts the image set into slices and overlaps the copies of neighbouring slices with the kernel (what the
@@ -1108,20 +1181,21 @@ def main():
             print(json.dumps(rec))
         return
     ctx = Ctx(need_gpu=True)
+    dump = {} if args.dump_outputs and ctx.rank == 0 else None   # outputs of the headline workload's timed path
     try:
         if args.workload in ("cfg0", "cfg1", "cfg4"):
-            rec = run_label(args, ctx, args.workload, args.steps, args.warmup, headline=True)
+            rec = run_label(args, ctx, args.workload, args.steps, args.warmup, headline=True, dump=dump)
         elif args.workload == "cfg2":
-            rec = run_cfg2(args, ctx, args.steps, args.warmup)
+            rec = run_cfg2(args, ctx, args.steps, args.warmup, dump=dump)
         elif args.workload == "cfg3":
-            recs = run_cfg3(args, ctx, args.steps, args.warmup)
+            recs = run_cfg3(args, ctx, args.steps, args.warmup, dump=dump)
             rec = recs[args.score_mode] if recs is not None else None
         else:
-            rec = run_label(args, ctx, "cfg1", args.steps, args.warmup, headline=True)
+            rec = run_label(args, ctx, "cfg1", args.steps, args.warmup, headline=True, dump=dump)
             s_steps, s_warm = max(3, min(args.steps, 20)), max(3, min(args.warmup, 5))
             subs = {}
             sub_args = argparse.Namespace(**vars(args))
-            sub_args.pairs, sub_args.rotation = 0, 0
+            sub_args.pairs, sub_args.rotation, sub_args.dump_outputs = 0, 0, None
             subs["cfg0"] = guarded("cfg0", lambda: run_label(sub_args, ctx, "cfg0", s_steps, s_warm), ctx)
             subs["cfg2"] = guarded("cfg2", lambda: run_cfg2(sub_args, ctx, s_steps, s_warm), ctx)
             for D, modes in ((10, ["matrix", "topk", "both"]), (50, ["matrix", "both"])):
@@ -1136,6 +1210,8 @@ def main():
                 rec["workloads"] = subs
         if rec is not None:
             print(json.dumps(rec))
+        if dump is not None:
+            write_dump(args.dump_outputs, dump)
     finally:
         ctx.close()
 
