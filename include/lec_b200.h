@@ -426,6 +426,37 @@ int64_t lec_f1_workspace_bytes(void);
 int lec_f1_sweep(const float* sorted_energies, const int64_t* pos_prefix, int64_t n, int64_t n_pos, int64_t n_neg,
                  double* out7, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* Reconstruction check without the energies: lec_recon_* replaces check_graph_embedding (order_embeddings.py:512-559 =
+ * oe.py:1923-1990) at any size.  Positives are E(x = rows[u], y = rows[v]) for every v that is a strict descendant of
+ * u (tin[u] < tin[v] <= tout[u], the Euler-tour intervals of the forest), negatives every other ordered pair u != v; the
+ * result is the row lec_f1_sweep returns for those energies, bit for bit, where the energies are the ones
+ * lec_score_topk_ex(..., LEC_PREC_F32, ...) computes for labels = images = rows.  Energies are histogrammed, never
+ * stored: round 0 counts every pair into coarse bins, later rounds recount the pairs of the bins that can hold the
+ * best threshold by exact value.
+ *   rows           device [n, ld] fp32, 16-byte aligned; ld == D or ld % 4 == 0 (the padded rows of lec_rows_fwd)
+ *   D              1..64 (what the SIMT scoring kernel supports)
+ *   tin, tout      device int32[n]
+ *   u_begin/u_end  the apex rows this call evaluates (a rank's share, [0, n) on one GPU); v always spans [0, n)
+ *   workspace      device, 16-byte aligned, >= lec_recon_workspace_bytes(1) bytes, zeroed by the caller once before
+ *                  round 0.  Its first lec_recon_counter_bytes(workspace_bytes) bytes are the counters a pass adds to;
+ *                  ranks that split [0, n) sum that span (all_reduce) after every pass and before lec_recon_finish.
+ * A round is lec_recon_pass then lec_recon_finish, which evaluates the round, clears the counters and writes
+ *   out7           device double[7]: the best row found so far (final once status[0] == 0)
+ *   status         device int64[4]: {1 if another round is needed else 0, coarse bins opened after round 0, n_pos, n_neg}
+ * Neither call allocates or synchronises; the round lives in the workspace.  lec_recon_workspace_bytes returns the
+ * size for a given number of coarse bins counted per fine round (about 1 MB each); more open bins take more rounds. */
+typedef struct lec_recon {
+    int geom; float K;
+    const float* rows; int64_t n; int D; int ld;
+    const int32_t* tin; const int32_t* tout;
+    int64_t u_begin, u_end;
+    void* workspace; int64_t workspace_bytes;
+} lec_recon_t;
+int64_t lec_recon_workspace_bytes(int open_bins_per_round);
+int64_t lec_recon_counter_bytes(int64_t workspace_bytes);
+int lec_recon_pass(const lec_recon_t* r, void* stream);
+int lec_recon_finish(const lec_recon_t* r, double* out7, int64_t* status, void* stream);
+
 /* lec_classify_counts replaces the per-image bookkeeping of JointEmbeddings.calculate_classification_metrics
  * (oe.py:1775-1796, oe_h.py:2030-2051) on the output of lec_score_topk*.
  *   topk_idx  device int32 [n_img, n_levels, k]   truth  device int32 [n_img, n_levels] (true label per level, < 0: skip)

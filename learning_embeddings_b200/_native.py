@@ -25,6 +25,7 @@ EXPORTS = (
     "lec_score_workspace_bytes", "lec_score_topk_tc", "lec_mt_seed", "lec_mt_uint32", "lec_mt_randbelow",
     "lec_sample_negatives", "lec_sample_negatives_philox", "lec_philox_below", "lec_f1_workspace_bytes", "lec_f1_sweep",
     "lec_classify_counts", "lec_caption_hinge",
+    "lec_recon_workspace_bytes", "lec_recon_counter_bytes", "lec_recon_pass", "lec_recon_finish",
     "lec_host_pipe_create", "lec_host_pipe_destroy", "lec_host_pipe_submit", "lec_host_pipe_wait",
 )
 
@@ -77,6 +78,17 @@ class LecStep(ctypes.Structure):
 class LecHostSample(ctypes.Structure):
     """lec_host_sample_t of include/lec_b200.h."""
     _fields_ = [("graph", ctypes.c_void_p), ("seed", ctypes.c_uint64), ("stream_id", ctypes.c_uint64), ("status", ctypes.c_void_p)]
+
+
+class LecRecon(ctypes.Structure):
+    """lec_recon_t of include/lec_b200.h."""
+    _fields_ = [
+        ("geom", ctypes.c_int), ("K", ctypes.c_float),
+        ("rows", ctypes.c_void_p), ("n", ctypes.c_int64), ("D", ctypes.c_int), ("ld", ctypes.c_int),
+        ("tin", ctypes.c_void_p), ("tout", ctypes.c_void_p),
+        ("u_begin", ctypes.c_int64), ("u_end", ctypes.c_int64),
+        ("workspace", ctypes.c_void_p), ("workspace_bytes", ctypes.c_int64),
+    ]
 
 
 UPD_NONE, UPD_RSGD, UPD_SGD, UPD_ADAM = 0, 1, 2, 3
@@ -146,6 +158,12 @@ def lib():
         L.lec_f1_workspace_bytes.restype = c_i64
         L.lec_f1_sweep.argtypes = [c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_i64, c_vp]
         L.lec_classify_counts.argtypes = [c_vp, c_vp, c_i64, c_i, c_i, c_vp, c_i, c_i64, c_vp, c_vp, c_vp, c_vp]
+        L.lec_recon_workspace_bytes.argtypes = [c_i]
+        L.lec_recon_workspace_bytes.restype = c_i64
+        L.lec_recon_counter_bytes.argtypes = [c_i64]
+        L.lec_recon_counter_bytes.restype = c_i64
+        L.lec_recon_pass.argtypes = [ctypes.POINTER(LecRecon), c_vp]
+        L.lec_recon_finish.argtypes = [ctypes.POINTER(LecRecon), c_vp, c_vp, c_vp]
         L.lec_caption_hinge.argtypes = [c_vp, c_vp, c_i64, c_i, c_f, c_vp, c_vp, c_vp, c_vp, c_vp]
         L.lec_host_pipe_create.argtypes = [ctypes.POINTER(c_vp), c_i]
         L.lec_host_pipe_destroy.argtypes = [c_vp]

@@ -19,6 +19,7 @@
 #include <atomic>
 
 #include "../../include/lec_b200.h"
+#include "lec_f1.cuh"
 
 namespace lec {
 extern std::atomic<unsigned long long> g_launches;  // lec_api.cu
@@ -29,11 +30,6 @@ constexpr int kF1Blocks = 592;   // 4 x 148
 constexpr int kF1Threads = 256;
 
 struct F1Best { double f1; int64_t idx; };
-
-__device__ __forceinline__ bool f1_better(double fa, int64_t ia, double fb, int64_t ib) {
-    // higher F1 wins; ties go to the lower threshold (np.argmax returns the first maximum)
-    return fa > fb || (fa == fb && ia < ib);
-}
 
 // number of non-NaN energies: the sort puts NaNs last, so "is NaN" is monotone over the array
 __device__ __forceinline__ int64_t first_nan(const float* sorted, int64_t n) {
@@ -46,24 +42,18 @@ __device__ __forceinline__ int64_t first_nan(const float* sorted, int64_t n) {
     return lo;
 }
 
-// metrics of threshold sorted[i] (a run end): the reference's expression tree in fp64.  NaN energies (the zero label
-// row of the reference's off-by-one, SURVEY F9) satisfy neither E <= t nor E > t: they count in n_pos / n_neg only.
-__device__ __forceinline__ void f1_row(const float* sorted, const int64_t* pos_prefix, int64_t i, int64_t n_pos, int64_t n_neg,
-                                       int64_t n_fin, double* row) {
+// metrics of threshold sorted[i] (a run end): counts from the positive prefix, then lec_f1.cuh's expression tree
+__device__ __forceinline__ void sorted_f1_row(const float* sorted, const int64_t* pos_prefix, int64_t i, int64_t n_pos,
+                                              int64_t n_neg, int64_t n_fin, double* row) {
     const float t = sorted[i];
-    int64_t cp, cn;
-    if (t != t) { cp = 0; cn = 0; }   // NaN threshold: no comparison holds
-    else {
+    int64_t cp = 0, cn = 0;   // NaN threshold: no comparison holds
+    if (t == t) {
         cp = pos_prefix[i];                                              // positives with E <= t
         const int64_t pos_fin = n_fin > 0 ? pos_prefix[n_fin - 1] : 0;   // positives that are not NaN
         const int64_t neg_fin = n_fin - pos_fin;
         cn = neg_fin - ((i + 1) - cp);                                   // negatives with E > t
     }
-    const double acc = (double)(cp + cn) / (double)(n_pos + n_neg);
-    const double prec = (double)cp / (double)(cp + (n_neg - cn));   // 0/0 -> NaN (the reference raises ZeroDivisionError)
-    const double rec = (double)cp / (double)n_pos;
-    const double f1 = (prec + rec == 0.0) ? 0.0 : (2.0 * prec * rec) / (prec + rec);
-    row[0] = f1; row[1] = (double)t; row[2] = acc; row[3] = prec; row[4] = rec; row[5] = (double)cp; row[6] = (double)cn;
+    f1_row(t, cp, cn, n_pos, n_neg, row);
 }
 
 __global__ void __launch_bounds__(kF1Threads) f1_sweep_kernel(const float* __restrict__ sorted, const int64_t* __restrict__ pos_prefix,
@@ -80,7 +70,7 @@ __global__ void __launch_bounds__(kF1Threads) f1_sweep_kernel(const float* __res
         }
         if (!end) continue;
         double row[7];
-        f1_row(sorted, pos_prefix, i, n_pos, n_neg, n_fin, row);
+        sorted_f1_row(sorted, pos_prefix, i, n_pos, n_neg, n_fin, row);
         double f1 = row[0];
         if (f1 != f1) f1 = -1.0;   // NaN never wins
         if (f1_better(f1, i, best.f1, best.idx)) { best.f1 = f1; best.idx = i; }
@@ -118,7 +108,7 @@ __global__ void __launch_bounds__(kF1Threads) f1_final_kernel(const float* __res
     }
     if (threadIdx.x == 0) {
         if (sh[0].idx == INT64_MAX) { for (int j = 0; j < 7; ++j) out7[j] = nan(""); }
-        else f1_row(sorted, pos_prefix, sh[0].idx, n_pos, n_neg, first_nan(sorted, n), out7);
+        else sorted_f1_row(sorted, pos_prefix, sh[0].idx, n_pos, n_neg, first_nan(sorted, n), out7);
     }
 }
 

@@ -51,6 +51,25 @@ struct FastArgs {
     int32_t* topk_idx; float* topk_val;
     int64_t groups;  // image groups of NT*RI images
     int ring;        // candidate ring entries per thread (> RI)
+    // reconstruction pass (EPI = 1, lec_recon.cu): labels = images = rows, row stride ld; a block evaluates the
+    // apex rows [u_begin + c*chunk, ...) of chunk c against its image group
+    int64_t ld, u_begin, u_end, chunk;
+    const int32_t* tin; const int32_t* tout;
+    const struct ReconState* rstate; const struct ReconOpen* ropen;
+    unsigned long long* rhdr; unsigned long long* rhist;
+};
+
+// Reconstruction check (lec_recon.cu).  Key of an energy = its fp32 bit pattern (energies are >= 0 or NaN, -0 is
+// counted as 0); the coarse round histograms key >> kReconShift, a fine round counts every key of the open coarse bins.
+constexpr int kReconShift = 16;
+constexpr int kReconBins = 1 << (31 - kReconShift);  // coarse bins of a non-negative fp32 key (+inf included)
+constexpr int kReconFine = 1 << kReconShift;         // fine bins (one fp32 value each) per coarse bin
+struct ReconOpen { uint32_t bin, pad; unsigned long long cp_below, fp_below; };  // finite energies below the bin
+struct ReconState {
+    int phase, pad;                  // 0 coarse round, 1 fine rounds, 2 done
+    long long n_open, next, m, batch;  // open coarse bins; first one and number of them in this round; bins per round
+    unsigned long long n_pos, n_neg, nan_pos, nan_neg;
+    double best_f1; unsigned long long best_cp, best_cn; unsigned best_key; int has_best;
 };
 
 // Shared-memory layout of one staged label: DQ float4 chunks of the row (zero padded), then one float4
@@ -64,7 +83,8 @@ struct IntC {
     static constexpr int value = V;
 };
 
-template <int GEOM, int DH, int RI, int NT, int MINB>
+// EPI = 1: the reconstruction pass -- the same energies, counted into the lec_recon.cu histograms instead of stored
+template <int GEOM, int DH, int RI, int NT, int MINB, int EPI = 0>
 __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) {
     static_assert(RI % 2 == 0, "images are packed in pairs");
     constexpr int DQ = (DH + 1) / 2;     // float4 chunks per row
@@ -80,7 +100,9 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     const int tid = threadIdx.x;
     const int seg = (int)(blockIdx.x / a.groups);
     const int64_t group = blockIdx.x % a.groups;
-    const int l_begin = a.seg_start[seg], l_end = a.seg_stop[seg], level = a.seg_level[seg];
+    const int l_begin = EPI ? (int)(a.u_begin + (int64_t)seg * a.chunk) : a.seg_start[seg];
+    const int l_end = EPI ? (int)min(a.u_end, a.u_begin + (int64_t)(seg + 1) * a.chunk) : a.seg_stop[seg];
+    const int level = EPI ? -1 : a.seg_level[seg];
     const bool want_topk = (level >= 0) && (a.topk_idx != nullptr);
     const int k = a.k;
     const int D = a.D;
@@ -92,8 +114,8 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
 #pragma unroll
     for (int j = 0; j < NP; ++j) {
         const int64_t i0 = img0 + (2 * j) * NT, i1 = img0 + (2 * j + 1) * NT;
-        const float* s0 = a.images + (i0 < a.N ? i0 : 0) * (int64_t)D;
-        const float* s1 = a.images + (i1 < a.N ? i1 : 0) * (int64_t)D;
+        const float* s0 = a.images + (i0 < a.N ? i0 : 0) * (EPI ? a.ld : (int64_t)D);
+        const float* s1 = a.images + (i1 < a.N ? i1 : 0) * (EPI ? a.ld : (int64_t)D);
         float b0 = 0.f, b1 = 0.f;
 #pragma unroll
         for (int d = 0; d < 4 * DQ; ++d) {
@@ -118,6 +140,59 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         for (int s = 0; s < RI * k; ++s) top[s * NT + tid] = make_float2(INFINITY, __int_as_float(-1));
     }
     const bool full = (group + 1) * (int64_t)(NT * RI) <= a.N;  // block-uniform: every image of the group exists
+
+    // ---- reconstruction pass: coarse round = negatives per coarse bin in shared memory (positives, which are a
+    // fraction of a percent of the pairs, go straight to global memory); fine rounds = the batch slot of every coarse
+    // bin (or -1) in the same shared array.  Zeros, NaNs and the pair counts stay in registers until the block ends.
+    unsigned* rsh = reinterpret_cast<unsigned*>(smem + kTileLabels * LS);
+    int rphase = 0;
+    int tin_v[RI];
+    unsigned c_np = 0, c_nn = 0, c_nanp = 0, c_nann = 0, c_zp = 0, c_zn = 0;
+    if (EPI) {
+        rphase = a.rstate->phase;
+        if (rphase == 2) return;
+#pragma unroll
+        for (int r = 0; r < RI; ++r) {
+            const int64_t v = img0 + r * NT;
+            tin_v[r] = v < a.N ? a.tin[v] : 0;
+        }
+        for (int b = tid; b < kReconBins; b += NT) rsh[b] = rphase == 0 ? 0u : ~0u;
+        if (rphase == 1) {
+            __syncthreads();
+            const long long first = a.rstate->next, m = a.rstate->m;
+            for (long long i = tid; i < m; i += NT) rsh[a.ropen[first + i].bin] = (unsigned)i;
+        }
+        // the tile loop's first barrier orders these stores before any use
+    }
+    // one ordered pair (x = label u, y = image v); valid excludes the diagonal and images past the table
+    auto recon_count = [&](float e, bool valid, bool pos) {
+        const bool fin = e == e;
+        const bool zero = e == 0.f;
+        const unsigned key = __float_as_uint(e);
+        c_zp += valid & pos & zero;
+        c_zn += valid & !pos & zero;
+        if (rphase == 0) {
+            c_np += valid & pos;
+            c_nn += valid & !pos;
+            c_nanp += valid & pos & !fin;
+            c_nann += valid & !pos & !fin;
+            if (valid && fin && !zero) {
+                if (pos) atomicAdd(a.rhist + (key >> kReconShift), 1ull);
+                else atomicAdd(rsh + (key >> kReconShift), 1u);
+            }
+        } else {
+            int tag = -1;  // (slot, low key bits, positive) of a pair inside an open coarse bin
+            if (valid && fin && !zero) {
+                const int s = (int)rsh[key >> kReconShift];
+                if (s >= 0) tag = (((s << kReconShift) | (int)(key & (kReconFine - 1))) << 1) | (int)pos;
+            }
+            // equal tags of a warp are added once: a heavily populated value costs one atomic per warp, not per pair
+            if (__any_sync(0xffffffffu, tag >= 0)) {
+                const unsigned peers = __match_any_sync(0xffffffffu, tag);
+                if (tag >= 0 && (int)(tid & 31) == __ffs(peers) - 1) atomicAdd(a.rhist + tag, (unsigned long long)__popc(peers));
+            }
+        }
+    };
 
     auto merge = [&]() {
         // insert this thread's ring entries into its sorted per-image lists (stable: ties keep the lower label)
@@ -327,7 +402,8 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         }
     };
 
-    // STORE: 0 no matrix, 1 label-major and every image of the group exists, 2 generic strides / partial group
+    // STORE: 0 no matrix, 1 label-major and every image of the group exists, 2 generic strides / partial group,
+    // 3 reconstruction counts
     auto tile_loop = [&](int l0, int tl, auto store_c, auto topk_c) {
         constexpr int STORE = decltype(store_c)::value;
         constexpr bool TOPK = decltype(topk_c)::value != 0;
@@ -349,6 +425,15 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 for (int r = 0; r < RI; ++r) {
                     const int64_t i = img0 + r * NT;
                     if (i < a.N) row[i * a.s_img] = E[r];
+                }
+            } else if (STORE == 3) {
+                const int u = l0 + t;
+                const int* ue = reinterpret_cast<const int*>(lab + t * LS + 4 * DQ + 6);  // Euler interval of u
+                const int tin_u = ue[0], tout_u = ue[1];
+#pragma unroll
+                for (int r = 0; r < RI; ++r) {
+                    const int64_t v = img0 + r * NT;
+                    recon_count(E[r], v < a.N && v != u, tin_u < tin_v[r] && tin_v[r] <= tout_u);
                 }
             }
             if (TOPK) {
@@ -372,12 +457,12 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         // ---- stage the tile: rows zero-padded to whole float4 chunks
         for (int i = tid; i < tl * 4 * DQ; i += NT) {
             const int t = i / (4 * DQ), d = i - t * (4 * DQ);
-            lab[t * LS + d] = (d < D) ? __ldg(a.labels + (int64_t)(l0 + t) * D + d) : 0.f;
+            lab[t * LS + d] = (d < D) ? __ldg(a.labels + (int64_t)(l0 + t) * (EPI ? a.ld : (int64_t)D) + d) : 0.f;
         }
         // ---- per-label constants in fp64 (same terms as lec_rows_fwd's aux)
         if (GEOM != LEC_GEOM_OE) {
             for (int t = tid; t < tl; t += NT) {
-                const float* src = a.labels + (int64_t)(l0 + t) * D;
+                const float* src = a.labels + (int64_t)(l0 + t) * (EPI ? a.ld : (int64_t)D);
                 double A = 0.0;
                 for (int d = 0; d < D; ++d) { const double v = (double)__ldg(src + d); A += v * v; }
                 const Aux<double> x = row_aux<double>(GEOM, A, a.K);
@@ -393,6 +478,13 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 *reinterpret_cast<float4*>(lab + t * LS + 4 * DQ + 4) = c2;
             }
         }
+        if (EPI) {  // the apex's Euler interval in the last two constant slots (after the stores above, same thread)
+            for (int t = tid; t < tl; t += NT) {
+                int* ue = reinterpret_cast<int*>(lab + t * LS + 4 * DQ + 6);
+                ue[0] = a.tin[l0 + t];
+                ue[1] = a.tout[l0 + t];
+            }
+        }
         __syncthreads();
         if (GEOM == LEC_GEOM_HYP && want_topk && store == 0) {
             if (tid < 32) {
@@ -405,7 +497,9 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
             __syncthreads();
             refresh_filter();
         }
-        if (want_topk) {
+        if (EPI) {
+            tile_loop(l0, tl, IntC<3>(), IntC<0>());
+        } else if (want_topk) {
             if (store == 0 && GEOM == LEC_GEOM_HYP) tile_loop_deferred(l0, tl);
             else if (store == 0) tile_loop(l0, tl, IntC<0>(), IntC<1>());
             else if (store == 1) tile_loop(l0, tl, IntC<1>(), IntC<1>());
@@ -414,6 +508,44 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
             if (store == 1) tile_loop(l0, tl, IntC<1>(), IntC<0>());
             else if (store == 2) tile_loop(l0, tl, IntC<2>(), IntC<0>());
         }
+    }
+
+    if (EPI) {
+        // register counters: one global add per warp; then the block's coarse negatives
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            c_np += __shfl_xor_sync(0xffffffffu, c_np, o);
+            c_nn += __shfl_xor_sync(0xffffffffu, c_nn, o);
+            c_nanp += __shfl_xor_sync(0xffffffffu, c_nanp, o);
+            c_nann += __shfl_xor_sync(0xffffffffu, c_nann, o);
+            c_zp += __shfl_xor_sync(0xffffffffu, c_zp, o);
+            c_zn += __shfl_xor_sync(0xffffffffu, c_zn, o);
+        }
+        if ((tid & 31) == 0) {
+            if (rphase == 0) {
+                if (c_np) atomicAdd(a.rhdr + 0, (unsigned long long)c_np);
+                if (c_nn) atomicAdd(a.rhdr + 1, (unsigned long long)c_nn);
+                if (c_nanp) atomicAdd(a.rhdr + 2, (unsigned long long)c_nanp);
+                if (c_nann) atomicAdd(a.rhdr + 3, (unsigned long long)c_nann);
+                if (c_zp) atomicAdd(a.rhist + 0, (unsigned long long)c_zp);
+                if (c_zn) atomicAdd(a.rhist + kReconBins, (unsigned long long)c_zn);
+            } else {
+                const int s0 = (int)rsh[0];  // key 0 is fine bin 0 of coarse bin 0
+                if (s0 >= 0) {
+                    const int64_t z = (int64_t)s0 << (kReconShift + 1);
+                    if (c_zp) atomicAdd(a.rhist + z + 1, (unsigned long long)c_zp);
+                    if (c_zn) atomicAdd(a.rhist + z, (unsigned long long)c_zn);
+                }
+            }
+        }
+        if (rphase == 0) {
+            __syncthreads();
+            for (int b = tid; b < kReconBins; b += NT) {
+                const unsigned c = rsh[b];
+                if (c) atomicAdd(a.rhist + kReconBins + b, (unsigned long long)c);
+            }
+        }
+        return;
     }
 
     if (want_topk) {

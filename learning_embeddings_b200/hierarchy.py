@@ -45,6 +45,34 @@ class Hierarchy:
             else:
                 self.tout[node] = clock - 1
 
+    @classmethod
+    def from_closure_edges(cls, n, edges):
+        """The forest whose transitive closure is `edges`, (ancestor, descendant) pairs -- the reference's G_tc edge
+        list (order_embeddings.py:371).  A node's parent is its ancestor with the most ancestors.  Raises ValueError
+        when the edges are not the closure of a forest on n nodes (a diamond, a cycle, a missing transitive edge)."""
+        e = np.asarray(edges, dtype=np.int64).reshape(-1, 2)
+        if len(e) and (e.min() < 0 or e.max() >= n):
+            raise ValueError("closure edge endpoint outside [0, %d)" % n)
+        if np.any(e[:, 0] == e[:, 1]):
+            raise ValueError("closure edge from a node to itself")
+        if len(e) == 0:
+            return cls(np.full(n, -1, dtype=np.int64))
+        e = np.unique(e, axis=0)
+        n_anc = np.bincount(e[:, 1], minlength=n)
+        o = np.lexsort((n_anc[e[:, 0]], e[:, 1]))          # per descendant, ancestors by their own ancestor count
+        u, v = e[o, 0], e[o, 1]
+        last = np.r_[v[1:] != v[:-1], True]
+        parents = np.full(n, -1, dtype=np.int64)
+        parents[v[last]] = u[last]
+        has = parents >= 0
+        # in a forest the parent has exactly one ancestor fewer; this also rules out cycles
+        if np.any(n_anc[parents[has]] != n_anc[has] - 1):
+            raise ValueError("the edges are not the transitive closure of a forest")
+        h = cls(parents)
+        if not np.array_equal(h.closure_edges(), e):
+            raise ValueError("the edges are not the transitive closure of a forest")
+        return h
+
     def _children(self, node):
         lo, hi = self.children_ptr[node + 1], self.children_ptr[node + 2]
         return self.children_idx[lo:hi]

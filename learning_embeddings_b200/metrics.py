@@ -37,6 +37,82 @@ def best_f1_sweep(e_pos, e_neg):
     return out.cpu().numpy()
 
 
+RECON_OPEN_BINS = 128   # default coarse bins recounted per round of reconstruction_f1 (about 1 MB of workspace each)
+
+
+def recon_args(rows, tin, tout, geom, K, D, u_begin, u_end, workspace):
+    """lec_recon_t for device rows [n, >= D] (fp32, unit column stride), device int32 Euler intervals tin / tout [n]
+    and a device workspace tensor; apex rows [u_begin, u_end)."""
+    r = N.LecRecon()
+    r.geom, r.K = N.GEOM[geom], float(K or 0.0)
+    r.rows, r.n, r.D, r.ld = rows.data_ptr(), rows.shape[0], int(D), rows.stride(0)
+    r.tin, r.tout = tin.data_ptr(), tout.data_ptr()
+    r.u_begin, r.u_end = int(u_begin), int(u_end)
+    r.workspace, r.workspace_bytes = workspace.data_ptr(), workspace.numel() * workspace.element_size()
+    return r
+
+
+def reconstruction_f1(rows, hierarchy, geom, K, D=None, group=None, workspace_bytes=None, stats=None):
+    """check_graph_embedding (order_embeddings.py:512-559 = oe.py:1923-1990) without materialising the n (n-1)
+    energies: positives are E(x = rows[u], y = rows[v]) for every v below u in `hierarchy` (a hierarchy.Hierarchy),
+    negatives every other ordered pair u != v, and the result is best_f1_sweep's numpy row (f1, threshold, accuracy,
+    precision, recall, correct_positives, correct_negatives) over those energies, bit for bit, with the energies of
+    the fp32 SIMT scoring kernel (lec_recon_pass / lec_recon_finish).
+
+    rows: device fp32 [n, ld] -- a plain [n, D] table or an engine's padded rows (ConeStep.rows with D = ConeStep.D).
+    group: a torch.distributed group whose ranks each evaluate a contiguous share of the apex rows on their own GPU
+    (every rank passes the same rows); the counters are summed after every round, so every rank returns the row.
+    workspace_bytes: device workspace, lec_recon_workspace_bytes(RECON_OPEN_BINS) by default; a smaller one costs
+    rounds, not exactness.  stats: a dict that receives the rounds run, the open coarse bins, the numbers of positive
+    and negative pairs and the workspace size."""
+    N.require_cuda(rows)
+    if rows.dim() != 2 or rows.dtype != torch.float32:
+        raise N.LecError("reconstruction_f1: rows must be a float32 [n, ld] tensor")
+    n = rows.shape[0]
+    D = rows.shape[1] if D is None else int(D)
+    if n != hierarchy.n:
+        raise ValueError("reconstruction_f1: %d rows for a hierarchy of %d nodes" % (n, hierarchy.n))
+    if n < 2:
+        raise ValueError("reconstruction_f1: no pairs")
+    if D > rows.shape[1]:
+        raise ValueError("reconstruction_f1: D = %d exceeds the row width %d" % (D, rows.shape[1]))
+    rows = rows.detach()
+    if rows.stride(1) != 1 or (rows.stride(0) != D and rows.stride(0) % 4 != 0) or rows.data_ptr() % 16 != 0:
+        rows = rows[:, :D].contiguous()
+    dev = rows.device
+    lib = N.lib()
+    tin = torch.as_tensor(np.asarray(hierarchy.tin), dtype=torch.int32).to(dev)
+    tout = torch.as_tensor(np.asarray(hierarchy.tout), dtype=torch.int32).to(dev)
+    nb = int(lib.lec_recon_workspace_bytes(RECON_OPEN_BINS)) if workspace_bytes is None else int(workspace_bytes)
+    cb = int(lib.lec_recon_counter_bytes(nb))
+    if cb < 0:
+        N.check(cb, "lec_recon_counter_bytes")
+    ws = torch.zeros(nb, device=dev, dtype=torch.uint8)
+    rank, world = 0, 1
+    if group is not None:
+        import torch.distributed as dist
+        rank, world = dist.get_rank(group), dist.get_world_size(group)
+    r = recon_args(rows, tin, tout, geom, K, D, n * rank // world, n * (rank + 1) // world, ws)
+    out = torch.empty(7, device=dev, dtype=torch.float64)
+    status = torch.zeros(4, device=dev, dtype=torch.int64)
+    stream = N.stream_ptr(dev)
+    rounds = 0
+    while True:
+        N.check(lib.lec_recon_pass(ctypes.byref(r), stream), "lec_recon_pass")
+        rounds += 1
+        if group is not None:
+            dist.all_reduce(ws[:cb].view(torch.int64), group=group)
+        N.check(lib.lec_recon_finish(ctypes.byref(r), N._p(out), N._p(status), stream), "lec_recon_finish")
+        more, open_bins, n_pos, n_neg = (int(v) for v in status.cpu())
+        if not more:
+            break
+        if rounds > open_bins + 1:   # each fine round retires at least one open bin
+            raise N.LecError("lec_recon_finish asks for round %d with %d open bins" % (rounds + 1, open_bins))
+    if stats is not None:
+        stats.update(rounds=rounds, open_bins=open_bins, n_pos=n_pos, n_neg=n_neg, workspace_bytes=nb)
+    return out.cpu().numpy()
+
+
 class EmbeddingMetrics:
     """Same constructor and `calculate_metrics` contract as the reference's class."""
 
