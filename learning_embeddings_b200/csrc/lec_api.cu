@@ -287,7 +287,7 @@ int lec_cone_step(const lec_step_t* s, void* stream) {
     if (!u.rows_out || !u.loss_acc) return LEC_E_NULL;
     struct PdlScope {   // the kernels of this step are launched as programmatic dependents of one another
         int prev;
-        PdlScope() : prev(t_pdl) { static const int on = [] { const char* e = getenv("LEC_PDL"); return e ? atoi(e) : 1; }(); t_pdl = on; }
+        PdlScope() : prev(t_pdl) { t_pdl = 1; }
         ~PdlScope() { t_pdl = prev; }
     } pdl_scope;
     cudaStream_t st = (cudaStream_t)stream;

@@ -13,8 +13,11 @@ __device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
 __device__ __forceinline__ void mbar_expect_tx(unsigned bar, unsigned bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
+// Back-off of a warp that keeps finding an mbarrier phase incomplete: a waiting warp must not eat the issue slots of
+// the working ones.
+constexpr unsigned kMbarSleepNs = 32;
 // Spins on the phase; a lost arrival traps instead of hanging the GPU.
-__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity, int sleep_ns = 32) {
+__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
     unsigned ok = 0;
     for (unsigned spin = 0; !ok; ++spin) {
         asm volatile(
@@ -23,7 +26,7 @@ __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity, int sle
             "selp.u32 %0, 1, 0, p;\n\t}"
             : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
         if (!ok) {
-            if (spin > 4 && sleep_ns > 0) __nanosleep((unsigned)sleep_ns);   // a waiting warp must not eat the issue slots of the working ones
+            if (spin > 4) __nanosleep(kMbarSleepNs);
             if (spin > (1u << 22)) __trap();
         }
     }

@@ -69,16 +69,14 @@ __device__ __forceinline__ S warp_sum(S v) {
     return team_sum<32, S>(v);
 }
 
-// staged: `rows` is the block's shared-memory copy of the table (plain loads), else global memory (read-only path)
 template <int T, int V>
-__device__ __forceinline__ void load_row(Vec<V>& r, const float* __restrict__ rows, int64_t row, int ld, int lane_t,
-                                         bool staged = false) {
+__device__ __forceinline__ void load_row(Vec<V>& r, const float* __restrict__ rows, int64_t row, int ld, int lane_t) {
     const float* base = rows + row * (int64_t)ld;
     const int Q = ld >> 2;
 #pragma unroll
     for (int j = 0; j < V; ++j) {
         const int q = lane_t + T * j;
-        if (q < Q) r.c[j] = staged ? *reinterpret_cast<const float4*>(base + 4 * q) : ldg4(base + 4 * q);
+        if (q < Q) r.c[j] = ldg4(base + 4 * q);
         else r.c[j] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
 }

@@ -2,15 +2,10 @@
 // core.  Each lec_pairs_<core>.cu instantiates this header once for its core and exports three
 // launchers that lec_api.cu dispatches to.
 #pragma once
-#include <cstdlib>
-
 #include "lec_common.cuh"
 
 namespace lec {
 
-#ifndef LEC_GROUPED_MINBLOCKS
-#define LEC_GROUPED_MINBLOCKS 2   // default of the grouped kernel's register cap (LEC_GROUP_MINBLOCKS overrides at run time)
-#endif
 enum Core { CORE_EUC32 = 0, CORE_HYP32 = 1, CORE_HYP64 = 2, CORE_OE32 = 3 };
 
 template <int CORE> struct CoreTraits;
@@ -40,9 +35,7 @@ struct GroupArgs {
     float K, alpha;
     float* E_pos; float* E_neg; double* loss_out; float* grad_rows; int grad_replicas; int64_t replica_stride;
     int64_t n_rows; unsigned* index_errors;
-    int pdl_late;  // 1: let the dependent launch in only when this block has finished its groups (LEC_PDL_LATE)
     int split;  // teams per group (>= 1): team s of a group takes negatives p = s, s + split, ... of both lists
-    int64_t stage_floats;  // > 0: every block first copies the transformed table (n * ld floats) into shared memory
     int narrow_tail;       // the last float4 chunk of a row holds <= 2 live floats (D % 4 in {1, 2}): its reductions are 64-bit
     unsigned long long* trace;   // LEC_STEP_TRACE builds only
 };
@@ -180,28 +173,26 @@ __global__ void __launch_bounds__(kThreads) pairs_flat_kernel(const FlatArgs a) 
 // (cfg4: 2 520 positives x 51 pairs), a group is split over `split` teams: team s evaluates the positive
 // (s == 0 only) and every split-th negative of both lists, and flushes its own partial sums for u_i, v_i.
 // ------------------------------------------------------------------------------------------------
-// MB: minimum resident 256-thread blocks per SM the register allocation must allow.  MB = 2 caps the fp64-core kernel at
-// 128 registers (28 bytes of spill) and doubles the resident warps; MB = 1 lets it take the 184 it asks for.
-template <int CORE, int T, int V, bool GRAD, int MB>
-__global__ void __launch_bounds__(kThreads, MB) pairs_grouped_kernel(const GroupArgs a) {
+// Block size: the fp64-core kernel needs ~166 registers per thread, i.e. one 256-thread block (8 warps) per SM;
+// 128-thread blocks fit three (12 warps), which is what hides the gather / reduction latency.
+constexpr int kGroupThreads = 128;
+// Minimum resident 256-thread blocks per SM the register allocation must allow: 2 caps the kernel at 128 registers
+// (fp64 core: 28 bytes of spill, against the 184 it asks for uncapped) and doubles the resident warps.  The fp32 cores
+// with one float4 per row (D <= 4: cfg0) fit under a tighter cap without spilling and are gather-latency-bound -- r2x
+// sweep on cfg0: cap 128 / 80 / 64 -> pair kernel 29.8 / 26.8 / 29.2 us; rows of three chunks (D = 10) spill at 80 and
+// lose (18.0 -> 23.1 us).
+template <int CORE, int V>
+constexpr int kGroupedMinBlocks = (CORE != CORE_HYP64 && V == 1) ? LEC_FP32_MINBLOCKS : 2;
+
+template <int CORE, int T, int V, bool GRAD>
+__global__ void __launch_bounds__(kThreads, (kGroupedMinBlocks<CORE, V>)) pairs_grouped_kernel(const GroupArgs a) {
     using Tr = CoreTraits<CORE>;
     using Acc = typename Tr::Acc;
-    if (!a.pdl_late) pdl_launch_dependents();   // the update kernel may take its (few) SM slots now; it parks in pdl_wait()
+    pdl_launch_dependents();   // the update kernel may take its (few) SM slots now; it parks in pdl_wait()
     pdl_wait();                // rows / aux / cleared replicas of the previous update are complete
     if (threadIdx.x == 0) LEC_TRACE_MIN(a.trace, 0);
-    // Hot label table in shared memory (ETHEC: 723 x 12 floats = 35 KB): every endpoint gather of the block then is an
-    // LDS.128 instead of an L1-cached global load.
-    extern __shared__ __align__(16) float s_rows[];
-    const bool staged = a.stage_floats > 0;
-    const float* const rows_p = staged ? s_rows : a.rows;
-    if (staged) {
-        const float4* src = reinterpret_cast<const float4*>(a.rows);
-        float4* dst = reinterpret_cast<float4*>(s_rows);
-        for (int64_t i = threadIdx.x; i < (a.stage_floats >> 2); i += blockDim.x) dst[i] = __ldg(src + i);
-        __syncthreads();
-    }
     const int lane_t = threadIdx.x % T;
-    const int tpb = (int)blockDim.x / T;   // teams per block (the launcher picks the block size, <= kThreads)
+    constexpr int tpb = kGroupThreads / T;   // teams per block
     const int64_t n_teams = (int64_t)gridDim.x * tpb;
     const int64_t team = (int64_t)blockIdx.x * tpb + threadIdx.x / T;
     const int split = a.split;
@@ -224,8 +215,8 @@ __global__ void __launch_bounds__(kThreads, MB) pairs_grouped_kernel(const Group
         const int64_t iu = ld_index_checked(a.pos_from, gc, a.idx_bytes, a.n_rows, a.index_errors, writer && sub == 0, ok_g);
         const int64_t iv = ld_index_checked(a.pos_to, gc, a.idx_bytes, a.n_rows, a.index_errors, writer && sub == 0, ok_g);
         Vec<V> U, W;
-        load_row<T, V>(U, rows_p, iu, a.ld, lane_t, staged);
-        load_row<T, V>(W, rows_p, iv, a.ld, lane_t, staged);
+        load_row<T, V>(U, a.rows, iu, a.ld, lane_t);
+        load_row<T, V>(W, a.rows, iv, a.ld, lane_t);
         Aux<Acc> au{};
         Acc AW = 0;
         if (Tr::cone) au = load_aux<Acc>(a.aux, iu);
@@ -276,7 +267,7 @@ __global__ void __launch_bounds__(kThreads, MB) pairs_grouped_kernel(const Group
             bool ok = ok_g;
             const int64_t ic = ld_index_checked(a.neg_to, nbase + p, a.idx_bytes, a.n_rows, a.index_errors, writer && act, ok);
             Vec<V> C;
-            load_row<T, V>(C, rows_p, ic, a.ld, lane_t, staged);
+            load_row<T, V>(C, a.rows, ic, a.ld, lane_t);
             Acc AC = 0;
             if (Tr::hyp) AC = load_aux_A<Acc>(a.aux, ic);
             eval_pair<CORE, T, V, GRAD>(U, C, au, AC, g);
@@ -312,7 +303,7 @@ __global__ void __launch_bounds__(kThreads, MB) pairs_grouped_kernel(const Group
             bool ok = ok_g;
             const int64_t ic = ld_index_checked(a.neg_from, nbase + p, a.idx_bytes, a.n_rows, a.index_errors, writer && act, ok);
             Vec<V> C;
-            load_row<T, V>(C, rows_p, ic, a.ld, lane_t, staged);
+            load_row<T, V>(C, a.rows, ic, a.ld, lane_t);
             Aux<Acc> ac{};
             if (Tr::cone) ac = load_aux<Acc>(a.aux, ic);
             eval_pair<CORE, T, V, GRAD>(C, W, ac, AW, g);
@@ -362,7 +353,6 @@ __global__ void __launch_bounds__(kThreads, MB) pairs_grouped_kernel(const Group
             }
         }
     }
-    if (a.pdl_late) pdl_launch_dependents();
     block_add_double(loss, a.loss_out);
     if (threadIdx.x == 0) LEC_TRACE_MAX(a.trace, 1);
 }
@@ -440,10 +430,8 @@ int launch_flat_tv(const FlatArgs& a, cudaStream_t st) {
 // of a split group), so splitting only pays while the batch cannot fill the GPU: s is the largest split that still
 // fits one resident wave of `cap` teams.  cfg4 (2 569 positives x 51 pairs, cap 9 472) -> s = 3, measured 30.8 us against
 // 71.7 us unsplit and 37.0 us at s = 5 (profiles/r1d_cfg4_split_sweep.md); a batch that already fills the GPU (cfg1: 190 650
-// positives) stays at s = 1, where no pair is evaluated twice.  LEC_GROUP_SPLIT overrides (tuning).
+// positives) stays at s = 1, where no pair is evaluated twice.
 inline int choose_split(int64_t B, int N, int64_t cap) {
-    static const int forced = [] { const char* e = getenv("LEC_GROUP_SPLIT"); return e ? atoi(e) : 0; }();
-    if (forced > 0) return forced < N ? forced : (N > 0 ? N : 1);
     if (B <= 0 || N <= 1 || cap <= 0) return 1;
     int64_t s = cap / B;
     if (s > N) s = N;
@@ -453,48 +441,19 @@ inline int choose_split(int64_t B, int N, int64_t cap) {
 template <int CORE, int T, int V>
 int launch_grouped_tv(const GroupArgs& a0, cudaStream_t st) {
     GroupArgs a = a0;
-    // Block size: the fp64-core kernel needs ~166 registers per thread, i.e. one 256-thread block (8 warps) per SM;
-    // 128-thread blocks fit three (12 warps), which is what hides the gather / reduction latency (LEC_GROUP_BLOCK tunes).
-    static const int block = [] {
-        const char* e = getenv("LEC_GROUP_BLOCK");
-        int b = e ? atoi(e) : 128;
-        if (b < 32 || b > kThreads || (b & 31)) b = 128;
-        return b;
-    }();
-    static const int mb = [] { const char* e = getenv("LEC_GROUP_MINBLOCKS"); return (e ? atoi(e) : LEC_GROUPED_MINBLOCKS) >= 2 ? 2 : 1; }();
-    // register cap of the default build: 128 (two resident 256-thread blocks); 80 for the fp32 cores with one float4 per
-    // row (D <= 4: cfg0), which fit without spilling and are gather-latency-bound -- r2x sweep on cfg0: cap 128 / 80 / 64
-    // -> pair kernel 29.8 / 26.8 / 29.2 us; rows of three chunks (D = 10) spill at 80 and lose (18.0 -> 23.1 us).
-    constexpr int MBX = (CORE != CORE_HYP64 && V == 1) ? LEC_FP32_MINBLOCKS : 2;
+    constexpr int block = kGroupThreads;
     static const int resident_blocks = [] {
         int nb = 0;
-        if (mb == 2) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pairs_grouped_kernel<CORE, T, V, true, MBX>, block, 0);
-        else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pairs_grouped_kernel<CORE, T, V, true, 1>, block, 0);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, pairs_grouped_kernel<CORE, T, V, true>, block, 0);
         return nb > 0 ? nb : 1;
     }();
-    static const int pdl_late = [] { const char* e = getenv("LEC_PDL_LATE"); return e ? atoi(e) : 0; }();
-    a.pdl_late = pdl_late;
 #ifdef LEC_STEP_TRACE
     a.trace = g_step_trace;
 #endif
     a.split = choose_split(a.B, a.N, (int64_t)sm_count() * resident_blocks * (block / T));
     const int grid = grid_for(a.B * a.split, block / T, 8 * kThreads / block);
-    // Shared-memory staging of the table (LEC_STAGE_ROWS=1; tables <= 40 KB) was measured and is OFF by default: on
-    // cfg1 (723 x 12 floats) the per-block copy and the smaller L1 cost more than the LDS gathers save -- pair kernel
-    // 65.4 us staged vs 56.2 us with L1-resident read-only gathers (cfg0: 29.3 vs 27.6 us); profiles/r1f_notes.md.
-    static const int stage_env = [] { const char* e = getenv("LEC_STAGE_ROWS"); return e ? atoi(e) : 0; }();
-    const int64_t table_floats = a.replica_stride;   // n_rows * ld
-    const bool stage = stage_env != 0 && table_floats * 4 <= 40960;
-    a.stage_floats = stage ? table_floats : 0;
-    const size_t smem = stage ? (size_t)table_floats * 4 : 0;
-    cudaError_t le;
-    if (mb == 2) {
-        if (a.grad_rows) le = launch_step_kernel(pairs_grouped_kernel<CORE, T, V, true, MBX>, grid, block, st, a, smem);
-        else le = launch_step_kernel(pairs_grouped_kernel<CORE, T, V, false, MBX>, grid, block, st, a, smem);
-    } else {
-        if (a.grad_rows) le = launch_step_kernel(pairs_grouped_kernel<CORE, T, V, true, 1>, grid, block, st, a, smem);
-        else le = launch_step_kernel(pairs_grouped_kernel<CORE, T, V, false, 1>, grid, block, st, a, smem);
-    }
+    const cudaError_t le = a.grad_rows ? launch_step_kernel(pairs_grouped_kernel<CORE, T, V, true>, grid, block, st, a)
+                                       : launch_step_kernel(pairs_grouped_kernel<CORE, T, V, false>, grid, block, st, a);
     ++g_launches;
     return (int)(le != cudaSuccess ? le : cudaGetLastError());
 }

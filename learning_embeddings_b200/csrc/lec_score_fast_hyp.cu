@@ -1,4 +1,3 @@
-#define LEC_SCORE_TUNING_VARIANTS 1
 #include "lec_score_fast_impl.cuh"
 namespace lec {
 int score_fast_hyp(FastArgs& a, cudaStream_t st) { return fast_launch_geom<LEC_GEOM_HYP>(a, st); }

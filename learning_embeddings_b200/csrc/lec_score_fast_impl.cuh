@@ -30,16 +30,13 @@
 // ring entries inside merge(), with the same instruction sequence as the full-matrix path, so top-k
 // values are bit-identical to the matrix entries.  thr > pi/2 or an unfilled list accepts everything.
 #pragma once
-#include <cstdio>
-#include <cstdlib>
-
 #include "lec_common.cuh"
 #include "lec_packed.cuh"
 
 namespace lec {
 
 constexpr int kMaxSeg = 2 * LEC_MAX_LEVELS + 1;
-constexpr int kRingDefault = 16;  // candidate ring entries per thread
+constexpr int kRing = 16;  // candidate ring entries per thread
 constexpr int kTileLabels = 96;  // labels per shared-memory tile
 
 struct FastArgs {
@@ -565,29 +562,18 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     }
 }
 
-// experiment knob: LEC_SCORE_CFG="<images per thread>,<threads>,<min blocks>,<ring entries>" picks another instantiation
-static void tuning(int& ri, int& nt, int& minb, int& ring) {
-    static int cfg[4] = {0, 0, 0, 0};
-    static bool read = false;
-    if (!read) {
-        read = true;
-        const char* e = getenv("LEC_SCORE_CFG");
-        if (e) sscanf(e, "%d,%d,%d,%d", &cfg[0], &cfg[1], &cfg[2], &cfg[3]);
-    }
-    if (cfg[0]) ri = cfg[0];
-    if (cfg[1]) nt = cfg[1];
-    if (cfg[2]) minb = cfg[2];
-    if (cfg[3]) ring = cfg[3];
-}
-
-template <int GEOM, int DH, int RI, int NT, int MINB>
-static int fast_launch_cfg(FastArgs& a, cudaStream_t st) {
+// 128-thread blocks whose register allocation need only allow one resident block per SM; a thread holds RI images.
+template <int GEOM, int DH, int RI>
+static int fast_launch_dh(FastArgs& a, cudaStream_t st) {
+    constexpr int NT = 128;
+    static_assert(kRing > RI, "a thread appends up to RI candidates per label before the ring is merged");
+    a.ring = kRing;
     constexpr int LS = 4 * ((DH + 1) / 2) + 8;
     const size_t smem = (size_t)kTileLabels * LS * sizeof(float) + ((size_t)RI * a.k + a.ring) * NT * sizeof(float2) +
                         (size_t)a.ring * NT * sizeof(float) + 16;
     static size_t configured = 0;
     if (smem > configured) {
-        cudaError_t e = cudaFuncSetAttribute(score_fast_kernel<GEOM, DH, RI, NT, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(score_fast_kernel<GEOM, DH, RI, NT, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
         configured = smem;
     }
@@ -595,25 +581,9 @@ static int fast_launch_cfg(FastArgs& a, cudaStream_t st) {
     const int64_t blocks = a.groups * a.n_seg;
     if (blocks <= 0) return 0;
     if (blocks > 0x7fffffffLL) return LEC_E_SIZE;
-    score_fast_kernel<GEOM, DH, RI, NT, MINB><<<(unsigned)blocks, NT, smem, st>>>(a);
+    score_fast_kernel<GEOM, DH, RI, NT, 1><<<(unsigned)blocks, NT, smem, st>>>(a);
     ++g_launches;
     return (int)cudaGetLastError();
-}
-
-template <int GEOM, int DH, int RI_DEFAULT>
-static int fast_launch_dh(FastArgs& a, cudaStream_t st) {
-    int ri = RI_DEFAULT, nt = 128, minb = 1, ring = kRingDefault;
-    tuning(ri, nt, minb, ring);
-    a.ring = ring < 2 * ri ? 2 * ri : ring;
-#ifdef LEC_SCORE_TUNING_VARIANTS
-    if (ri == 4 && nt == 256) return fast_launch_cfg<GEOM, DH, 4, 256, 1>(a, st);
-    if (ri == 4 && nt == 128 && minb == 4) return fast_launch_cfg<GEOM, DH, 4, 128, 4>(a, st);
-    if (ri == 2 && nt == 256 && minb == 4) return fast_launch_cfg<GEOM, DH, 2, 256, 4>(a, st);
-    if (ri == 2 && nt == 128) return fast_launch_cfg<GEOM, DH, 2, 128, 1>(a, st);
-    if (ri == 6 && nt == 128) return fast_launch_cfg<GEOM, DH, 6, 128, 1>(a, st);
-    if (ri == 8 && nt == 128) return fast_launch_cfg<GEOM, DH, 8, 128, 1>(a, st);
-#endif
-    return fast_launch_cfg<GEOM, DH, RI_DEFAULT, 128, 1>(a, st);
 }
 
 template <int GEOM>

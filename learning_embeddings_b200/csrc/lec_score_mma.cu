@@ -248,8 +248,6 @@ struct MmaArgs {
     int cstages;             // constant + header stages (1..4), released by the epilogue threads
     int acc_stages;          // accumulator buffers in TMEM (1 or 2)
     int tmem_cols;           // power of two >= acc_stages * 96 + 2 Kp
-    int sleep_ns;            // back-off of a warp that keeps finding its mbarrier phase incomplete
-    int alt;                 // matrix-only launches: the two epilogue warp groups alternate chunks
 };
 
 constexpr int kMmaMaxStages = 4;
@@ -384,7 +382,7 @@ __global__ void __launch_bounds__(kMmaThreads, 2) score_mma_kernel(const MmaArgs
             mbar_init(bar_tfree0 + 8 * s, 1);
             // matrix-only launches with two accumulators split the chunks between the two 4-warp groups (see the
             // epilogue): a stage is then released by the 128 threads of its owner group only
-            const unsigned owners = (MODE == 1 && NA == 2 && a.alt) ? kEpiThreads / 2 : kEpiThreads;
+            const unsigned owners = (MODE == 1 && NA == 2) ? kEpiThreads / 2 : kEpiThreads;
             mbar_init(bar_empty0 + 8 * s, owners);
             mbar_init(bar_accfree0 + 8 * s, owners);
         }
@@ -465,7 +463,7 @@ __global__ void __launch_bounds__(kMmaThreads, 2) score_mma_kernel(const MmaArgs
                 }
                 if (moved) idle = 0;
                 else {
-                    if (a.sleep_ns > 0) __nanosleep((unsigned)a.sleep_ns);
+                    __nanosleep(kMbarSleepNs);
                     if (++idle > (1u << 24)) __trap();   // a lost arrival traps instead of hanging the GPU
                 }
             }
@@ -511,7 +509,7 @@ __global__ void __launch_bounds__(kMmaThreads, 2) score_mma_kernel(const MmaArgs
             if ((tid & 31) == 0) trace_issue[c & 255] = clock64();
 #endif
         };
-        if (MODE == 1 && NA == 2 && a.alt) {
+        if (MODE == 1 && NA == 2) {
             // Matrix-only launches: each 4-warp epilogue group owns one accumulator and every other chunk.  The two
             // chunk streams are served independently -- whichever group has released its accumulator (and has its tiles)
             // gets its next chunk; with in-order issue the faster group waited for the slower one's release.
@@ -546,10 +544,10 @@ __global__ void __launch_bounds__(kMmaThreads, 2) score_mma_kernel(const MmaArgs
             unsigned par = 0, par_t = 1;   // accfree[t] is first waited on for chunk NA, i.e. after one wrap of t
             for (int c = 0; c < a.n_chunks; ++c) {
                 TC_T0(w0);
-                mbar_wait(bar_tfull0 + 8 * s, par, a.sleep_ns);
+                mbar_wait(bar_tfull0 + 8 * s, par);
                 TC_ADD(0, w0);
                 TC_T0(w1);
-                if (c >= NA) mbar_wait(bar_accfree0 + 8 * t, par_t, a.sleep_ns);
+                if (c >= NA) mbar_wait(bar_accfree0 + 8 * t, par_t);
                 TC_ADD(1, w1);
                 TC_T0(w2);
                 issue(c, s, t);
@@ -624,7 +622,7 @@ __global__ void __launch_bounds__(kMmaThreads, 2) score_mma_kernel(const MmaArgs
         // accumulator buffers (ALT): warps 0-3 take the even chunks and warps 4-7 the odd ones, all labels of the chunk in
         // two batches -- half as many barrier / header / TMEM-load prologues per warp, and the two groups run out of
         // phase, so their MUFU- and FMA-heavy stretches interleave on an SM sub-partition instead of colliding.
-        const bool alt = (MODE == 1) && NA == 2 && a.alt;
+        const bool alt = (MODE == 1) && NA == 2;
         const int cstep = alt ? 2 : 1;
         // stage indices and phase parities advance by increments (no integer division in the chunk loop)
         int s = alt ? half : 0, t = alt ? half : 0;
@@ -637,7 +635,7 @@ __global__ void __launch_bounds__(kMmaThreads, 2) score_mma_kernel(const MmaArgs
 #endif
         for (int c = alt ? half : 0; c < a.n_chunks; c += cstep) {
             TC_T0(e0);
-            mbar_wait(bar_full0 + 8 * s, par, a.sleep_ns);   // constants + header of chunk c visible to this thread
+            mbar_wait(bar_full0 + 8 * s, par);   // constants + header of chunk c visible to this thread
             TC_ADD(4, e0);
             const unsigned char* bl = sC + (size_t)s * cstride;
             const float* cst = reinterpret_cast<const float*>(bl);
@@ -654,7 +652,7 @@ __global__ void __launch_bounds__(kMmaThreads, 2) score_mma_kernel(const MmaArgs
                 refresh();
             }
             TC_T0(e1);
-            mbar_wait(bar_done0 + 8 * t, par_t, a.sleep_ns);   // accumulator of chunk c complete
+            mbar_wait(bar_done0 + 8 * t, par_t);   // accumulator of chunk c complete
             TC_ADD(5, e1);
 #ifdef LEC_TC_TRACE
             trace_acc[9] += clock64() - trace_issue[c & 255];
@@ -930,10 +928,6 @@ int score_mma_launch(const float* labels, int64_t L, const float* images, int64_
     a.npsi = npsi;
     a.ring = topk_idx ? kMmaRing : 0;   // matrix-only launches need no candidate ring
     const int kk = (a.k == 5) ? 5 : LEC_MAX_TOPK;
-    static const int sleep_env = [] { const char* e = getenv("LEC_TC_SLEEP_NS"); return e ? atoi(e) : 32; }();
-    a.sleep_ns = sleep_env;
-    static const int alt_env = [] { const char* e = getenv("LEC_TC_ALT"); return e ? atoi(e) : 1; }();
-    a.alt = alt_env;
     const size_t fixed = (topk_idx ? (size_t)(2 * kk * kMmaM + kEpiThreads) * 8 : 0) + (size_t)a.ring * kEpiThreads * 8 + 256;
     // Stages.  Constants + header: four small stages (the epilogue holds one per chunk in flight).  Tiles: a stage is
     // free again as soon as the MMAs that read it complete, so one stage already overlaps the copy of chunk c + 1 with
@@ -944,10 +938,9 @@ int score_mma_launch(const float* labels, int64_t L, const float* images, int64_
     a.cstages = kMmaMaxStages;
     const size_t fixed_c = fixed + (size_t)a.cstages * cstride;
     const size_t half_sm = 113 * 1024, whole_sm = 226 * 1024;
-    static const int min_stages = [] { const char* e = getenv("LEC_TC_MIN_STAGES"); return e ? atoi(e) : 1; }();
     auto stages_for = [&](size_t budget) { return budget > fixed_c ? (int)((budget - fixed_c) / tiles) : 0; };
     int stages = a.tmem_cols <= 256 ? stages_for(half_sm) : 0;
-    if (stages < min_stages) stages = stages_for(whole_sm);
+    if (stages < 1) stages = stages_for(whole_sm);
     if (stages < 1) return LEC_E_DIM;
     a.stages = stages > kMmaMaxStages ? kMmaMaxStages : stages;
     const size_t smem = fixed_c + (size_t)a.stages * tiles;

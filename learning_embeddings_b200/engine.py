@@ -13,7 +13,6 @@ Euclidean one) with the negatives already drawn, as two launches (lec_cone_step)
 Index batches use the compact training layout of include/lec_b200.h (lec_pairs_grouped) as one uint16 / int32
 block [pos_from | pos_to | neg_to | neg_from] so a step's indices travel host->device in one copy.
 """
-import os
 
 import numpy as np
 import torch
@@ -98,13 +97,12 @@ class ConeStep:
             self.opt_v = torch.zeros((self.n, self.ld), device=dev, dtype=torch.float32)
         self.opt_step = 0
         self.write_grad_table = self.update == "none"   # set to True to keep d loss / d table of every step
-        # fused: the update also produces the rows / aux / cleared replicas the next step starts from (two launches per
-        # step).  LEC_FUSED_STEP=0 re-runs lec_rows_fwd at the start of every step instead (three launches).
-        self.fused = os.environ.get("LEC_FUSED_STEP", "1") != "0"
+        # the update also produces the rows / aux / cleared replicas the next step starts from (two launches per step);
+        # only the first step, and the first after invalidate_rows(), runs lec_rows_fwd first (three launches)
         self._rows_valid = False
         # host->device staging: `depth` slots so that the copies of steps i+1, i+2 overlap the kernels of step i (r2: with
         # host-drawn negatives the step is PCIe-bound; depth 2 -> 3: 101 -> 88.6 us per step, no change beyond 3)
-        self.depth = max(1, min(16, int(os.environ.get("LEC_PIPE_DEPTH", "3"))))
+        self.depth = 3
         self._idx_bytes_dev = [torch.empty(self.max_groups * (2 + 2 * self.n_neg) * 4, device=dev, dtype=torch.uint8)
                                for _ in range(self.depth)]
         self.loss_host = torch.zeros(self.depth, dtype=torch.float64).pin_memory()
@@ -186,7 +184,7 @@ class ConeStep:
         B = int(pos_from.numel())
         if B > self.max_groups:
             raise N.LecError("batch of %d positives exceeds max_groups=%d" % (B, self.max_groups))
-        if not (self.fused and self._rows_valid):
+        if not self._rows_valid:
             self._rows_fwd()
         self._rows_valid = False
         ev = self.kernel_events
@@ -234,7 +232,7 @@ class ConeStep:
             self.opt_step += 1
         if self.comm == "p2p":
             self.px.step += 1
-        self._rows_valid = self.fused
+        self._rows_valid = True
 
     def check_exchange(self):
         """Raises if the peer exchange reported a failure (a rank did not deliver its gradient in time).  Synchronises."""
@@ -267,7 +265,7 @@ class ConeStep:
             if self.comm == "p2p":
                 self.px.fill(s.xchg)
         s.geom, s.precision, s.alpha = N.GEOM[self.geom], self.precision, self.alpha
-        s.fused = 1 if (self.fused and self._rows_valid) else 0
+        s.fused = 1 if self._rows_valid else 0
         s.pos_from, s.pos_to, s.neg_to, s.neg_from = p_from, p_to, n_to, n_from
         s.idx_bytes, s.B = idx_bytes, B
         s.w_pos = w_pos.data_ptr() if w_pos is not None else None

@@ -17,10 +17,9 @@ def default_replicas(n_rows, ld):
     """How many private copies of the gradient table the pair kernels scatter into.
 
     Same-address L2 reductions serialise, so a small hot table (ETHEC: 723 rows) is replicated; a big
-    table (82 K rows) has little per-address contention and stays single.  Budget: 2 M floats."""
-    import os
-    cap = int(os.environ.get("LEC_REPLICAS", "8"))   # r1g sweep: 4..32 replicas differ by < 2 us in the pair kernel; 8 keeps the update short
-    return int(max(1, min(cap, (2 << 20) // max(1, int(n_rows) * int(ld)))))
+    table (82 K rows) has little per-address contention and stays single.  Budget: 2 M floats, at most 8 copies
+    (r1g sweep: 4..32 replicas differ by < 2 us in the pair kernel; 8 keeps the update short)."""
+    return int(max(1, min(8, (2 << 20) // max(1, int(n_rows) * int(ld)))))
 
 
 def reduce_replicas(grad_rows):

@@ -21,11 +21,6 @@ for spec in ${VARIANTS:-}; do
   timeout 300 python scripts/score_bench.py --dims ${DIMS:-10,50} --iters 9 --modes ${MODES:-topk,matrix_lm,both_lm} --engines tc > $O/score_bench_$name.log 2>&1
   echo "== variant $name ($flags)"; cat $O/score_bench_$name.log
 done
-for spec in ${ENV_VARIANTS:-}; do   # name:VAR=value -- same binary, another environment
-  name=${spec%%:*}; kv=${spec#*:}
-  env $kv timeout 300 python scripts/score_bench.py --dims ${DIMS:-10,50} --iters 9 --modes ${MODES:-topk,matrix_lm,both_lm} --engines tc > $O/score_bench_$name.log 2>&1
-  echo "== env variant $name ($kv)"; cat $O/score_bench_$name.log
-done
 if [ -n "${VARIANTS:-}" ]; then
   rm -f learning_embeddings_b200/csrc/build/lec_score_mma.o
   make -C learning_embeddings_b200/csrc > $O/make_restore.log 2>&1

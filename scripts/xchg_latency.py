@@ -52,7 +52,7 @@ def main():
                            process_group=None if comm == "none" else dist.group.WORLD,
                            comm="auto" if comm == "none" else ("nccl" if comm == "nccl" else "p2p"), exchange_mode=mode)
             eng._rows_fwd()
-            eng.fused, eng._rows_valid = True, True
+            eng._rows_valid = True
             res[comm] = timed(eng.reduce_and_update)
             if comm in ("p2p", "two_shot"):
                 eng.check_exchange()

@@ -685,10 +685,10 @@ def test_engine_step_at_wordnet_scale_matches_fp64_oracle():
 
 
 @pytest.mark.parametrize("D", (2, 10, 50))
-def test_fused_update_and_row_transform_equals_separate_launches(D):
+def test_fused_step_equals_three_launch_step_after_invalidate_rows(D):
     """lec_cone_step with fused = 1 (pairs -> lec_update_rows: update + the next step's Embedder.forward in one launch)
-    must leave the same tables and losses as the three-launch step (lec_rows_fwd first), and the same rows / aperture
-    terms as a separate lec_rows_fwd of the updated table."""
+    must leave the same tables and losses as the three-launch step (lec_rows_fwd first, which invalidate_rows() asks
+    for), and the same rows / aperture terms as a separate lec_rows_fwd of the updated table."""
     from learning_embeddings_b200.engine import ConeStep, pack_index_block
     from learning_embeddings_b200 import hierarchy
     ethec = hierarchy.ethec()
@@ -698,26 +698,25 @@ def test_fused_update_and_row_transform_equals_separate_launches(D):
     gen = torch.Generator().manual_seed(4)
     w = torch.randn(ethec.n, D, generator=gen)
     w = w / w.norm(dim=1, keepdim=True) * (0.05 + 0.9 * torch.rand(ethec.n, 1, generator=gen))   # some rows inside r_in
-    tabs, engs = [], []
-    for fused in (True, False):
-        tab = w.to(DEV).clone()
-        e = ConeStep(tab, "hyp", Nn, B, K=0.1, alpha=0.05, lr=0.01)
-        assert e.fused
-        e.fused = fused
-        e._struct = None
-        tabs.append(tab)
-        engs.append(e)
+    tabs = [w.to(DEV).clone() for _ in range(2)]
+    engs = [ConeStep(tab, "hyp", Nn, B, K=0.1, alpha=0.05, lr=0.01) for tab in tabs]
+
+    def step_both(blk):
+        engs[1].invalidate_rows()   # every step of the second engine is the three-launch step
+        return [e.step_host(blk, B) for e in engs]
+
     for step in range(4):
         sel = rng.integers(0, len(edges), size=B)
         u, v = edges[sel, 0], edges[sel, 1]
         neg_to, neg_from = ethec.sample_negatives(u, v, Nn, rng)
         blk = pack_index_block(u, v, neg_to, neg_from)
-        losses = [e.step_host(blk, B) for e in engs]
+        losses = step_both(blk)
         # the gradient scatter uses fp32 L2 reductions, whose order differs from launch to launch: two runs of the SAME
         # step agree to ~1e-5 on the table, not bit for bit -- that is the resolution of this comparison
         assert np.isfinite(losses[0]) and abs(losses[0] - losses[1]) <= 1e-6 * abs(losses[1])
         assert float((tabs[0] - tabs[1]).abs().max()) < 5e-5
         np.testing.assert_allclose(engs[0].E_neg.cpu().numpy(), engs[1].E_neg.cpu().numpy(), rtol=0, atol=2e-3)
+    assert engs[0]._struct.fused == 1 and engs[1]._struct.fused == 0
     # the fused engine already holds the rows of the NEXT step: what a separate lec_rows_fwd of its table gives
     rows, aux = ops.rows_forward(tabs[0], N.ROWS_HYP_SHELL, 0.1, geom="hyp")
     # (the two kernels reduce a row's norm over different team widths, so a row sitting exactly on the inner shell can
@@ -730,7 +729,7 @@ def test_fused_update_and_row_transform_equals_separate_launches(D):
         tabs[0].mul_(0.5)
         tabs[1].copy_(tabs[0])
     engs[0].invalidate_rows()
-    losses = [e.step_host(blk, B) for e in engs]
+    losses = step_both(blk)
     assert abs(losses[0] - losses[1]) <= 1e-6 * abs(losses[1]) and float((tabs[0] - tabs[1]).abs().max()) < 5e-5
 
 
