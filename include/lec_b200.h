@@ -455,6 +455,17 @@ typedef struct lec_recon {
 int64_t lec_recon_workspace_bytes(int open_bins_per_round);
 int64_t lec_recon_counter_bytes(int64_t workspace_bytes);
 int lec_recon_pass(const lec_recon_t* r, void* stream);
+/* lec_recon_pass_dag is lec_recon_pass for a closure that is not a forest's (a DAG, e.g. WordNet's nouns).  tin / tout
+ * are then a cover of each apex's descendants by preorder numbers of a spanning forest: a pair v != u is positive iff
+ * tin[u] < tin[v] <= tout[u] or tin[v] lies in one of u's extra intervals [lo[i], hi[i]], i in [ptr[u], ptr[u+1]),
+ * sorted by lo and disjoint (hierarchy.DagHierarchy builds them).  Rounds, workspace, the [u_begin, u_end) shards and
+ * lec_recon_finish are those of lec_recon_pass.  x == NULL or x->count == 0 is exactly lec_recon_pass; otherwise a
+ * NULL ptr / lo / hi returns LEC_E_NULL and count < 0 or > INT32_MAX returns LEC_E_SIZE. */
+typedef struct lec_recon_extra {
+    const int32_t* ptr; const int32_t* lo; const int32_t* hi;  /* device: ptr[n+1], lo/hi[ptr[n]] */
+    int64_t count;                                             /* ptr[n] */
+} lec_recon_extra_t;
+int lec_recon_pass_dag(const lec_recon_t* r, const lec_recon_extra_t* x, void* stream);
 int lec_recon_finish(const lec_recon_t* r, double* out7, int64_t* status, void* stream);
 
 /* lec_classify_counts replaces the per-image bookkeeping of JointEmbeddings.calculate_classification_metrics

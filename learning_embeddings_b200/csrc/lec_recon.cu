@@ -3,7 +3,8 @@
 // pair u != v, then EmbeddingMetrics.calculate_metrics('val')).
 //
 // The energies are the SIMT scoring kernel's (score_fast_kernel with EPI = 1: same per-pair instructions, so the same
-// bits as the lec_score_topk_ex matrix), classified by the Euler intervals and counted, never stored:
+// bits as the lec_score_topk_ex matrix), classified by the Euler intervals and counted, never stored (EPI = 2,
+// lec_recon_pass_dag: a DAG's interval cover, the Euler-like primary interval plus each apex's extra intervals):
 //   round 0      every pair's key (fp32 bits; energies are >= 0 or NaN) into 2 x 32 768 coarse bins (key >> 16)
 //   select       exact F1 at each coarse bin's largest value gives a lower bound LB on the best F1; a bin can
 //                only hold a better threshold if 2 CP_b / (n_pos + CP_b + FP_{b-1}) >= LB (1 - 1e-12) -- the slack
@@ -250,14 +251,15 @@ __global__ void __launch_bounds__(kSelThreads) recon_merge_kernel(ReconState* __
     }
 }
 
-template <int GEOM, int DH, int RI>
+template <int GEOM, int DH, int RI, int EPI>
 int recon_launch_dh(FastArgs& a, cudaStream_t st) {
     constexpr int NT = recon_threads<DH>();
     constexpr int LS = 4 * ((DH + 1) / 2) + 8;
-    const size_t smem = (size_t)kTileLabels * LS * sizeof(float) + (size_t)kReconBins * sizeof(unsigned);
+    const size_t smem = (size_t)kTileLabels * LS * sizeof(float) + (size_t)kReconBins * sizeof(unsigned) +
+                        (EPI == 2 ? (size_t)kTileLabels * sizeof(int2) : 0);
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(score_fast_kernel<GEOM, DH, RI, NT, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(score_fast_kernel<GEOM, DH, RI, NT, 1, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
         configured = true;
     }
@@ -271,21 +273,21 @@ int recon_launch_dh(FastArgs& a, cudaStream_t st) {
     chunks = (rows + chunk - 1) / chunk;
     const int64_t blocks = a.groups * chunks;
     if (blocks > 0x7fffffffLL) return LEC_E_SIZE;
-    score_fast_kernel<GEOM, DH, RI, NT, 1, 1><<<(unsigned)blocks, NT, smem, st>>>(a);
+    score_fast_kernel<GEOM, DH, RI, NT, 1, EPI><<<(unsigned)blocks, NT, smem, st>>>(a);
     ++g_launches;
     return (int)cudaGetLastError();
 }
 
-template <int GEOM>
+template <int GEOM, int EPI>
 int recon_launch_geom(FastArgs& a, cudaStream_t st) {
     const int dh = (a.D + 1) / 2;   // the scoring kernel's instantiations (fast_launch_geom)
-    if (dh <= 1) return recon_launch_dh<GEOM, 1, 4>(a, st);
-    if (dh <= 2) return recon_launch_dh<GEOM, 2, 4>(a, st);
-    if (dh <= 5) return recon_launch_dh<GEOM, 5, 4>(a, st);
-    if (dh <= 8) return recon_launch_dh<GEOM, 8, 4>(a, st);
-    if (dh <= 16) return recon_launch_dh<GEOM, 16, 2>(a, st);
-    if (dh <= 25) return recon_launch_dh<GEOM, 25, 2>(a, st);
-    if (dh <= 32) return recon_launch_dh<GEOM, 32, 2>(a, st);
+    if (dh <= 1) return recon_launch_dh<GEOM, 1, 4, EPI>(a, st);
+    if (dh <= 2) return recon_launch_dh<GEOM, 2, 4, EPI>(a, st);
+    if (dh <= 5) return recon_launch_dh<GEOM, 5, 4, EPI>(a, st);
+    if (dh <= 8) return recon_launch_dh<GEOM, 8, 4, EPI>(a, st);
+    if (dh <= 16) return recon_launch_dh<GEOM, 16, 2, EPI>(a, st);
+    if (dh <= 25) return recon_launch_dh<GEOM, 25, 2, EPI>(a, st);
+    if (dh <= 32) return recon_launch_dh<GEOM, 32, 2, EPI>(a, st);
     return LEC_E_DIM;
 }
 
@@ -313,10 +315,15 @@ extern "C" int64_t lec_recon_counter_bytes(int64_t workspace_bytes) {
     return b < 1 ? (int64_t)LEC_E_SIZE : lec::counter_bytes_of(b);
 }
 
-extern "C" int lec_recon_pass(const lec_recon_t* r, void* stream) {
+extern "C" int lec_recon_pass_dag(const lec_recon_t* r, const lec_recon_extra_t* x, void* stream) {
     using namespace lec;
     const int err = validate(r);
     if (err) return err;
+    const bool dag = x != nullptr && x->count != 0;
+    if (dag) {
+        if (x->count < 0 || x->count > 0x7fffffffLL) return LEC_E_SIZE;
+        if (!x->ptr || !x->lo || !x->hi) return LEC_E_NULL;
+    }
     if (r->u_end == r->u_begin) return 0;
     const Layout l = layout(r->workspace, r->workspace_bytes);
     FastArgs a{};
@@ -325,11 +332,23 @@ extern "C" int lec_recon_pass(const lec_recon_t* r, void* stream) {
     a.tin = r->tin; a.tout = r->tout;
     a.rstate = l.state; a.ropen = l.open; a.rhdr = l.hdr; a.rhist = l.hist;
     cudaStream_t st = (cudaStream_t)stream;
-    switch (r->geom) {
-        case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC>(a, st);
-        case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP>(a, st);
-        default: return recon_launch_geom<LEC_GEOM_OE>(a, st);
+    if (dag) {  // only apexes with extra intervals leave the forest kernel's instructions
+        a.xptr = x->ptr; a.xlo = x->lo; a.xhi = x->hi;
+        switch (r->geom) {
+            case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 2>(a, st);
+            case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 2>(a, st);
+            default: return recon_launch_geom<LEC_GEOM_OE, 2>(a, st);
+        }
     }
+    switch (r->geom) {
+        case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 1>(a, st);
+        case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 1>(a, st);
+        default: return recon_launch_geom<LEC_GEOM_OE, 1>(a, st);
+    }
+}
+
+extern "C" int lec_recon_pass(const lec_recon_t* r, void* stream) {
+    return lec_recon_pass_dag(r, nullptr, stream);
 }
 
 extern "C" int lec_recon_finish(const lec_recon_t* r, double* out7, int64_t* status, void* stream) {

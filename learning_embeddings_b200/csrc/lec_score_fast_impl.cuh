@@ -54,6 +54,8 @@ struct FastArgs {
     const int32_t* tin; const int32_t* tout;
     const struct ReconState* rstate; const struct ReconOpen* ropen;
     unsigned long long* rhdr; unsigned long long* rhist;
+    // DAG reconstruction pass (EPI = 2): apex u's extra preorder intervals [xlo[i], xhi[i]], i in [xptr[u], xptr[u+1])
+    const int32_t* xptr; const int32_t* xlo; const int32_t* xhi;
 };
 
 // Reconstruction check (lec_recon.cu).  Key of an energy = its fp32 bit pattern (energies are >= 0 or NaN, -0 is
@@ -81,6 +83,7 @@ struct IntC {
 };
 
 // EPI = 1: the reconstruction pass -- the same energies, counted into the lec_recon.cu histograms instead of stored
+// EPI = 2: the same pass on a DAG: a pair is also positive when tin[v] lies in one of the apex's extra intervals
 template <int GEOM, int DH, int RI, int NT, int MINB, int EPI = 0>
 __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) {
     static_assert(RI % 2 == 0, "images are packed in pairs");
@@ -142,6 +145,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     // fraction of a percent of the pairs, go straight to global memory); fine rounds = the batch slot of every coarse
     // bin (or -1) in the same shared array.  Zeros, NaNs and the pair counts stay in registers until the block ends.
     unsigned* rsh = reinterpret_cast<unsigned*>(smem + kTileLabels * LS);
+    int2* xsh = reinterpret_cast<int2*>(rsh + kReconBins);  // EPI = 2: [kTileLabels] {first extra interval, count}
     int rphase = 0;
     int tin_v[RI];
     unsigned c_np = 0, c_nn = 0, c_nanp = 0, c_nann = 0, c_zp = 0, c_zn = 0;
@@ -400,7 +404,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     };
 
     // STORE: 0 no matrix, 1 label-major and every image of the group exists, 2 generic strides / partial group,
-    // 3 reconstruction counts
+    // 3 reconstruction counts, 4 reconstruction counts with extra intervals (DAG)
     auto tile_loop = [&](int l0, int tl, auto store_c, auto topk_c) {
         constexpr int STORE = decltype(store_c)::value;
         constexpr bool TOPK = decltype(topk_c)::value != 0;
@@ -431,6 +435,36 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 for (int r = 0; r < RI; ++r) {
                     const int64_t v = img0 + r * NT;
                     recon_count(E[r], v < a.N && v != u, tin_u < tin_v[r] && tin_v[r] <= tout_u);
+                }
+            } else if (STORE == 4) {
+                const int u = l0 + t;
+                const int* ue = reinterpret_cast<const int*>(lab + t * LS + 4 * DQ + 6);
+                const int tin_u = ue[0], tout_u = ue[1];
+                bool pos[RI];
+#pragma unroll
+                for (int r = 0; r < RI; ++r) pos[r] = tin_u < tin_v[r] && tin_v[r] <= tout_u;
+                const int2 xe = xsh[t];
+                if (xe.y > 0) {  // block-uniform: every thread is on apex u
+                    // per image: how many of u's extra intervals start at or before tin_v (binary lifting over the
+                    // sorted starts, the same ceil(log2(count + 1)) steps in every lane), then the end of the last one
+                    int below[RI];
+#pragma unroll
+                    for (int r = 0; r < RI; ++r) below[r] = 0;
+                    for (int s = 1 << (31 - __clz(xe.y)); s > 0; s >>= 1) {
+#pragma unroll
+                        for (int r = 0; r < RI; ++r) {
+                            const int i = below[r] + s;
+                            if (i <= xe.y && __ldg(a.xlo + xe.x + i - 1) <= tin_v[r]) below[r] = i;
+                        }
+                    }
+#pragma unroll
+                    for (int r = 0; r < RI; ++r)
+                        pos[r] |= below[r] > 0 && tin_v[r] <= __ldg(a.xhi + xe.x + below[r] - 1);
+                }
+#pragma unroll
+                for (int r = 0; r < RI; ++r) {
+                    const int64_t v = img0 + r * NT;
+                    recon_count(E[r], v < a.N && v != u, pos[r]);
                 }
             }
             if (TOPK) {
@@ -480,6 +514,10 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 int* ue = reinterpret_cast<int*>(lab + t * LS + 4 * DQ + 6);
                 ue[0] = a.tin[l0 + t];
                 ue[1] = a.tout[l0 + t];
+                if (EPI == 2) {
+                    const int x0 = a.xptr[l0 + t];
+                    xsh[t] = make_int2(x0, a.xptr[l0 + t + 1] - x0);
+                }
             }
         }
         __syncthreads();
@@ -495,7 +533,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
             refresh_filter();
         }
         if (EPI) {
-            tile_loop(l0, tl, IntC<3>(), IntC<0>());
+            tile_loop(l0, tl, IntC<EPI == 2 ? 4 : 3>(), IntC<0>());
         } else if (want_topk) {
             if (store == 0 && GEOM == LEC_GEOM_HYP) tile_loop_deferred(l0, tl);
             else if (store == 0) tile_loop(l0, tl, IntC<0>(), IntC<1>());

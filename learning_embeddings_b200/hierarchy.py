@@ -2,8 +2,9 @@
 
 The ETHEC parent array in data/ethec_hierarchy.npz was extracted from the reference's hard-coded
 taxonomy (data/db.py:3480-3510, ETHECLabelMapMerged) by tests/golden/make_golden.py; it is data, not
-code.  Closure / non-edge queries use Euler-tour intervals, so nothing here needs the reference's dense
-n x n adjacency (order_embeddings.py:417-423), which does not exist at 82 K nodes (SURVEY F7).
+code.  Closure / non-edge queries use Euler-tour intervals (a forest) or an interval cover (DagHierarchy, a node with
+several parents), so nothing here needs the reference's dense n x n adjacency (order_embeddings.py:417-423), which does
+not exist at 82 K nodes (SURVEY F7).
 """
 import os
 
@@ -12,17 +13,70 @@ import numpy as np
 _DATA = os.path.join(os.path.dirname(os.path.abspath(__file__)), "data")
 
 
-class Hierarchy:
-    """Forest given by a parent array (-1 = root).  Node ids are level-major like the reference's."""
+class _Closure:
+    """Queries shared by Hierarchy and DagHierarchy, written in terms of is_descendant(u, v), closure_edges() and
+    the per-node counts n_desc (strict descendants) and n_anc (strict ancestors)."""
 
-    def __init__(self, parents, levels=None):
-        self.parents = np.asarray(parents, dtype=np.int64)
-        self.n = len(self.parents)
+    def _set_levels(self, levels):
         self.levels = None if levels is None else [int(v) for v in levels]
         if self.levels is not None:
             stops = np.cumsum(self.levels)
             self.level_start = [int(v) for v in stops - np.asarray(self.levels)]
             self.level_stop = [int(v) for v in stops]
+
+    def negative_adjacency(self):
+        """Dense bool matrix of the reference (ones - closure - diagonal); only sensible for small n."""
+        A = np.ones((self.n, self.n), dtype=bool)
+        e = self.closure_edges()
+        A[e[:, 0], e[:, 1]] = False
+        np.fill_diagonal(A, False)
+        return A
+
+    def sample_negatives(self, u, v, n_neg, rng):
+        """Uniform draws from the reference's candidate sets, vectorised (rejection on is_descendant).
+
+        neg_to[i, p]   uniform over {x : x != u_i, x not a descendant of u_i}   (corrupt the child)
+        neg_from[i, p] uniform over {x : x != v_i, x not an ancestor of v_i}    (corrupt the parent)
+        Same distribution as random.choice(np.where(negative_G[u])) but NOT the same stream: used for
+        synthetic benchmark batches; the bit-exact sampler is criterion.sample_negative_edge.
+        Raises IndexError, before any draw, when a candidate set is empty: u_i above every other node, or v_i below
+        every other node (a Hierarchy that is a chain, where the rejection loop could never end)."""
+        u = np.asarray(u)
+        v = np.asarray(v)
+        B = len(u)
+        uu = np.repeat(u[:, None], n_neg, 1)
+        vv = np.repeat(v[:, None], n_neg, 1)
+        # a node whose subtree is everything else has no "corrupted child" candidate: the reference's
+        # random.choice raises IndexError on the empty list (order_embeddings.py:1007); likewise a child below
+        # every other node has no "corrupted parent" candidate
+        if len(u) and int(self.n_desc[u].max()) >= self.n - 1:
+            raise IndexError("a positive's parent is an ancestor of every other node: no negative candidate")
+        if len(v) and int(self.n_anc[v].max()) >= self.n - 1:
+            raise IndexError("a positive's child is a descendant of every other node: no negative candidate")
+        neg_to = rng.integers(0, self.n, size=(B, n_neg))
+        neg_from = rng.integers(0, self.n, size=(B, n_neg))
+        while True:
+            bad = (neg_to == uu) | self.is_descendant(uu, neg_to)
+            k = int(bad.sum())
+            if k == 0:
+                break
+            neg_to[bad] = rng.integers(0, self.n, size=k)
+        while True:
+            bad = (neg_from == vv) | self.is_descendant(neg_from, vv)
+            k = int(bad.sum())
+            if k == 0:
+                break
+            neg_from[bad] = rng.integers(0, self.n, size=k)
+        return neg_to, neg_from
+
+
+class Hierarchy(_Closure):
+    """Forest given by a parent array (-1 = root).  Node ids are level-major like the reference's."""
+
+    def __init__(self, parents, levels=None):
+        self.parents = np.asarray(parents, dtype=np.int64)
+        self.n = len(self.parents)
+        self._set_levels(levels)
         order = np.argsort(self.parents, kind="stable")
         self.children_ptr = np.searchsorted(self.parents[order], np.arange(-1, self.n + 1))
         self.children_idx = order
@@ -44,6 +98,8 @@ class Hierarchy:
                     stack.append((int(c), 0))
             else:
                 self.tout[node] = clock - 1
+        self.n_desc = self.tout - self.tin
+        self.n_anc = self.depth
 
     @classmethod
     def from_closure_edges(cls, n, edges):
@@ -99,45 +155,120 @@ class Hierarchy:
         o = np.lexsort((v, u))
         return np.stack([u[o], v[o]], axis=1)
 
-    def negative_adjacency(self):
-        """Dense bool matrix of the reference (ones - closure - diagonal); only sensible for small n."""
-        A = np.ones((self.n, self.n), dtype=bool)
-        e = self.closure_edges()
-        A[e[:, 0], e[:, 1]] = False
-        np.fill_diagonal(A, False)
-        return A
 
-    def sample_negatives(self, u, v, n_neg, rng):
-        """Uniform draws from the reference's candidate sets, vectorised (rejection on Euler intervals).
+def _edge_keys(e, n):
+    return e[:, 0] * n + e[:, 1]
 
-        neg_to[i, p]   uniform over {x : x != u_i, x not a descendant of u_i}   (corrupt the child)
-        neg_from[i, p] uniform over {x : x != v_i, x not an ancestor of v_i}    (corrupt the parent)
-        Same distribution as random.choice(np.where(negative_G[u])) but NOT the same stream: used for
-        synthetic benchmark batches; the bit-exact sampler is criterion.sample_negative_edge."""
-        u = np.asarray(u)
-        v = np.asarray(v)
-        B = len(u)
-        uu = np.repeat(u[:, None], n_neg, 1)
-        vv = np.repeat(v[:, None], n_neg, 1)
-        # a node whose subtree is everything else has no "corrupted child" candidate: the reference's
-        # random.choice raises IndexError on the empty list (order_embeddings.py:1007)
-        if len(u) and int((self.tout[u] - self.tin[u]).max()) >= self.n - 1:
-            raise IndexError("a positive's parent is an ancestor of every other node: no negative candidate")
-        neg_to = rng.integers(0, self.n, size=(B, n_neg))
-        neg_from = rng.integers(0, self.n, size=(B, n_neg))
-        while True:
-            bad = (neg_to == uu) | self.is_descendant(uu, neg_to)
-            k = int(bad.sum())
-            if k == 0:
-                break
-            neg_to[bad] = rng.integers(0, self.n, size=k)
-        while True:
-            bad = (neg_from == vv) | self.is_descendant(neg_from, vv)
-            k = int(bad.sum())
-            if k == 0:
-                break
-            neg_from[bad] = rng.integers(0, self.n, size=k)
-        return neg_to, neg_from
+
+def _compose(first, second, n):
+    """Keys a * n + c of the pairs (a, c) with (a, b) in `first` and (b, c) in `second`, with repeats."""
+    o = np.argsort(second[:, 0], kind="stable")
+    src, dst = second[o, 0], second[o, 1]
+    ptr = np.searchsorted(src, np.arange(n + 1))
+    b = first[:, 1]
+    cnt = ptr[b + 1] - ptr[b]
+    total = int(cnt.sum())
+    at = np.arange(total) - np.repeat(np.cumsum(cnt) - cnt, cnt) + np.repeat(ptr[b], cnt)
+    return np.repeat(first[:, 0], cnt) * n + dst[at]
+
+
+def _in_sorted(keys, sorted_keys):
+    if len(sorted_keys) == 0:
+        return np.zeros(len(keys), dtype=bool)
+    i = np.minimum(np.searchsorted(sorted_keys, keys), len(sorted_keys) - 1)
+    return sorted_keys[i] == keys
+
+
+def _edge_array(n, edges, what):
+    e = np.asarray(edges, dtype=np.int64).reshape(-1, 2)
+    if len(e) and (e.min() < 0 or e.max() >= n):
+        raise ValueError("%s endpoint outside [0, %d)" % (what, n))
+    if np.any(e[:, 0] == e[:, 1]):
+        raise ValueError("%s from a node to itself" % what)
+    k = np.unique(_edge_keys(e, n))
+    return np.stack([k // n, k % n], axis=1), k
+
+
+class DagHierarchy(_Closure):
+    """Transitive closure of a DAG: a node may have several parents (the WordNet noun hierarchy is one).  Descendant
+    queries use an interval cover instead of the dense n x n closure: the preorder numbers `tin` of a spanning
+    forest, a primary interval [tin[u], tout[u]] of numbers that are all u or below u, and the maximal runs of u's
+    other descendants' numbers as extra intervals [extra_lo[i], extra_hi[i]], i in [extra_ptr[u], extra_ptr[u+1]),
+    sorted and disjoint.  The closure of a forest has Hierarchy's tin / tout and no extra interval."""
+
+    def __init__(self, n, edges, levels=None):
+        """`edges`: the closure's (ancestor, descendant) pairs, unique, sorted and checked; build one with
+        from_closure_edges or from_parents."""
+        self.n = int(n)
+        self._set_levels(levels)
+        e = self._edges = np.asarray(edges, dtype=np.int64).reshape(-1, 2)
+        self.n_anc = np.bincount(e[:, 1], minlength=n)
+        self.n_desc = np.bincount(e[:, 0], minlength=n)
+        # spanning forest: a node's tree parent is its ancestor with the most ancestors (always a direct parent),
+        # ties to the larger id as in Hierarchy.from_closure_edges
+        o = np.lexsort((self.n_anc[e[:, 0]], e[:, 1]))
+        u, v = e[o, 0], e[o, 1]
+        last = np.r_[v[1:] != v[:-1], True] if len(v) else np.zeros(0, dtype=bool)
+        parents = np.full(n, -1, dtype=np.int64)
+        parents[v[last]] = u[last]
+        self.parents = parents
+        self.tin = Hierarchy(parents).tin
+        # every node's own number and its descendants' numbers, in order per node, cut into maximal runs; a run is
+        # also cut before tin[u], so the run that starts there is the primary interval and the rest are extra
+        a = np.concatenate([e[:, 0], np.arange(n)])
+        t = np.concatenate([self.tin[e[:, 1]], self.tin])
+        o = np.lexsort((t, a))
+        a, t = a[o], t[o]
+        first = np.r_[True, (a[1:] != a[:-1]) | (t[1:] != t[:-1] + 1)] | (t == self.tin[a])
+        s = np.flatnonzero(first)
+        owner, lo, hi = a[s], t[s], t[np.r_[s[1:] - 1, len(t) - 1]]
+        primary = lo == self.tin[owner]
+        self.tout = np.empty(n, dtype=np.int64)
+        self.tout[owner[primary]] = hi[primary]
+        x = ~primary
+        self.extra_ptr = np.r_[0, np.cumsum(np.bincount(owner[x], minlength=n))].astype(np.int32)
+        self.extra_lo = lo[x].astype(np.int32)
+        self.extra_hi = hi[x].astype(np.int32)
+        self._extra_key = owner[x] * self.n + lo[x]   # sorted: owner, then lo
+
+    @classmethod
+    def from_closure_edges(cls, n, edges, levels=None):
+        """From (ancestor, descendant) pairs in any order -- the reference's G_tc edge list (order_embeddings.py:371).
+        Raises ValueError for an endpoint outside [0, n), a self edge or a set that is not transitively closed (in a
+        closed set a cycle implies a self edge)."""
+        e, k = _edge_array(n, edges, "closure edge")
+        if len(e) and not np.all(_in_sorted(_compose(e, e, n), k)):
+            raise ValueError("the edges are not transitively closed")
+        return cls(n, e, levels)
+
+    @classmethod
+    def from_parents(cls, n, edges, levels=None):
+        """From direct (parent, child) edges; the closure is computed here.  Raises ValueError for an endpoint outside
+        [0, n), a self edge or a cycle."""
+        direct, known = _edge_array(n, edges, "parent edge")
+        frontier = direct
+        while len(frontier):   # pairs joined by a path of one more edge; a cycle shows up as a pair (u, u)
+            k = np.unique(_compose(frontier, direct, n))
+            if np.any(k // n == k % n):
+                raise ValueError("the parent edges contain a cycle")
+            k = k[~_in_sorted(k, known)]
+            known = np.union1d(known, k)
+            frontier = np.stack([k // n, k % n], axis=1)
+        return cls(n, np.stack([known // n, known % n], axis=1), levels)
+
+    def is_descendant(self, u, v):
+        """v is a strict descendant of u (vectorised, broadcasting)."""
+        u, v = np.broadcast_arrays(np.asarray(u, dtype=np.int64), np.asarray(v, dtype=np.int64))
+        tv = self.tin[v]
+        below = (tv > self.tin[u]) & (tv <= self.tout[u])
+        if len(self.extra_lo):
+            i = np.searchsorted(self._extra_key, u * self.n + tv, side="right") - 1   # last extra run starting <= tv
+            below |= (i >= self.extra_ptr[u]) & (tv <= self.extra_hi[np.maximum(i, 0)])
+        return below
+
+    def closure_edges(self):
+        """All (ancestor, descendant) pairs, sorted like Hierarchy.closure_edges."""
+        return self._edges.copy()
 
 
 def ethec():
@@ -156,3 +287,35 @@ def random_tree(n, gamma, seed=0, roots=8):
     parents[1:] = np.minimum(parents[1:], np.arange(1, n) - 1)
     parents[:roots] = -1
     return Hierarchy(parents)
+
+
+def random_dag(n, gamma, frac, seed=0, roots=8):
+    """random_tree(n, gamma, seed, roots) plus, for each non-root node with probability frac, a second parent drawn
+    uniformly from the lower ids that are not already its ancestors (WordNet-like multiple inheritance; edges still
+    point from lower to higher ids, so the graph is acyclic).  frac = 0 gives random_tree's closure."""
+    par = random_tree(n, gamma, seed, roots).parents
+    rng = np.random.default_rng([seed, 1])
+    second = {}
+    for i in np.flatnonzero(rng.random(n) < frac):
+        i = int(i)
+        if i < roots:
+            continue
+        anc, stack = set(), [int(par[i])]   # lower ids only: their parents are final
+        while stack:
+            a = stack.pop()
+            if a < 0 or a in anc:
+                continue
+            anc.add(a)
+            stack.append(int(par[a]))
+            stack.append(second.get(a, -1))
+        if len(anc) >= i:
+            continue
+        while True:
+            j = int(rng.integers(0, i))
+            if j not in anc:
+                break
+        second[i] = j
+    has = np.flatnonzero(par >= 0)
+    edges = np.concatenate([np.stack([par[has], has], axis=1),
+                            np.array(sorted((p, c) for c, p in second.items()), dtype=np.int64).reshape(-1, 2)])
+    return DagHierarchy.from_parents(n, edges)

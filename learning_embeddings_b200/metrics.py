@@ -54,17 +54,18 @@ def recon_args(rows, tin, tout, geom, K, D, u_begin, u_end, workspace):
 
 def reconstruction_f1(rows, hierarchy, geom, K, D=None, group=None, workspace_bytes=None, stats=None):
     """check_graph_embedding (order_embeddings.py:512-559 = oe.py:1923-1990) without materialising the n (n-1)
-    energies: positives are E(x = rows[u], y = rows[v]) for every v below u in `hierarchy` (a hierarchy.Hierarchy),
-    negatives every other ordered pair u != v, and the result is best_f1_sweep's numpy row (f1, threshold, accuracy,
-    precision, recall, correct_positives, correct_negatives) over those energies, bit for bit, with the energies of
-    the fp32 SIMT scoring kernel (lec_recon_pass / lec_recon_finish).
+    energies: positives are E(x = rows[u], y = rows[v]) for every v below u in `hierarchy` (a hierarchy.Hierarchy or
+    DagHierarchy), negatives every other ordered pair u != v, and the result is best_f1_sweep's numpy row (f1,
+    threshold, accuracy, precision, recall, correct_positives, correct_negatives) over those energies, bit for bit, with
+    the energies of the fp32 SIMT scoring kernel (lec_recon_pass / lec_recon_finish; lec_recon_pass_dag when a
+    DagHierarchy has extra intervals).
 
     rows: device fp32 [n, ld] -- a plain [n, D] table or an engine's padded rows (ConeStep.rows with D = ConeStep.D).
     group: a torch.distributed group whose ranks each evaluate a contiguous share of the apex rows on their own GPU
     (every rank passes the same rows); the counters are summed after every round, so every rank returns the row.
     workspace_bytes: device workspace, lec_recon_workspace_bytes(RECON_OPEN_BINS) by default; a smaller one costs
     rounds, not exactness.  stats: a dict that receives the rounds run, the open coarse bins, the numbers of positive
-    and negative pairs and the workspace size."""
+    and negative pairs, the workspace size and the number of extra intervals (0 for a forest)."""
     N.require_cuda(rows)
     if rows.dim() != 2 or rows.dtype != torch.float32:
         raise N.LecError("reconstruction_f1: rows must be a float32 [n, ld] tensor")
@@ -83,6 +84,11 @@ def reconstruction_f1(rows, hierarchy, geom, K, D=None, group=None, workspace_by
     lib = N.lib()
     tin = torch.as_tensor(np.asarray(hierarchy.tin), dtype=torch.int32).to(dev)
     tout = torch.as_tensor(np.asarray(hierarchy.tout), dtype=torch.int32).to(dev)
+    n_extra = int(hierarchy.extra_ptr[-1]) if hasattr(hierarchy, "extra_ptr") else 0
+    if n_extra:
+        xptr, xlo, xhi = (torch.as_tensor(np.asarray(a), dtype=torch.int32).to(dev)
+                          for a in (hierarchy.extra_ptr, hierarchy.extra_lo, hierarchy.extra_hi))
+        x = N.LecReconExtra(xptr.data_ptr(), xlo.data_ptr(), xhi.data_ptr(), n_extra)
     nb = int(lib.lec_recon_workspace_bytes(RECON_OPEN_BINS)) if workspace_bytes is None else int(workspace_bytes)
     cb = int(lib.lec_recon_counter_bytes(nb))
     if cb < 0:
@@ -98,7 +104,10 @@ def reconstruction_f1(rows, hierarchy, geom, K, D=None, group=None, workspace_by
     stream = N.stream_ptr(dev)
     rounds = 0
     while True:
-        N.check(lib.lec_recon_pass(ctypes.byref(r), stream), "lec_recon_pass")
+        if n_extra:
+            N.check(lib.lec_recon_pass_dag(ctypes.byref(r), ctypes.byref(x), stream), "lec_recon_pass_dag")
+        else:
+            N.check(lib.lec_recon_pass(ctypes.byref(r), stream), "lec_recon_pass")
         rounds += 1
         if group is not None:
             dist.all_reduce(ws[:cb].view(torch.int64), group=group)
@@ -109,7 +118,8 @@ def reconstruction_f1(rows, hierarchy, geom, K, D=None, group=None, workspace_by
         if rounds > open_bins + 1:   # each fine round retires at least one open bin
             raise N.LecError("lec_recon_finish asks for round %d with %d open bins" % (rounds + 1, open_bins))
     if stats is not None:
-        stats.update(rounds=rounds, open_bins=open_bins, n_pos=n_pos, n_neg=n_neg, workspace_bytes=nb)
+        stats.update(rounds=rounds, open_bins=open_bins, n_pos=n_pos, n_neg=n_neg, workspace_bytes=nb,
+                     extra_intervals=n_extra)
     return out.cpu().numpy()
 
 

@@ -5,7 +5,9 @@ materialised path (SIMT score matrix + torch.sort + lec_f1_sweep) in the same ru
     python scripts/recon_bench.py [--reps 5] [--warmup 2] [--out FILE]
 
 Workloads: ETHEC hyp D = 10 after training (the reference's own size), random tree n = 20 000 D = 50 (A/B), cfg4 tree
-n = 82 115 D = 50 after 2 000 ConeStep steps (no other path fits).  One JSON line per workload.
+n = 82 115 D = 50 after 2 000 ConeStep steps (no other path fits), and the cfg4-sized DAG random_dag(82 115, 1.0831,
+0.02) D = 50 after as many steps (WordNet's nouns have several parents per node; lec_recon_pass_dag).  One JSON line
+per workload.
 """
 import argparse
 import json
@@ -34,14 +36,15 @@ def gpu_info():
     return {"gpu": name, "power_limit": power, "max_sm_clock": clock}
 
 
-def pass_kernel_sass(DH, NT):
-    """Static instructions of the innermost loop of score_fast_kernel<HYP, DH, ., NT, 1, EPI = 1> (the tile loop,
-    unrolled twice: 2 labels x RI images per trip) from cuobjdump -sass of the built object."""
+def pass_kernel_sass(DH, NT, EPI=1):
+    """Static instructions of the tile loop of score_fast_kernel<HYP, DH, ., NT, 1, EPI> (unrolled twice: 2 labels x RI
+    images per trip) from cuobjdump -sass of the built object.  With EPI = 2 the loop holds, per label, the
+    block-uniform branch of apexes with extra intervals and its binary-search loop, summarised separately."""
     obj = os.path.join(ROOT, "learning_embeddings_b200", "csrc", "build", "lec_recon.o")
     sass = subprocess.run(["cuobjdump", "-sass", obj], capture_output=True, text=True).stdout
     sym = "_ZN3lec17score_fast_kernelILi1ELi%dELi" % DH
     blocks = sass.split("Function : ")
-    body = next(b for b in blocks if b.startswith(sym) and b.split("\n", 1)[0].endswith("ELi%dELi1ELi1EEEvNS_8FastArgsE" % NT))
+    body = next(b for b in blocks if b.startswith(sym) and b.split("\n", 1)[0].endswith("ELi%dELi1ELi%dEEEvNS_8FastArgsE" % (NT, EPI)))
     ins = []
     for line in body.splitlines():
         m = re.match(r"\s+/\*([0-9a-f]{4,})\*/\s+(.*?);", line)
@@ -53,11 +56,31 @@ def pass_kernel_sass(DH, NT):
         m = re.search(r"\bBRA\b.*?(0x[0-9a-f]+)", t)
         if m and int(m.group(1), 16) < a and int(m.group(1), 16) in addr:
             loops.append((addr[int(m.group(1), 16)], i))
-    inner = [(s, e) for s, e in loops if not any(s <= s2 and e2 <= e and (s2, e2) != (s, e) for s2, e2 in loops)]
-    s, e = max(inner, key=lambda se: sum("FFMA2" in ins[k][1] for k in range(se[0], se[1] + 1)))
+    ffma2 = lambda se: sum("FFMA2" in ins[k][1] for k in range(se[0], se[1] + 1))  # noqa: E731
+    # innermost among the loops that do arithmetic (EPI = 2's search loops hold no FFMA2 and sit inside the tile loop)
+    inner = [(s, e) for s, e in loops
+             if not any(s <= s2 and e2 <= e and (s2, e2) != (s, e) and ffma2((s2, e2)) for s2, e2 in loops)]
+    s, e = max(inner, key=ffma2)
     body = [t for _, t in ins[s:e + 1]]
-    return {"loop_instructions": len(body), "ffma2": sum("FFMA2" in t for t in body),
-            "mufu": sum("MUFU" in t for t in body), "atomics": sum(("ATOM" in t or "RED" in t) for t in body)}
+    rec = {"loop_instructions": len(body), "ffma2": sum("FFMA2" in t for t in body),
+           "mufu": sum("MUFU" in t for t in body), "atomics": sum(("ATOM" in t or "RED" in t) for t in body)}
+    if EPI == 2:
+        search = [(s2, e2) for s2, e2 in loops if s <= s2 and e2 <= e and (s2, e2) != (s, e)]
+        rec["search_loops"] = len(search)
+        rec["search_loop_instructions"] = [e2 - s2 + 1 for s2, e2 in search]
+        rec["search_loop_loads"] = [sum("LDG" in ins[k][1] for k in range(s2, e2 + 1)) for s2, e2 in search]
+        # the branch that an apex without extra intervals jumps over: the nearest forward BRA before each search loop
+        # whose target lies past it; what is left of the loop is the fast path every other apex runs
+        skipped = 0
+        for s2, e2 in search:
+            for b in range(s2 - 1, s - 1, -1):
+                m = re.search(r"\bBRA\b.*?(0x[0-9a-f]+)", ins[b][1])
+                if m and int(m.group(1), 16) in addr and addr[int(m.group(1), 16)] > e2:
+                    skipped += addr[int(m.group(1), 16)] - b - 1
+                    break
+        rec["branch_instructions"] = skipped
+        rec["fast_path_instructions"] = len(body) - skipped
+    return rec
 
 
 def hyp_rows(h, D, seed=0):
@@ -115,14 +138,17 @@ def workload(name, h, rows, D, args, info, sass, ab=False):
     pairs = n * (n - 1)
     passes = stats["rounds"]
     RI = 4 if (D + 1) // 2 <= 8 else 2
-    per_pair = sass["loop_instructions"] / (2 * RI)            # one trip: 2 labels x RI images per thread
+    # one trip: 2 labels x RI images per thread; for a DAG the fast path (apexes with extra intervals, a few percent,
+    # also run the skipped branch: the bound leaves that out)
+    per_pair = sass.get("fast_path_instructions", sass["loop_instructions"]) / (2 * RI)
     clk = float(info["max_sm_clock"].split()[0]) * 1e6
     bound_ms = passes * pairs * per_pair / 32 / (148 * 4 * clk) * 1e3   # 4 warp instructions per clock per SM
     rec = {"workload": name, "n": n, "D": D, "pairs": pairs, **info, **t, "rounds": passes,
            "open_bins": stats["open_bins"], "n_pos": stats["n_pos"], "n_neg": stats["n_neg"],
            "workspace_mb": stats["workspace_bytes"] / 2**20, "pairs_per_s": pairs / (t["median_ms"] * 1e-3),
            "pair_evals_per_s": passes * pairs / (t["median_ms"] * 1e-3), "pass_loop_sass": sass,
-           "sass_instr_per_pair": per_pair, "issue_bound_ms": bound_ms, "row": [float(v) for v in row]}
+           "sass_instr_per_pair": per_pair, "issue_bound_ms": bound_ms, "extra_intervals": stats["extra_intervals"],
+           "row": [float(v) for v in row]}
     if ab:
         torch.cuda.empty_cache()
         ref, tm = timed(lambda: materialised(rows, h, D), args.reps, args.warmup)
@@ -153,6 +179,11 @@ def main():
     h = H.random_tree(82115, 1.0831)
     rows, D = trained(h, 50, args.cfg4_steps)
     lines.append(workload("cfg4_hyp_D50_trained%d" % args.cfg4_steps, h, rows, D, args, info, sass50))
+    h = H.random_dag(82115, 1.0831, 0.02)
+    rows, D = trained(h, 50, args.cfg4_steps)
+    lines.append(workload("cfg4dag002_hyp_D50_trained%d" % args.cfg4_steps, h, rows, D, args, info,
+                          pass_kernel_sass(25, 256, EPI=2)))
+    lines[-1]["pair_evals_per_s_vs_cfg4_tree"] = lines[-1]["pair_evals_per_s"] / lines[-2]["pair_evals_per_s"]
     out = open(args.out, "w") if args.out else None
     for rec in lines:
         s = json.dumps(rec)
