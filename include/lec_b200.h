@@ -468,6 +468,44 @@ typedef struct lec_recon_extra {
 int lec_recon_pass_dag(const lec_recon_t* r, const lec_recon_extra_t* x, void* stream);
 int lec_recon_finish(const lec_recon_t* r, double* out7, int64_t* status, void* stream);
 
+/* Reconstruction mean rank and MAP (Nickel & Kiela's filtered ranking) over the pairs of lec_recon_*: apex u, other
+ * endpoint v, every ordered pair u != v, energy E(x = rows[u], y = rows[v]) with the fp32 bits of the
+ * lec_score_topk_ex(..., LEC_PREC_F32, ...) matrix; positive iff v is a strict descendant of u in the cover (tin / tout,
+ * plus extra intervals when extra != NULL and extra->count != 0, as lec_recon_pass_dag), negative otherwise.
+ *   key(u, v)   the energy's fp32 bits, -0 counted as 0, every NaN one value ordered after +inf
+ *   per closure edge (u, v), neg(u) = the negatives of apex u (other positives of u are not counted):
+ *     rank_opt  = 1 + #{w in neg(u) : key(u, w) <  key(u, v)}
+ *     rank_pess = 1 + #{w in neg(u) : key(u, w) <= key(u, v)}
+ *   per apex with P_u >= 1 positives, average precision with tied keys grouped (sklearn's average_precision_score of
+ *   -E): AP_u = sum over the distinct positive keys t of (#pos with key t) / P_u * TP(<= t) / (TP(<= t) + FP(<= t)),
+ *   computed in fp64 in a fixed order (two calls give the same bits)
+ * Positive slots: v's slot under u is tin[v] - tin[u] - 1 inside the primary interval, then u's extra intervals in
+ * order; pos_ptr[u] + slot is the pair's index in [0, n_pos).
+ *   pos_ptr        device int64[n+1]: prefix of the strict descendant counts P_u, pos_ptr[n] = n_pos <= INT32_MAX;
+ *                  it must agree with the cover
+ *   u_begin/u_end  the apexes this call evaluates (a rank's share); only those with P_u >= 1 are visited
+ *   workspace      device, 16-byte aligned, >= lec_rank_workspace_bytes(n, n_pos); needs no initialisation
+ *   stage_ms       HOST float[4] or NULL: when set, the call times its stages (positive keys, sort, count, finish) with
+ *                  events and synchronises the stream
+ * lec_rank_run writes rank_sums (device int64[3]) = {sum rank_opt, sum rank_pess, negatives at or below their apex's
+ * largest positive key} over the closure edges of the visited apexes, ap[u] (device fp64[n]) for every visited apex
+ * (other entries are untouched) and, when ranks != NULL, ranks[j] = {rank_opt, rank_pess} (device int32[n_pos][2]) for
+ * the slots j of the visited apexes.  It neither allocates nor synchronises (unless stage_ms is set).
+ * lec_rank_workspace_bytes returns the size, a negative LEC_E_* for bad counts, or -e for a CUDA error e of the sort's
+ * size query (which may need a device). */
+typedef struct lec_rank {
+    int geom; float K;
+    const float* rows; int64_t n; int D; int ld;          /* as lec_recon_t, D 1..64 */
+    const int32_t* tin; const int32_t* tout;
+    const lec_recon_extra_t* extra;                       /* NULL: a forest */
+    const int64_t* pos_ptr; int64_t n_pos;
+    int64_t u_begin, u_end;
+    void* workspace; int64_t workspace_bytes;
+    float* stage_ms;
+} lec_rank_t;
+int64_t lec_rank_workspace_bytes(int64_t n, int64_t n_pos);
+int lec_rank_run(const lec_rank_t* r, int64_t* rank_sums, double* ap, int32_t* ranks, void* stream);
+
 /* lec_classify_counts replaces the per-image bookkeeping of JointEmbeddings.calculate_classification_metrics
  * (oe.py:1775-1796, oe_h.py:2030-2051) on the output of lec_score_topk*.
  *   topk_idx  device int32 [n_img, n_levels, k]   truth  device int32 [n_img, n_levels] (true label per level, < 0: skip)

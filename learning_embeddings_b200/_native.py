@@ -26,6 +26,7 @@ EXPORTS = (
     "lec_sample_negatives", "lec_sample_negatives_philox", "lec_philox_below", "lec_f1_workspace_bytes", "lec_f1_sweep",
     "lec_classify_counts", "lec_caption_hinge",
     "lec_recon_workspace_bytes", "lec_recon_counter_bytes", "lec_recon_pass", "lec_recon_pass_dag", "lec_recon_finish",
+    "lec_rank_workspace_bytes", "lec_rank_run",
     "lec_host_pipe_create", "lec_host_pipe_destroy", "lec_host_pipe_submit", "lec_host_pipe_wait",
 )
 
@@ -94,6 +95,19 @@ class LecRecon(ctypes.Structure):
 class LecReconExtra(ctypes.Structure):
     """lec_recon_extra_t of include/lec_b200.h."""
     _fields_ = [("ptr", ctypes.c_void_p), ("lo", ctypes.c_void_p), ("hi", ctypes.c_void_p), ("count", ctypes.c_int64)]
+
+
+class LecRank(ctypes.Structure):
+    """lec_rank_t of include/lec_b200.h."""
+    _fields_ = [
+        ("geom", ctypes.c_int), ("K", ctypes.c_float),
+        ("rows", ctypes.c_void_p), ("n", ctypes.c_int64), ("D", ctypes.c_int), ("ld", ctypes.c_int),
+        ("tin", ctypes.c_void_p), ("tout", ctypes.c_void_p), ("extra", ctypes.POINTER(LecReconExtra)),
+        ("pos_ptr", ctypes.c_void_p), ("n_pos", ctypes.c_int64),
+        ("u_begin", ctypes.c_int64), ("u_end", ctypes.c_int64),
+        ("workspace", ctypes.c_void_p), ("workspace_bytes", ctypes.c_int64),
+        ("stage_ms", ctypes.POINTER(ctypes.c_float)),
+    ]
 
 
 UPD_NONE, UPD_RSGD, UPD_SGD, UPD_ADAM = 0, 1, 2, 3
@@ -170,6 +184,9 @@ def lib():
         L.lec_recon_pass.argtypes = [ctypes.POINTER(LecRecon), c_vp]
         L.lec_recon_pass_dag.argtypes = [ctypes.POINTER(LecRecon), ctypes.POINTER(LecReconExtra), c_vp]
         L.lec_recon_finish.argtypes = [ctypes.POINTER(LecRecon), c_vp, c_vp, c_vp]
+        L.lec_rank_workspace_bytes.argtypes = [c_i64, c_i64]
+        L.lec_rank_workspace_bytes.restype = c_i64
+        L.lec_rank_run.argtypes = [ctypes.POINTER(LecRank), c_vp, c_vp, c_vp, c_vp]
         L.lec_caption_hinge.argtypes = [c_vp, c_vp, c_i64, c_i, c_f, c_vp, c_vp, c_vp, c_vp, c_vp]
         L.lec_host_pipe_create.argtypes = [ctypes.POINTER(c_vp), c_i]
         L.lec_host_pipe_destroy.argtypes = [c_vp]

@@ -56,6 +56,11 @@ struct FastArgs {
     unsigned long long* rhdr; unsigned long long* rhist;
     // DAG reconstruction pass (EPI = 2): apex u's extra preorder intervals [xlo[i], xhi[i]], i in [xptr[u], xptr[u+1])
     const int32_t* xptr; const int32_t* xlo; const int32_t* xhi;
+    // reconstruction ranks (EPI = 3 positive keys, EPI = 4 negative counts, lec_rank.cu): block chunks index the apex
+    // list rapex[0, *rnapex); apex u's positives own slots [rpos[u], rpos[u+1]); rxcum[i] = slots of u's primary interval
+    // and of its extra intervals before i
+    const int32_t* rapex; const int* rnapex; const int64_t* rpos; const int32_t* rxcum;
+    unsigned* rkey; int32_t* rval; const unsigned* rsorted; unsigned* rcnt; unsigned* req;
 };
 
 // Reconstruction check (lec_recon.cu).  Key of an energy = its fp32 bit pattern (energies are >= 0 or NaN, -0 is
@@ -71,6 +76,16 @@ struct ReconState {
     double best_f1; unsigned long long best_cp, best_cn; unsigned best_key; int has_best;
 };
 
+// Reconstruction ranks (lec_rank.cu).  Rank key of an energy: its fp32 bits, -0 counted as 0, every NaN one value
+// after +inf.  A staged tile counts the negatives of its apexes in up to kRankShared shared buckets {count, equal}
+// (16 bits each: at most NT * RI images per block add to a bucket before the tile's flush); larger apexes count in
+// global memory.
+constexpr int kRankShared = 16384;
+__device__ __forceinline__ unsigned rank_key(float e) {
+    const unsigned k = __float_as_uint(e);
+    return e != e ? 0x7fc00000u : (k == 0x80000000u ? 0u : k);
+}
+
 // Shared-memory layout of one staged label: DQ float4 chunks of the row (zero padded), then one float4
 // of constants.   hyp: {A, 1+A, A^2, -psi} {cos psi, sin psi, 0, 0}   euc: {A, t0, 0, 0}   oe: unused
 // Label values enter the packed FMAs as scalar-broadcast operands (FFMA2 takes a .F32 operand that
@@ -84,6 +99,9 @@ struct IntC {
 
 // EPI = 1: the reconstruction pass -- the same energies, counted into the lec_recon.cu histograms instead of stored
 // EPI = 2: the same pass on a DAG: a pair is also positive when tin[v] lies in one of the apex's extra intervals
+// EPI = 3: reconstruction ranks, the rank key of every positive pair into its slot (forest or DAG)
+// EPI = 4: reconstruction ranks, every negative pair at or below its apex's largest positive key into the bucket of its
+//          lower bound among the apex's sorted positive keys
 template <int GEOM, int DH, int RI, int NT, int MINB, int EPI = 0>
 __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) {
     static_assert(RI % 2 == 0, "images are packed in pairs");
@@ -101,7 +119,11 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     const int seg = (int)(blockIdx.x / a.groups);
     const int64_t group = blockIdx.x % a.groups;
     const int l_begin = EPI ? (int)(a.u_begin + (int64_t)seg * a.chunk) : a.seg_start[seg];
-    const int l_end = EPI ? (int)min(a.u_end, a.u_begin + (int64_t)(seg + 1) * a.chunk) : a.seg_stop[seg];
+    const int l_end = EPI ? (int)min(EPI >= 3 ? (int64_t)*a.rnapex : a.u_end, a.u_begin + (int64_t)(seg + 1) * a.chunk)
+                          : a.seg_stop[seg];
+    if (EPI >= 3 && l_begin >= l_end) return;  // the grid is sized for every apex row, the list holds those with P_u >= 1
+    // row of staged label l: the apex list indexes the rows in the rank passes
+    auto label_row = [&](int l) -> int64_t { return EPI >= 3 ? (int64_t)a.rapex[l] : (int64_t)l; };
     const int level = EPI ? -1 : a.seg_level[seg];
     const bool want_topk = (level >= 0) && (a.topk_idx != nullptr);
     const int k = a.k;
@@ -149,7 +171,24 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     int rphase = 0;
     int tin_v[RI];
     unsigned c_np = 0, c_nn = 0, c_nanp = 0, c_nann = 0, c_zp = 0, c_zn = 0;
-    if (EPI) {
+    // rank passes: per staged apex {first slot, P_u, smallest and largest sorted positive key}, {first extra interval,
+    // count}, the first shared bucket (-1: global counters) and the prefix the flush searches; then the buckets
+    int4* rsk = reinterpret_cast<int4*>(smem + kTileLabels * LS);
+    int2* rxs = reinterpret_cast<int2*>(rsk + kTileLabels);
+    int* rso = reinterpret_cast<int*>(rxs + kTileLabels);
+    int* rpre = rso + kTileLabels;
+    int* rused = rpre + kTileLabels;
+    unsigned* rbk = reinterpret_cast<unsigned*>(rused + 4);
+    if (EPI >= 3) {
+#pragma unroll
+        for (int r = 0; r < RI; ++r) {
+            const int64_t v = img0 + r * NT;
+            tin_v[r] = v < a.N ? a.tin[v] : 0;
+        }
+        if (EPI == 4)
+            for (int b = tid; b < kRankShared; b += NT) rbk[b] = 0u;
+    }
+    if (EPI == 1 || EPI == 2) {
         rphase = a.rstate->phase;
         if (rphase == 2) return;
 #pragma unroll
@@ -466,6 +505,92 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                     const int64_t v = img0 + r * NT;
                     recon_count(E[r], v < a.N && v != u, pos[r]);
                 }
+            } else if (STORE == 5 || STORE == 6) {
+                const int* ue = reinterpret_cast<const int*>(lab + t * LS + 4 * DQ + 6);
+                const int tin_u = ue[0], tout_u = ue[1];
+                const int4 rk = rsk[t];  // {first slot, P_u, smallest key, largest key}
+                bool pos[RI];
+                int slot[RI];
+#pragma unroll
+                for (int r = 0; r < RI; ++r) {
+                    pos[r] = img0 + r * NT < a.N && tin_u < tin_v[r] && tin_v[r] <= tout_u;
+                    slot[r] = tin_v[r] - tin_u - 1;
+                }
+                const int2 xe = rxs[t];
+                if (xe.y > 0) {  // block-uniform: EPI = 2's search of the apex's extra intervals
+                    int below[RI];
+#pragma unroll
+                    for (int r = 0; r < RI; ++r) below[r] = 0;
+                    for (int s = 1 << (31 - __clz(xe.y)); s > 0; s >>= 1) {
+#pragma unroll
+                        for (int r = 0; r < RI; ++r) {
+                            const int i = below[r] + s;
+                            if (i <= xe.y && __ldg(a.xlo + xe.x + i - 1) <= tin_v[r]) below[r] = i;
+                        }
+                    }
+#pragma unroll
+                    for (int r = 0; r < RI; ++r) {
+                        const int i = xe.x + below[r] - 1;
+                        if (img0 + r * NT < a.N && below[r] > 0 && tin_v[r] <= __ldg(a.xhi + i)) {
+                            pos[r] = true;
+                            if (STORE == 5) slot[r] = __ldg(a.rxcum + i) + tin_v[r] - __ldg(a.xlo + i);
+                        }
+                    }
+                }
+                if (STORE == 5) {
+#pragma unroll
+                    for (int r = 0; r < RI; ++r) {
+                        if (pos[r] && slot[r] < rk.y) {  // a slot past P_u would mean pos_ptr disagrees with the cover
+                            const int j = rk.x + slot[r];
+                            a.rkey[j] = rank_key(E[r]);
+                            a.rval[j] = j;
+                        }
+                    }
+                } else {
+                    unsigned key[RI];
+                    bool neg[RI], srch = false;
+                    int lb[RI];
+#pragma unroll
+                    for (int r = 0; r < RI; ++r) {
+                        key[r] = rank_key(E[r]);
+                        neg[r] = img0 + r * NT < a.N && tin_v[r] != tin_u && !pos[r] && key[r] <= (unsigned)rk.w;
+                        lb[r] = 0;
+                        srch |= neg[r] && key[r] > (unsigned)rk.z;
+                    }
+                    // lower bound among the sorted positive keys: the same ceil(log2(P_u + 1)) steps in every lane
+                    const unsigned* sk = a.rsorted + rk.x;
+                    if (__any_sync(0xffffffffu, srch)) {
+                        for (int s = 1 << (31 - __clz(rk.y)); s > 0; s >>= 1) {
+#pragma unroll
+                            for (int r = 0; r < RI; ++r) {
+                                const int i = lb[r] + s;
+                                if (neg[r] && i <= rk.y && __ldg(sk + i - 1) < key[r]) lb[r] = i;
+                            }
+                        }
+                    }
+                    const int so = rso[t];
+                    if (so >= 0) {  // block-uniform
+#pragma unroll
+                        for (int r = 0; r < RI; ++r)
+                            if (neg[r]) atomicAdd(rbk + so + lb[r], __ldg(sk + lb[r]) == key[r] ? 0x10001u : 1u);
+                    } else {
+                        // equal buckets of a warp are added once, as in the fine round of the F1 pass
+#pragma unroll
+                        for (int r = 0; r < RI; ++r) {
+                            const int tag = neg[r] ? rk.x + lb[r] : -1;
+                            const bool eq = neg[r] && __ldg(sk + lb[r]) == key[r];
+                            if (__any_sync(0xffffffffu, tag >= 0)) {
+                                const unsigned peers = __match_any_sync(0xffffffffu, tag);
+                                const unsigned eqm = __ballot_sync(0xffffffffu, eq);
+                                if (tag >= 0 && (int)(tid & 31) == __ffs(peers) - 1) {
+                                    atomicAdd(a.rcnt + tag, (unsigned)__popc(peers));
+                                    const int ne = __popc(peers & eqm);
+                                    if (ne) atomicAdd(a.req + tag, (unsigned)ne);
+                                }
+                            }
+                        }
+                    }
+                }
             }
             if (TOPK) {
 #pragma unroll
@@ -488,12 +613,12 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         // ---- stage the tile: rows zero-padded to whole float4 chunks
         for (int i = tid; i < tl * 4 * DQ; i += NT) {
             const int t = i / (4 * DQ), d = i - t * (4 * DQ);
-            lab[t * LS + d] = (d < D) ? __ldg(a.labels + (int64_t)(l0 + t) * (EPI ? a.ld : (int64_t)D) + d) : 0.f;
+            lab[t * LS + d] = (d < D) ? __ldg(a.labels + label_row(l0 + t) * (EPI ? a.ld : (int64_t)D) + d) : 0.f;
         }
         // ---- per-label constants in fp64 (same terms as lec_rows_fwd's aux)
         if (GEOM != LEC_GEOM_OE) {
             for (int t = tid; t < tl; t += NT) {
-                const float* src = a.labels + (int64_t)(l0 + t) * (EPI ? a.ld : (int64_t)D);
+                const float* src = a.labels + label_row(l0 + t) * (EPI ? a.ld : (int64_t)D);
                 double A = 0.0;
                 for (int d = 0; d < D; ++d) { const double v = (double)__ldg(src + d); A += v * v; }
                 const Aux<double> x = row_aux<double>(GEOM, A, a.K);
@@ -512,15 +637,61 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         if (EPI) {  // the apex's Euler interval in the last two constant slots (after the stores above, same thread)
             for (int t = tid; t < tl; t += NT) {
                 int* ue = reinterpret_cast<int*>(lab + t * LS + 4 * DQ + 6);
-                ue[0] = a.tin[l0 + t];
-                ue[1] = a.tout[l0 + t];
+                if (EPI < 3) {
+                    ue[0] = a.tin[l0 + t];
+                    ue[1] = a.tout[l0 + t];
+                }
                 if (EPI == 2) {
                     const int x0 = a.xptr[l0 + t];
                     xsh[t] = make_int2(x0, a.xptr[l0 + t + 1] - x0);
                 }
+                if (EPI >= 3) {
+                    const int64_t u = label_row(l0 + t);
+                    ue[0] = a.tin[u];
+                    ue[1] = a.tout[u];
+                    const int x0 = a.xptr ? a.xptr[u] : 0;
+                    rxs[t] = make_int2(x0, a.xptr ? a.xptr[u + 1] - x0 : 0);
+                    const int base = (int)a.rpos[u], P = (int)(a.rpos[u + 1] - base);
+                    rsk[t] = EPI == 4 ? make_int4(base, P, (int)a.rsorted[base], (int)a.rsorted[base + P - 1])
+                                      : make_int4(base, P, 0, 0);
+                }
             }
         }
         __syncthreads();
+        if (EPI == 4) {
+            // shared buckets for the tile's apexes in order while their P_u sum stays within kRankShared; an apex
+            // larger than that, and every apex after the budget is spent, counts in global memory
+            if (tid < 32) {
+                static_assert(kTileLabels == 3 * 32, "three staged apexes per lane");
+                int s[3], loc = 0;
+#pragma unroll
+                for (int j = 0; j < 3; ++j) {
+                    const int t = 3 * tid + j;
+                    const int P = t < tl ? rsk[t].y : 0;
+                    s[j] = P <= kRankShared ? P : 0;
+                    loc += s[j];
+                }
+                int inc = loc;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const int y = __shfl_up_sync(0xffffffffu, inc, o);
+                    if (tid >= o) inc += y;
+                }
+                int pre = inc - loc, used = 0;
+#pragma unroll
+                for (int j = 0; j < 3; ++j) {
+                    const int t = 3 * tid + j;
+                    const bool fits = s[j] > 0 && pre + s[j] <= kRankShared;
+                    if (t < tl) { rpre[t] = pre; rso[t] = fits ? pre : -1; }
+                    if (fits) used = pre + s[j];
+                    pre += s[j];
+                }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) used = max(used, __shfl_xor_sync(0xffffffffu, used, o));
+                if (tid == 0) *rused = used;
+            }
+            __syncthreads();
+        }
         if (GEOM == LEC_GEOM_HYP && want_topk && store == 0) {
             if (tid < 32) {
                 float mx = -INFINITY;
@@ -532,7 +703,27 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
             __syncthreads();
             refresh_filter();
         }
-        if (EPI) {
+        if (EPI >= 3) {
+            tile_loop(l0, tl, IntC<EPI == 4 ? 6 : 5>(), IntC<0>());
+            if (EPI == 4) {  // flush the tile's non-zero buckets and clear them for the next tile
+                __syncthreads();
+                const int used = *rused;
+                for (int i = tid; i < used; i += NT) {
+                    const unsigned c = rbk[i];
+                    if (!c) continue;
+                    rbk[i] = 0u;
+                    int lo = 0, hi = tl - 1;  // owner: the last staged apex whose buckets start at or before i
+                    while (lo < hi) {
+                        const int mid = (lo + hi + 1) >> 1;
+                        if (rpre[mid] <= i) lo = mid;
+                        else hi = mid - 1;
+                    }
+                    const int g = rsk[lo].x + (i - rpre[lo]);
+                    atomicAdd(a.rcnt + g, c & 0xffffu);
+                    if (c >> 16) atomicAdd(a.req + g, c >> 16);
+                }
+            }
+        } else if (EPI) {
             tile_loop(l0, tl, IntC<EPI == 2 ? 4 : 3>(), IntC<0>());
         } else if (want_topk) {
             if (store == 0 && GEOM == LEC_GEOM_HYP) tile_loop_deferred(l0, tl);
@@ -545,6 +736,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         }
     }
 
+    if (EPI >= 3) return;
     if (EPI) {
         // register counters: one global add per warp; then the block's coarse negatives
 #pragma unroll

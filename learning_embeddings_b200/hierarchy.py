@@ -24,6 +24,35 @@ class _Closure:
             self.level_start = [int(v) for v in stops - np.asarray(self.levels)]
             self.level_stop = [int(v) for v in stops]
 
+    def rank_slots(self):
+        """(pos_ptr, slot_of_edge) of the reconstruction ranks (metrics.reconstruction_ranks), computed once.  Apex u's
+        positives own the slots [pos_ptr[u], pos_ptr[u+1]) (pos_ptr: int64 [n+1], the prefix of n_desc); v's slot
+        under u is tin[v] - tin[u] - 1 inside u's primary interval, then u's extra intervals follow in order.
+        slot_of_edge[i] (int64 [n_edges]) is the slot of closure_edges()[i]: a permutation of [0, n_edges)."""
+        if getattr(self, "_rank_slots", None) is None:
+            pos_ptr = np.r_[0, np.cumsum(np.asarray(self.n_desc, dtype=np.int64))].astype(np.int64)
+            if pos_ptr[-1] == 0:   # no edge (Hierarchy.closure_edges needs one)
+                self._rank_slots = (pos_ptr, np.zeros(0, dtype=np.int64))
+                return self._rank_slots
+            e = self.closure_edges()
+            u, v = e[:, 0], e[:, 1]
+            tin, tout = np.asarray(self.tin, dtype=np.int64), np.asarray(self.tout, dtype=np.int64)
+            tv = tin[v]
+            s = tv - tin[u] - 1
+            lo = getattr(self, "extra_lo", None)
+            if lo is not None and len(lo):
+                lo = lo.astype(np.int64)
+                size = self.extra_hi.astype(np.int64) - lo + 1
+                first = self.extra_ptr[:-1].astype(np.int64)
+                owner = np.repeat(np.arange(self.n), np.diff(self.extra_ptr))
+                before = np.cumsum(size) - size                              # sizes of all earlier extra intervals
+                xcum = (tout - tin)[owner] + before - before[first[owner]]   # slots of owner's cover before interval i
+                out = ~((tv > tin[u]) & (tv <= tout[u]))
+                i = np.searchsorted(self._extra_key, u[out] * self.n + tv[out], side="right") - 1
+                s[out] = xcum[i] + tv[out] - lo[i]
+            self._rank_slots = (pos_ptr, pos_ptr[u] + s)
+        return self._rank_slots
+
     def negative_adjacency(self):
         """Dense bool matrix of the reference (ones - closure - diagonal); only sensible for small n."""
         A = np.ones((self.n, self.n), dtype=bool)

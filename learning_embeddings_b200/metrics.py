@@ -7,6 +7,7 @@ formulas, which the reference evaluates on Python ints, are evaluated here on Py
 reference's order, so every reported number is the same float.
 """
 import ctypes
+import math
 
 import numpy as np
 import torch
@@ -121,6 +122,110 @@ def reconstruction_f1(rows, hierarchy, geom, K, D=None, group=None, workspace_by
         stats.update(rounds=rounds, open_bins=open_bins, n_pos=n_pos, n_neg=n_neg, workspace_bytes=nb,
                      extra_intervals=n_extra)
     return out.cpu().numpy()
+
+
+RANK_SHARED_BUCKETS = 16384   # kRankShared of csrc/lec_score_fast_impl.cuh: a larger apex counts in global memory
+
+
+def rank_args(rows, tin, tout, extra, pos_ptr, n_pos, geom, K, D, u_begin, u_end, workspace, stage_ms=None):
+    """lec_rank_t for device rows [n, >= D] (fp32, unit column stride), device int32 tin / tout [n], an optional
+    LecReconExtra (None: a forest), device int64 pos_ptr [n+1] and a device workspace tensor; apexes [u_begin, u_end)."""
+    r = N.LecRank()
+    r.geom, r.K = N.GEOM[geom], float(K or 0.0)
+    r.rows, r.n, r.D, r.ld = rows.data_ptr(), rows.shape[0], int(D), rows.stride(0)
+    r.tin, r.tout = tin.data_ptr(), tout.data_ptr()
+    if extra is not None:
+        r.extra = ctypes.pointer(extra)
+    r.pos_ptr, r.n_pos = pos_ptr.data_ptr(), int(n_pos)
+    r.u_begin, r.u_end = int(u_begin), int(u_end)
+    r.workspace, r.workspace_bytes = workspace.data_ptr(), workspace.numel() * workspace.element_size()
+    if stage_ms is not None:
+        r.stage_ms = stage_ms
+    return r
+
+
+def reconstruction_ranks(rows, hierarchy, geom, K, D=None, group=None, return_ranks=False, stats=None,
+                         time_stages=False):
+    """Mean rank and mean average precision of the reconstruction check (Nickel & Kiela, Poincaré embeddings; the
+    numbers the hyperbolic-embedding literature reports for WordNet nouns) over the pairs of reconstruction_f1, without
+    materialising the n (n-1) energies (lec_rank_run).  For each closure edge (u, v) the rank of v among the negatives
+    of apex u (every w != u that is not below u) by the fp32 energy of the SIMT scoring kernel; other positives of u
+    are not counted ("filtered" ranks).  Ties: rank_opt counts the negatives with a smaller key, rank_pess those with a
+    smaller or equal one (key = the energy's fp32 bits, -0 as 0, NaN after +inf); the reference's unstable argsort
+    lands in between.  AP_u groups tied keys like sklearn's average_precision_score(labels, -E).
+
+    rows: device fp32 [n, ld] -- a plain [n, D] table or an engine's padded rows (ConeStep.rows with D = ConeStep.D).
+    hierarchy: a hierarchy.Hierarchy or DagHierarchy.
+    group: a torch.distributed group whose ranks each evaluate a contiguous share of the apexes on their own GPU (every
+    rank passes the same rows); the per-apex results are disjoint, so summing them is exact, and every rank returns
+    the result.
+    Returns a dict: mean_rank (pessimistic ties, the headline: trained cones put many pairs at exactly E = 0),
+    mean_rank_optimistic, map (math.fsum of AP_u over the n_apexes apexes with a descendant), n_edges, n_apexes and
+    ap (numpy fp64 [n], NaN where u has no descendant); with return_ranks also ranks, device int32 [n_edges, 2]
+    (optimistic, pessimistic) in hierarchy.closure_edges() order.  Without edges the three means are NaN.
+    stats: a dict that receives the workspace size, the negatives at or below their apex's largest positive key (the
+    ones that reach the count) and, with time_stages (which synchronises after each call), the four stage times in ms."""
+    N.require_cuda(rows)
+    if rows.dim() != 2 or rows.dtype != torch.float32:
+        raise N.LecError("reconstruction_ranks: rows must be a float32 [n, ld] tensor")
+    n = rows.shape[0]
+    D = rows.shape[1] if D is None else int(D)
+    if n != hierarchy.n:
+        raise ValueError("reconstruction_ranks: %d rows for a hierarchy of %d nodes" % (n, hierarchy.n))
+    if D > rows.shape[1]:
+        raise ValueError("reconstruction_ranks: D = %d exceeds the row width %d" % (D, rows.shape[1]))
+    rows = rows.detach()
+    if rows.stride(1) != 1 or (rows.stride(0) != D and rows.stride(0) % 4 != 0) or rows.data_ptr() % 16 != 0:
+        rows = rows[:, :D].contiguous()
+    dev = rows.device
+    lib = N.lib()
+    pos_ptr_h, slot_of_edge = hierarchy.rank_slots()
+    n_edges = int(pos_ptr_h[-1])
+    has = np.diff(pos_ptr_h) > 0
+    n_apexes = int(has.sum())
+    tin = torch.as_tensor(np.asarray(hierarchy.tin), dtype=torch.int32).to(dev)
+    tout = torch.as_tensor(np.asarray(hierarchy.tout), dtype=torch.int32).to(dev)
+    pos_ptr = torch.as_tensor(pos_ptr_h, dtype=torch.int64).to(dev)
+    n_extra = int(hierarchy.extra_ptr[-1]) if hasattr(hierarchy, "extra_ptr") else 0
+    x = None
+    if n_extra:
+        xptr, xlo, xhi = (torch.as_tensor(np.asarray(a), dtype=torch.int32).to(dev)
+                          for a in (hierarchy.extra_ptr, hierarchy.extra_lo, hierarchy.extra_hi))
+        x = N.LecReconExtra(xptr.data_ptr(), xlo.data_ptr(), xhi.data_ptr(), n_extra)
+    nb = int(lib.lec_rank_workspace_bytes(n, n_edges))
+    if nb < 0:
+        N.check(int(nb), "lec_rank_workspace_bytes")
+    ws = torch.empty(nb, device=dev, dtype=torch.uint8)
+    rank, world = 0, 1
+    if group is not None:
+        import torch.distributed as dist
+        rank, world = dist.get_rank(group), dist.get_world_size(group)
+    stage_ms = (ctypes.c_float * 4)() if time_stages else None
+    r = rank_args(rows, tin, tout, x, pos_ptr, n_edges, geom, K, D, n * rank // world, n * (rank + 1) // world, ws,
+                  stage_ms)
+    sums = torch.zeros(3, device=dev, dtype=torch.int64)
+    ap = torch.zeros(n, device=dev, dtype=torch.float64)
+    ranks = torch.zeros((n_edges, 2), device=dev, dtype=torch.int32) if return_ranks else None
+    N.check(lib.lec_rank_run(ctypes.byref(r), N._p(sums), N._p(ap), N._p(ranks), N.stream_ptr(dev)), "lec_rank_run")
+    if group is not None:
+        for t in (sums, ap) if ranks is None else (sums, ap, ranks):
+            dist.all_reduce(t, group=group)
+    s_opt, s_pess, counted = (int(v) for v in sums.cpu())
+    ap = ap.cpu().numpy()
+    ap[~has] = np.nan
+    if n_edges:
+        out = {"mean_rank": s_pess / n_edges, "mean_rank_optimistic": s_opt / n_edges,
+               "map": math.fsum(ap[has].tolist()) / n_apexes}
+    else:
+        out = {"mean_rank": math.nan, "mean_rank_optimistic": math.nan, "map": math.nan}
+    out.update(n_edges=n_edges, n_apexes=n_apexes, ap=ap)
+    if ranks is not None:
+        out["ranks"] = ranks[torch.as_tensor(slot_of_edge, device=dev)]
+    if stats is not None:
+        stats.update(workspace_bytes=nb, counted_negatives=counted)
+        if time_stages:
+            stats["stage_ms"] = dict(zip(("keys", "sort", "count", "finish"), (float(v) for v in stage_ms)))
+    return out
 
 
 class EmbeddingMetrics:
