@@ -506,6 +506,42 @@ typedef struct lec_rank {
 int64_t lec_rank_workspace_bytes(int64_t n, int64_t n_pos);
 int lec_rank_run(const lec_rank_t* r, int64_t* rank_sums, double* ap, int32_t* ranks, void* stream);
 
+/* Link prediction on held-out closure edges (Nickel & Kiela's "link prediction", Ganea et al.'s transitive closure
+ * completion): the pairs and energies of lec_recon_* and lec_rank_*, with
+ *   positives  the held-out pairs (u, v), a subset of the closure
+ *   negatives  every ordered pair u != w with w not below u in the FULL closure (as before)
+ *   skipped    the closure pairs that are not held out (the training pairs): neither positive nor negative
+ * A held-out set is given by the closure slots of lec_rank_t (every closure edge, pos_ptr = closure_ptr) and a map from
+ * each closure slot to its held-out slot; held-out slots keep the closure-slot order within each apex, so the held-out
+ * pairs of apex u own [eval_ptr[u], eval_ptr[u+1]) (hierarchy.heldout_slots builds all four arrays).
+ *   closure_ptr  device int64[n+1]: the closure layout; closure_ptr[n] must equal n_closure (not read: that would
+ *                synchronise)
+ *   slot_map     device int32[n_closure]: held-out slot of each closure slot, -1 for a skipped pair
+ *   xcum         device int32[extra count]: slots of an apex's primary interval and of its extra intervals before
+ *                interval i (the closure layout's offsets); needed when the cover has extra intervals, else may be NULL
+ *   n_closure    closure slots, 0..INT32_MAX
+ * lec_rank_run_heldout is lec_rank_run with r->pos_ptr / r->n_pos the held-out layout (eval_ptr, n_pos <= n_closure):
+ * ranks, AP and sums over the held-out pairs, ranks[j] for held-out slot j.  lec_recon_pass_heldout is
+ * lec_recon_pass_dag counting only held-out positives.  With h == NULL each is exactly its counterpart.  A NULL
+ * closure_ptr / slot_map (or xcum with extra intervals) returns LEC_E_NULL; n_closure out of range, n_pos > n_closure or
+ * more extra intervals than n_closure returns LEC_E_SIZE.
+ * lec_recon_finish_at finishes a round of lec_recon_pass* like lec_recon_finish, but writes the row of the fixed
+ * threshold t (EmbeddingMetrics.calculate_metrics, 'test' phase, order_embeddings.py:289-306): correct_positives =
+ * #{positives with E <= t}, correct_negatives = #{negatives with E > t}, precision 0 when nothing is predicted positive,
+ * recall NaN without positives; a NaN energy is never <= t, and a NaN t classifies nothing.  Round 0 counts the coarse
+ * bins below key(t)'s (keys as lec_recon_*, -0 as 0); one fine round opens only the bin that holds key(t), and none when
+ * that bin is empty or t is NaN or negative.  out7[1] is (double)t.  Nothing allocates or synchronises. */
+typedef struct lec_heldout {
+    const int64_t* closure_ptr;  /* [n+1] closure slots per apex (rank_slots' pos_ptr) */
+    const int32_t* slot_map;     /* [n_closure] held-out slot of each closure slot, -1: skipped */
+    const int32_t* xcum;         /* [extra count] as rank_xcum_kernel's, NULL for a forest */
+    int64_t n_closure;
+} lec_heldout_t;
+int lec_rank_run_heldout(const lec_rank_t* r, const lec_heldout_t* h, int64_t* rank_sums, double* ap,
+                         int32_t* ranks, void* stream);   /* r->pos_ptr / n_pos: the held-out layout */
+int lec_recon_pass_heldout(const lec_recon_t* r, const lec_recon_extra_t* x, const lec_heldout_t* h, void* stream);
+int lec_recon_finish_at(const lec_recon_t* r, float threshold, double* out7, int64_t* status, void* stream);
+
 /* lec_classify_counts replaces the per-image bookkeeping of JointEmbeddings.calculate_classification_metrics
  * (oe.py:1775-1796, oe_h.py:2030-2051) on the output of lec_score_topk*.
  *   topk_idx  device int32 [n_img, n_levels, k]   truth  device int32 [n_img, n_levels] (true label per level, < 0: skip)

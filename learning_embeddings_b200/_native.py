@@ -26,7 +26,7 @@ EXPORTS = (
     "lec_sample_negatives", "lec_sample_negatives_philox", "lec_philox_below", "lec_f1_workspace_bytes", "lec_f1_sweep",
     "lec_classify_counts", "lec_caption_hinge",
     "lec_recon_workspace_bytes", "lec_recon_counter_bytes", "lec_recon_pass", "lec_recon_pass_dag", "lec_recon_finish",
-    "lec_rank_workspace_bytes", "lec_rank_run",
+    "lec_rank_workspace_bytes", "lec_rank_run", "lec_rank_run_heldout", "lec_recon_pass_heldout", "lec_recon_finish_at",
     "lec_host_pipe_create", "lec_host_pipe_destroy", "lec_host_pipe_submit", "lec_host_pipe_wait",
 )
 
@@ -110,6 +110,12 @@ class LecRank(ctypes.Structure):
     ]
 
 
+class LecHeldout(ctypes.Structure):
+    """lec_heldout_t of include/lec_b200.h."""
+    _fields_ = [("closure_ptr", ctypes.c_void_p), ("slot_map", ctypes.c_void_p), ("xcum", ctypes.c_void_p),
+                ("n_closure", ctypes.c_int64)]
+
+
 UPD_NONE, UPD_RSGD, UPD_SGD, UPD_ADAM = 0, 1, 2, 3
 XCHG_ONE_SHOT, XCHG_TWO_SHOT = 0, 1
 
@@ -187,6 +193,10 @@ def lib():
         L.lec_rank_workspace_bytes.argtypes = [c_i64, c_i64]
         L.lec_rank_workspace_bytes.restype = c_i64
         L.lec_rank_run.argtypes = [ctypes.POINTER(LecRank), c_vp, c_vp, c_vp, c_vp]
+        L.lec_rank_run_heldout.argtypes = [ctypes.POINTER(LecRank), ctypes.POINTER(LecHeldout), c_vp, c_vp, c_vp, c_vp]
+        L.lec_recon_pass_heldout.argtypes = [ctypes.POINTER(LecRecon), ctypes.POINTER(LecReconExtra),
+                                             ctypes.POINTER(LecHeldout), c_vp]
+        L.lec_recon_finish_at.argtypes = [ctypes.POINTER(LecRecon), c_f, c_vp, c_vp, c_vp]
         L.lec_caption_hinge.argtypes = [c_vp, c_vp, c_i64, c_i, c_f, c_vp, c_vp, c_vp, c_vp, c_vp]
         L.lec_host_pipe_create.argtypes = [ctypes.POINTER(c_vp), c_i]
         L.lec_host_pipe_destroy.argtypes = [c_vp]

@@ -1,5 +1,6 @@
 // The best-F1 row of EmbeddingMetrics.calculate_metrics, 'val' phase (order_embeddings.py:272-287 = oe.py:380-395),
-// shared by the sweep over sorted energies (lec_metrics.cu) and the streaming reconstruction check (lec_recon.cu).
+// and its 'test' row at a given threshold, shared by the sweep over sorted energies (lec_metrics.cu) and the streaming
+// reconstruction check (lec_recon.cu).
 #pragma once
 #include <stdint.h>
 
@@ -18,6 +19,16 @@ __device__ __forceinline__ void f1_row(float t, int64_t cp, int64_t cn, int64_t 
     const double acc = (double)(cp + cn) / (double)(n_pos + n_neg);
     const double prec = (double)cp / (double)(cp + (n_neg - cn));   // 0/0 -> NaN (the reference raises ZeroDivisionError)
     const double rec = (double)cp / (double)n_pos;
+    const double f1 = (prec + rec == 0.0) ? 0.0 : (2.0 * prec * rec) / (prec + rec);
+    row[0] = f1; row[1] = (double)t; row[2] = acc; row[3] = prec; row[4] = rec; row[5] = (double)cp; row[6] = (double)cn;
+}
+
+// metrics of a fixed threshold t (EmbeddingMetrics.calculate_metrics, 'test' phase, order_embeddings.py:289-306): the
+// same counts and expression tree, except that a threshold without a predicted positive has precision 0, not 0/0
+__device__ __forceinline__ void f1_row_at(float t, int64_t cp, int64_t cn, int64_t n_pos, int64_t n_neg, double* row) {
+    const double acc = (double)(cp + cn) / (double)(n_pos + n_neg);
+    const double prec = cp + (n_neg - cn) == 0 ? 0.0 : (double)cp / (double)(cp + (n_neg - cn));
+    const double rec = (double)cp / (double)n_pos;   // no positive: 0/0 -> NaN (the reference raises ZeroDivisionError)
     const double f1 = (prec + rec == 0.0) ? 0.0 : (2.0 * prec * rec) / (prec + rec);
     row[0] = f1; row[1] = (double)t; row[2] = acc; row[3] = prec; row[4] = rec; row[5] = (double)cp; row[6] = (double)cn;
 }

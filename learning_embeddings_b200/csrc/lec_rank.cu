@@ -9,6 +9,9 @@
 //            when it equals sorted[b], to eq[b], where b is its lower bound among the apex's sorted keys
 //   finish   per apex: rank_pess = 1 + prefix(cnt) at the slot, rank_opt = rank_pess - eq[first slot of its tie group],
 //            AP_u in fp64 in a fixed order
+// On a held-out set (lec_rank_run_heldout) pos_ptr is the held-out layout and the key pass is EPI = 7: it finds each
+// positive's closure slot as EPI = 3 does and writes the key to the held-out slot the slot map gives, or nowhere.  Sort,
+// count and finish run unchanged: the count already leaves out every closure pair, held out or not.
 //
 // Workspace (caller-owned, needs no initialisation; each region 256-byte aligned):
 //   napex (int) | apex list int32[n] | xcum int32[n_pos] | keys, slot ids in and out (4 x 4 B x n_pos) |
@@ -232,7 +235,8 @@ int rank_launch(int geom, FastArgs& a, cudaStream_t st) {
     }
 }
 
-int validate(const lec_rank_t* r, const int64_t* rank_sums, const double* ap) {
+// n_slots: the positives an extra interval may hold (n_pos, or the closure's on a held-out set)
+int validate(const lec_rank_t* r, const int64_t* rank_sums, const double* ap, int64_t n_slots) {
     if (!r || !r->rows || !r->tin || !r->tout || !r->pos_ptr || !r->workspace || !rank_sums || !ap) return LEC_E_NULL;
     if (r->D < 1 || r->D > 64 || r->ld < r->D || (r->ld != r->D && r->ld % 4 != 0)) return LEC_E_DIM;
     if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE) return LEC_E_ENUM;
@@ -241,7 +245,7 @@ int validate(const lec_rank_t* r, const int64_t* rank_sums, const double* ap) {
         return LEC_E_SIZE;
     const lec_recon_extra_t* x = r->extra;
     if (x && x->count != 0) {
-        if (x->count < 0 || x->count > r->n_pos) return LEC_E_SIZE;  // an extra interval holds at least one positive
+        if (x->count < 0 || x->count > n_slots) return LEC_E_SIZE;  // an extra interval holds at least one positive
         if (!x->ptr || !x->lo || !x->hi) return LEC_E_NULL;
     }
     if ((reinterpret_cast<uintptr_t>(r->rows) & 15) || (reinterpret_cast<uintptr_t>(r->workspace) & 15)) return LEC_E_ALIGN;
@@ -260,10 +264,15 @@ extern "C" int64_t lec_rank_workspace_bytes(int64_t n, int64_t n_pos) {
     return (int64_t)(rank_layout(nullptr, n, n_pos).fixed + al256(temp));
 }
 
-extern "C" int lec_rank_run(const lec_rank_t* r, int64_t* rank_sums, double* ap, int32_t* ranks, void* stream) {
+extern "C" int lec_rank_run_heldout(const lec_rank_t* r, const lec_heldout_t* h, int64_t* rank_sums, double* ap,
+                                    int32_t* ranks, void* stream) {
     using namespace lec;
-    const int err = validate(r, rank_sums, ap);
+    int err = validate(r, rank_sums, ap, h ? h->n_closure : r ? r->n_pos : 0);
     if (err) return err;
+    if (h) {
+        if ((err = heldout_validate(h, r->extra && r->extra->count != 0))) return err;
+        if (r->n_pos > h->n_closure) return LEC_E_SIZE;
+    }
     const RankLayout l = rank_layout(r->workspace, r->n, r->n_pos);
     size_t temp = 0;
     cudaError_t e = sort_temp_bytes(r->u_end - r->u_begin, r->n_pos, temp);
@@ -291,7 +300,7 @@ extern "C" int lec_rank_run(const lec_rank_t* r, int64_t* rank_sums, double* ap,
         mark(0);
         rank_apex_kernel<<<1, kRankPrepThreads, 0, st>>>(r->pos_ptr, r->u_begin, r->u_end, l.apex, l.napex);
         ++g_launches;
-        if (x) {
+        if (x && !h) {
             rank_xcum_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>(r->tin, r->tout, x->ptr, x->lo, x->hi, r->u_begin,
                                                                         r->u_end, l.xcum);
             ++g_launches;
@@ -301,9 +310,10 @@ extern "C" int lec_rank_run(const lec_rank_t* r, int64_t* rank_sums, double* ap,
         a.ld = r->ld; a.u_begin = 0; a.u_end = rows;
         a.tin = r->tin; a.tout = r->tout;
         if (x) { a.xptr = x->ptr; a.xlo = x->lo; a.xhi = x->hi; }
-        a.rapex = l.apex; a.rnapex = l.napex; a.rpos = r->pos_ptr; a.rxcum = l.xcum;
+        a.rapex = l.apex; a.rnapex = l.napex; a.rpos = r->pos_ptr; a.rxcum = h ? h->xcum : l.xcum;
         a.rkey = l.key_in; a.rval = l.val_in; a.rsorted = l.key_out; a.rcnt = l.cnt; a.req = l.eq;
-        rc = rank_launch<3>(r->geom, a, st);
+        if (h) { a.hptr = h->closure_ptr; a.hmap = h->slot_map; }
+        rc = h ? rank_launch<7>(r->geom, a, st) : rank_launch<3>(r->geom, a, st);
         if (rc) return rc;
         mark(1);
         size_t tb = temp;
@@ -331,4 +341,8 @@ extern "C" int lec_rank_run(const lec_rank_t* r, int64_t* rank_sums, double* ap,
         }
     }
     return 0;
+}
+
+extern "C" int lec_rank_run(const lec_rank_t* r, int64_t* rank_sums, double* ap, int32_t* ranks, void* stream) {
+    return lec_rank_run_heldout(r, nullptr, rank_sums, ap, ranks, stream);
 }

@@ -4,7 +4,8 @@
 //
 // The energies are the SIMT scoring kernel's (score_fast_kernel with EPI = 1: same per-pair instructions, so the same
 // bits as the lec_score_topk_ex matrix), classified by the Euler intervals and counted, never stored (EPI = 2,
-// lec_recon_pass_dag: a DAG's interval cover, the Euler-like primary interval plus each apex's extra intervals):
+// lec_recon_pass_dag: a DAG's interval cover, the Euler-like primary interval plus each apex's extra intervals; EPI = 5, 6,
+// lec_recon_pass_heldout: positives only where the closure slot is held out, other closure pairs skipped):
 //   round 0      every pair's key (fp32 bits; energies are >= 0 or NaN) into 2 x 32 768 coarse bins (key >> 16)
 //   select       exact F1 at each coarse bin's largest value gives a lower bound LB on the best F1; a bin can
 //                only hold a better threshold if 2 CP_b / (n_pos + CP_b + FP_{b-1}) >= LB (1 - 1e-12) -- the slack
@@ -12,6 +13,8 @@
 //   round k      the energies again; pairs in the open bins are counted per exact key (65 536 fine bins each)
 //   finish       every distinct value of the open bins is a threshold with exact cp / cn: lec_f1.cuh's f1_row,
 //                first arg-max, carried across rounds when more bins are open than the workspace holds
+// At a fixed threshold t (lec_recon_finish_at) round 0 gives the counts below key(t)'s coarse bin and one fine round,
+// with only that bin open, the counts inside it up to key(t).
 //
 // Workspace (caller-owned, zeroed once before round 0):
 //   [counters]  8 x u64 header {n_pos, n_neg, NaN positives, NaN negatives} + batch x 2 x 65 536 u64 histogram
@@ -251,12 +254,80 @@ __global__ void __launch_bounds__(kSelThreads) recon_merge_kernel(ReconState* __
     }
 }
 
+// fixed threshold t (lec_recon_finish_at) after round 0: the finite pairs in the coarse bins below key(t)'s; that bin is
+// opened for one fine round unless it is empty or t decides every pair by itself (NaN, below 0); one block
+__global__ void __launch_bounds__(kSelThreads) recon_at_select_kernel(const u64c* __restrict__ hdr, const u64c* __restrict__ hist,
+                                                                      ReconState* __restrict__ s, ReconOpen* __restrict__ open,
+                                                                      int64_t batch, float t, double* __restrict__ out7,
+                                                                      long long* __restrict__ status) {
+    constexpr int PER = kReconBins / kSelThreads;
+    if (s->phase != 0) return;
+    const int tid = threadIdx.x;
+    const u64c n_pos = hdr[0], n_neg = hdr[1], nan_neg = hdr[3];
+    const unsigned bits = __float_as_uint(t);
+    const bool nan_t = t != t, neg_t = !nan_t && bits > 0x80000000u;  // -0 is 0
+    const int bin = nan_t || neg_t ? 0 : (int)((bits & 0x7fffffffu) >> kReconShift);
+    const u64c* hp = hist;
+    const u64c* hn = hist + kReconBins;
+    u64c sp = 0, sn = 0;
+    for (int j = 0; j < PER; ++j) {
+        const int b = tid * PER + j;
+        if (b < bin) { sp += hp[b]; sn += hn[b]; }
+    }
+    u64c cp, fp;
+    block_exclusive_scan<u64c, kSelThreads>(sp, cp);
+    block_exclusive_scan<u64c, kSelThreads>(sn, fp);   // finite negatives below the bin
+    if (tid == 0) {
+        const bool fine = !nan_t && !neg_t && (hp[bin] | hn[bin]) != 0;
+        s->n_pos = n_pos; s->n_neg = n_neg; s->nan_pos = hdr[2]; s->nan_neg = nan_neg;
+        s->batch = batch; s->n_open = fine; s->next = 0; s->m = fine;
+        s->phase = fine ? 1 : 2;
+        s->has_best = 0;
+        status[0] = fine; status[1] = fine; status[2] = (long long)n_pos; status[3] = (long long)n_neg;
+        if (fine) open[0] = ReconOpen{(uint32_t)bin, 0u, cp, fp};
+        else if (nan_t) f1_row_at(t, 0, 0, (int64_t)n_pos, (int64_t)n_neg, out7);   // no comparison with NaN holds
+        else f1_row_at(t, (int64_t)cp, (int64_t)(n_neg - nan_neg - fp), (int64_t)n_pos, (int64_t)n_neg, out7);
+    }
+}
+
+// fixed threshold, fine round: the exact values of key(t)'s coarse bin up to key(t); one block
+__global__ void __launch_bounds__(kSelThreads) recon_at_fine_kernel(const u64c* __restrict__ hist, ReconState* __restrict__ s,
+                                                                    const ReconOpen* __restrict__ open, float t,
+                                                                    double* __restrict__ out7, long long* __restrict__ status) {
+    constexpr int PER = kReconFine / kSelThreads;
+    const int tid = threadIdx.x;
+    const int phase = s->phase;
+    if (phase != 1) {
+        if (phase == 2 && tid == 0) { status[0] = 0; status[1] = s->n_open; status[2] = (long long)s->n_pos; status[3] = (long long)s->n_neg; }
+        return;
+    }
+    const int low = (int)(__float_as_uint(t) & 0x7fffffffu & (kReconFine - 1));   // t is >= 0 here; -0 is 0
+    const u64c* h = hist;   // batch slot 0: [fine][negative, positive]
+    u64c sp = 0, sn = 0;
+    for (int j = 0; j < PER; ++j) {
+        const int f = tid * PER + j;
+        if (f <= low) { sp += h[2 * f + 1]; sn += h[2 * f]; }
+    }
+    u64c cp, fp;
+    block_exclusive_scan<u64c, kSelThreads>(sp, cp);
+    block_exclusive_scan<u64c, kSelThreads>(sn, fp);
+    if (tid == 0) {
+        const ReconOpen o = open[0];
+        const ReconState st = *s;
+        cp += o.cp_below;
+        fp += o.fp_below;
+        f1_row_at(t, (int64_t)cp, (int64_t)(st.n_neg - st.nan_neg - fp), (int64_t)st.n_pos, (int64_t)st.n_neg, out7);
+        s->next = 1; s->m = 0; s->phase = 2;
+        status[0] = 0; status[1] = 1; status[2] = (long long)st.n_pos; status[3] = (long long)st.n_neg;
+    }
+}
+
 template <int GEOM, int DH, int RI, int EPI>
 int recon_launch_dh(FastArgs& a, cudaStream_t st) {
     constexpr int NT = recon_threads<DH>();
     constexpr int LS = 4 * ((DH + 1) / 2) + 8;
     const size_t smem = (size_t)kTileLabels * LS * sizeof(float) + (size_t)kReconBins * sizeof(unsigned) +
-                        (EPI == 2 ? (size_t)kTileLabels * sizeof(int2) : 0);
+                        (EPI == 2 || EPI == 6 ? (size_t)kTileLabels * sizeof(int2) : 0);
     static bool configured = false;
     if (!configured) {
         cudaError_t e = cudaFuncSetAttribute(score_fast_kernel<GEOM, DH, RI, NT, 1, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -315,7 +386,8 @@ extern "C" int64_t lec_recon_counter_bytes(int64_t workspace_bytes) {
     return b < 1 ? (int64_t)LEC_E_SIZE : lec::counter_bytes_of(b);
 }
 
-extern "C" int lec_recon_pass_dag(const lec_recon_t* r, const lec_recon_extra_t* x, void* stream) {
+extern "C" int lec_recon_pass_heldout(const lec_recon_t* r, const lec_recon_extra_t* x, const lec_heldout_t* h,
+                                      void* stream) {
     using namespace lec;
     const int err = validate(r);
     if (err) return err;
@@ -323,6 +395,11 @@ extern "C" int lec_recon_pass_dag(const lec_recon_t* r, const lec_recon_extra_t*
     if (dag) {
         if (x->count < 0 || x->count > 0x7fffffffLL) return LEC_E_SIZE;
         if (!x->ptr || !x->lo || !x->hi) return LEC_E_NULL;
+    }
+    if (h) {
+        const int herr = heldout_validate(h, dag);
+        if (herr) return herr;
+        if (dag && x->count > h->n_closure) return LEC_E_SIZE;   // an extra interval holds at least one closure pair
     }
     if (r->u_end == r->u_begin) return 0;
     const Layout l = layout(r->workspace, r->workspace_bytes);
@@ -332,6 +409,22 @@ extern "C" int lec_recon_pass_dag(const lec_recon_t* r, const lec_recon_extra_t*
     a.tin = r->tin; a.tout = r->tout;
     a.rstate = l.state; a.ropen = l.open; a.rhdr = l.hdr; a.rhist = l.hist;
     cudaStream_t st = (cudaStream_t)stream;
+    if (h) {  // only pairs below their apex look up the slot map
+        a.hptr = h->closure_ptr; a.hmap = h->slot_map;
+        if (dag) {
+            a.xptr = x->ptr; a.xlo = x->lo; a.xhi = x->hi; a.rxcum = h->xcum;
+            switch (r->geom) {
+                case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 6>(a, st);
+                case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 6>(a, st);
+                default: return recon_launch_geom<LEC_GEOM_OE, 6>(a, st);
+            }
+        }
+        switch (r->geom) {
+            case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 5>(a, st);
+            case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 5>(a, st);
+            default: return recon_launch_geom<LEC_GEOM_OE, 5>(a, st);
+        }
+    }
     if (dag) {  // only apexes with extra intervals leave the forest kernel's instructions
         a.xptr = x->ptr; a.xlo = x->lo; a.xhi = x->hi;
         switch (r->geom) {
@@ -345,6 +438,10 @@ extern "C" int lec_recon_pass_dag(const lec_recon_t* r, const lec_recon_extra_t*
         case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 1>(a, st);
         default: return recon_launch_geom<LEC_GEOM_OE, 1>(a, st);
     }
+}
+
+extern "C" int lec_recon_pass_dag(const lec_recon_t* r, const lec_recon_extra_t* x, void* stream) {
+    return lec_recon_pass_heldout(r, x, nullptr, stream);
 }
 
 extern "C" int lec_recon_pass(const lec_recon_t* r, void* stream) {
@@ -368,4 +465,22 @@ extern "C" int lec_recon_finish(const lec_recon_t* r, double* out7, int64_t* sta
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return (int)e;
     return (int)cudaMemsetAsync(r->workspace, 0, (size_t)l.counter_bytes, st);   // the next pass adds to zero
+}
+
+extern "C" int lec_recon_finish_at(const lec_recon_t* r, float threshold, double* out7, int64_t* status, void* stream) {
+    using namespace lec;
+    const int err = validate(r);
+    if (err) return err;
+    if (!out7 || !status) return LEC_E_NULL;
+    const Layout l = layout(r->workspace, r->workspace_bytes);
+    cudaStream_t st = (cudaStream_t)stream;
+    // as lec_recon_finish: the fine-round kernel returns at once unless the fine round is being finished, the round-0
+    // kernel unless round 0 is
+    recon_at_fine_kernel<<<1, kSelThreads, 0, st>>>(l.hist, l.state, l.open, threshold, out7, reinterpret_cast<long long*>(status));
+    recon_at_select_kernel<<<1, kSelThreads, 0, st>>>(l.hdr, l.hist, l.state, l.open, l.batch, threshold, out7,
+                                                       reinterpret_cast<long long*>(status));
+    g_launches += 2;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return (int)e;
+    return (int)cudaMemsetAsync(r->workspace, 0, (size_t)l.counter_bytes, st);
 }

@@ -61,6 +61,10 @@ struct FastArgs {
     // and of its extra intervals before i
     const int32_t* rapex; const int* rnapex; const int64_t* rpos; const int32_t* rxcum;
     unsigned* rkey; int32_t* rval; const unsigned* rsorted; unsigned* rcnt; unsigned* req;
+    // held-out evaluation (EPI = 5, 6 F1 pass, EPI = 7 rank keys): apex u's closure pairs own the closure slots
+    // [hptr[u], hptr[u+1]) (the layout of rpos for every closure edge, extra intervals offset by rxcum); hmap[j] is the
+    // held-out slot of closure slot j, -1 for a pair that is neither positive nor negative
+    const int64_t* hptr; const int32_t* hmap;
 };
 
 // Reconstruction check (lec_recon.cu).  Key of an energy = its fp32 bit pattern (energies are >= 0 or NaN, -0 is
@@ -102,9 +106,14 @@ struct IntC {
 // EPI = 3: reconstruction ranks, the rank key of every positive pair into its slot (forest or DAG)
 // EPI = 4: reconstruction ranks, every negative pair at or below its apex's largest positive key into the bucket of its
 //          lower bound among the apex's sorted positive keys
+// EPI = 5, 6: EPI = 1, 2 on a held-out set: a pair below its apex is positive only when its closure slot is held out
+//          and is skipped otherwise (only those pairs look the slot up); negatives are those of EPI = 1, 2
+// EPI = 7: EPI = 3 on a held-out set: the key of a held-out pair into its held-out slot hmap[closure slot]
 template <int GEOM, int DH, int RI, int NT, int MINB, int EPI = 0>
 __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) {
     static_assert(RI % 2 == 0, "images are packed in pairs");
+    constexpr bool RANK = EPI == 3 || EPI == 4 || EPI == 7;  // rank passes (lec_rank.cu); other EPI > 0: F1 passes
+    constexpr bool XDAG = EPI == 2 || EPI == 6;              // F1 pass with extra intervals
     constexpr int DQ = (DH + 1) / 2;     // float4 chunks per row
     constexpr int LS = 4 * DQ + 8;       // floats per staged label: row chunks + two float4 of constants
     constexpr int NP = RI / 2;           // packed image pairs per thread
@@ -119,11 +128,11 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     const int seg = (int)(blockIdx.x / a.groups);
     const int64_t group = blockIdx.x % a.groups;
     const int l_begin = EPI ? (int)(a.u_begin + (int64_t)seg * a.chunk) : a.seg_start[seg];
-    const int l_end = EPI ? (int)min(EPI >= 3 ? (int64_t)*a.rnapex : a.u_end, a.u_begin + (int64_t)(seg + 1) * a.chunk)
+    const int l_end = EPI ? (int)min(RANK ? (int64_t)*a.rnapex : a.u_end, a.u_begin + (int64_t)(seg + 1) * a.chunk)
                           : a.seg_stop[seg];
-    if (EPI >= 3 && l_begin >= l_end) return;  // the grid is sized for every apex row, the list holds those with P_u >= 1
+    if (RANK && l_begin >= l_end) return;  // the grid is sized for every apex row, the list holds those with P_u >= 1
     // row of staged label l: the apex list indexes the rows in the rank passes
-    auto label_row = [&](int l) -> int64_t { return EPI >= 3 ? (int64_t)a.rapex[l] : (int64_t)l; };
+    auto label_row = [&](int l) -> int64_t { return RANK ? (int64_t)a.rapex[l] : (int64_t)l; };
     const int level = EPI ? -1 : a.seg_level[seg];
     const bool want_topk = (level >= 0) && (a.topk_idx != nullptr);
     const int k = a.k;
@@ -167,7 +176,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     // fraction of a percent of the pairs, go straight to global memory); fine rounds = the batch slot of every coarse
     // bin (or -1) in the same shared array.  Zeros, NaNs and the pair counts stay in registers until the block ends.
     unsigned* rsh = reinterpret_cast<unsigned*>(smem + kTileLabels * LS);
-    int2* xsh = reinterpret_cast<int2*>(rsh + kReconBins);  // EPI = 2: [kTileLabels] {first extra interval, count}
+    int2* xsh = reinterpret_cast<int2*>(rsh + kReconBins);  // EPI = 2, 6: [kTileLabels] {first extra interval, count}
     int rphase = 0;
     int tin_v[RI];
     unsigned c_np = 0, c_nn = 0, c_nanp = 0, c_nann = 0, c_zp = 0, c_zn = 0;
@@ -179,7 +188,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     int* rpre = rso + kTileLabels;
     int* rused = rpre + kTileLabels;
     unsigned* rbk = reinterpret_cast<unsigned*>(rused + 4);
-    if (EPI >= 3) {
+    if (RANK) {
 #pragma unroll
         for (int r = 0; r < RI; ++r) {
             const int64_t v = img0 + r * NT;
@@ -188,7 +197,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         if (EPI == 4)
             for (int b = tid; b < kRankShared; b += NT) rbk[b] = 0u;
     }
-    if (EPI == 1 || EPI == 2) {
+    if (EPI && !RANK) {
         rphase = a.rstate->phase;
         if (rphase == 2) return;
 #pragma unroll
@@ -443,7 +452,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     };
 
     // STORE: 0 no matrix, 1 label-major and every image of the group exists, 2 generic strides / partial group,
-    // 3 reconstruction counts, 4 reconstruction counts with extra intervals (DAG)
+    // 3 reconstruction counts, 4 reconstruction counts with extra intervals (DAG), 5 rank keys, 6 rank counts
     auto tile_loop = [&](int l0, int tl, auto store_c, auto topk_c) {
         constexpr int STORE = decltype(store_c)::value;
         constexpr bool TOPK = decltype(topk_c)::value != 0;
@@ -473,15 +482,24 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
 #pragma unroll
                 for (int r = 0; r < RI; ++r) {
                     const int64_t v = img0 + r * NT;
-                    recon_count(E[r], v < a.N && v != u, tin_u < tin_v[r] && tin_v[r] <= tout_u);
+                    bool valid = v < a.N && v != u;
+                    const bool pos = tin_u < tin_v[r] && tin_v[r] <= tout_u;
+                    // held out: a pair below u loads the held-out slot of its closure slot (ue[-1]: u's first one); a
+                    // training pair is skipped
+                    if (EPI == 5 && valid && pos && __ldg(a.hmap + ue[-1] + tin_v[r] - tin_u - 1) < 0) valid = false;
+                    recon_count(E[r], valid, pos);
                 }
             } else if (STORE == 4) {
                 const int u = l0 + t;
                 const int* ue = reinterpret_cast<const int*>(lab + t * LS + 4 * DQ + 6);
                 const int tin_u = ue[0], tout_u = ue[1];
                 bool pos[RI];
+                int cs[RI];  // EPI = 6: closure slot of a pair below u
 #pragma unroll
-                for (int r = 0; r < RI; ++r) pos[r] = tin_u < tin_v[r] && tin_v[r] <= tout_u;
+                for (int r = 0; r < RI; ++r) {
+                    pos[r] = tin_u < tin_v[r] && tin_v[r] <= tout_u;
+                    if (EPI == 6) cs[r] = ue[-1] + tin_v[r] - tin_u - 1;
+                }
                 const int2 xe = xsh[t];
                 if (xe.y > 0) {  // block-uniform: every thread is on apex u
                     // per image: how many of u's extra intervals start at or before tin_v (binary lifting over the
@@ -496,14 +514,27 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                             if (i <= xe.y && __ldg(a.xlo + xe.x + i - 1) <= tin_v[r]) below[r] = i;
                         }
                     }
+                    if (EPI == 6) {
 #pragma unroll
-                    for (int r = 0; r < RI; ++r)
-                        pos[r] |= below[r] > 0 && tin_v[r] <= __ldg(a.xhi + xe.x + below[r] - 1);
+                        for (int r = 0; r < RI; ++r) {
+                            const int i = xe.x + below[r] - 1;
+                            if (below[r] > 0 && tin_v[r] <= __ldg(a.xhi + i)) {
+                                pos[r] = true;
+                                cs[r] = ue[-1] + __ldg(a.rxcum + i) + tin_v[r] - __ldg(a.xlo + i);
+                            }
+                        }
+                    } else {
+#pragma unroll
+                        for (int r = 0; r < RI; ++r)
+                            pos[r] |= below[r] > 0 && tin_v[r] <= __ldg(a.xhi + xe.x + below[r] - 1);
+                    }
                 }
 #pragma unroll
                 for (int r = 0; r < RI; ++r) {
                     const int64_t v = img0 + r * NT;
-                    recon_count(E[r], v < a.N && v != u, pos[r]);
+                    bool valid = v < a.N && v != u;
+                    if (EPI == 6 && valid && pos[r] && __ldg(a.hmap + cs[r]) < 0) valid = false;  // as EPI = 5
+                    recon_count(E[r], valid, pos[r]);
                 }
             } else if (STORE == 5 || STORE == 6) {
                 const int* ue = reinterpret_cast<const int*>(lab + t * LS + 4 * DQ + 6);
@@ -541,7 +572,8 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
 #pragma unroll
                     for (int r = 0; r < RI; ++r) {
                         if (pos[r] && slot[r] < rk.y) {  // a slot past P_u would mean pos_ptr disagrees with the cover
-                            const int j = rk.x + slot[r];
+                            const int j = EPI == 7 ? __ldg(a.hmap + rk.x + slot[r]) : rk.x + slot[r];
+                            if (EPI == 7 && j < 0) continue;  // a training pair
                             a.rkey[j] = rank_key(E[r]);
                             a.rval[j] = j;
                         }
@@ -637,21 +669,23 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         if (EPI) {  // the apex's Euler interval in the last two constant slots (after the stores above, same thread)
             for (int t = tid; t < tl; t += NT) {
                 int* ue = reinterpret_cast<int*>(lab + t * LS + 4 * DQ + 6);
-                if (EPI < 3) {
+                if (!RANK) {
                     ue[0] = a.tin[l0 + t];
                     ue[1] = a.tout[l0 + t];
                 }
-                if (EPI == 2) {
+                if (EPI == 5 || EPI == 6) ue[-1] = (int)a.hptr[l0 + t];  // the deferred top-k's sin(psi) slot
+                if (XDAG) {
                     const int x0 = a.xptr[l0 + t];
                     xsh[t] = make_int2(x0, a.xptr[l0 + t + 1] - x0);
                 }
-                if (EPI >= 3) {
+                if (RANK) {
                     const int64_t u = label_row(l0 + t);
                     ue[0] = a.tin[u];
                     ue[1] = a.tout[u];
                     const int x0 = a.xptr ? a.xptr[u] : 0;
                     rxs[t] = make_int2(x0, a.xptr ? a.xptr[u + 1] - x0 : 0);
-                    const int base = (int)a.rpos[u], P = (int)(a.rpos[u + 1] - base);
+                    const int64_t* sp = EPI == 7 ? a.hptr : a.rpos;  // EPI = 7 walks the closure slots
+                    const int base = (int)sp[u], P = (int)(sp[u + 1] - base);
                     rsk[t] = EPI == 4 ? make_int4(base, P, (int)a.rsorted[base], (int)a.rsorted[base + P - 1])
                                       : make_int4(base, P, 0, 0);
                 }
@@ -703,7 +737,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
             __syncthreads();
             refresh_filter();
         }
-        if (EPI >= 3) {
+        if (RANK) {
             tile_loop(l0, tl, IntC<EPI == 4 ? 6 : 5>(), IntC<0>());
             if (EPI == 4) {  // flush the tile's non-zero buckets and clear them for the next tile
                 __syncthreads();
@@ -724,7 +758,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 }
             }
         } else if (EPI) {
-            tile_loop(l0, tl, IntC<EPI == 2 ? 4 : 3>(), IntC<0>());
+            tile_loop(l0, tl, IntC<XDAG ? 4 : 3>(), IntC<0>());
         } else if (want_topk) {
             if (store == 0 && GEOM == LEC_GEOM_HYP) tile_loop_deferred(l0, tl);
             else if (store == 0) tile_loop(l0, tl, IntC<0>(), IntC<1>());
@@ -736,7 +770,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         }
     }
 
-    if (EPI >= 3) return;
+    if (RANK) return;
     if (EPI) {
         // register counters: one global add per warp; then the block's coarse negatives
 #pragma unroll
@@ -790,6 +824,15 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
             }
         }
     }
+}
+
+// arguments of a held-out set (lec_rank_run_heldout, lec_recon_pass_heldout); xcum is needed with extra intervals.
+// closure_ptr[n] == n_closure is the caller's to keep, like pos_ptr's agreement with the cover: reading it would
+// synchronise.
+inline int heldout_validate(const lec_heldout_t* h, bool dag) {
+    if (!h->closure_ptr || !h->slot_map || (dag && !h->xcum)) return LEC_E_NULL;
+    if (h->n_closure < 0 || h->n_closure > 0x7fffffffLL) return LEC_E_SIZE;
+    return 0;
 }
 
 // 128-thread blocks whose register allocation need only allow one resident block per SM; a thread holds RI images.

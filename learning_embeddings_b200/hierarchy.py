@@ -31,6 +31,7 @@ class _Closure:
         slot_of_edge[i] (int64 [n_edges]) is the slot of closure_edges()[i]: a permutation of [0, n_edges)."""
         if getattr(self, "_rank_slots", None) is None:
             pos_ptr = np.r_[0, np.cumsum(np.asarray(self.n_desc, dtype=np.int64))].astype(np.int64)
+            self._rank_xcum = None if getattr(self, "extra_lo", None) is None else np.zeros(0, dtype=np.int32)
             if pos_ptr[-1] == 0:   # no edge (Hierarchy.closure_edges needs one)
                 self._rank_slots = (pos_ptr, np.zeros(0, dtype=np.int64))
                 return self._rank_slots
@@ -50,8 +51,34 @@ class _Closure:
                 out = ~((tv > tin[u]) & (tv <= tout[u]))
                 i = np.searchsorted(self._extra_key, u[out] * self.n + tv[out], side="right") - 1
                 s[out] = xcum[i] + tv[out] - lo[i]
+                self._rank_xcum = xcum.astype(np.int32)
             self._rank_slots = (pos_ptr, pos_ptr[u] + s)
         return self._rank_slots
+
+    def heldout_slots(self, edges):
+        """(eval_ptr, slot_map, order, xcum) of link prediction on the held-out closure edges `edges` [m, 2]
+        (metrics.link_prediction_ranks / link_prediction_f1): the held-out pairs keep rank_slots()' order, so apex u's own
+        the held-out slots [eval_ptr[u], eval_ptr[u+1]) (eval_ptr: int64 [n+1]).  slot_map (int32 [n_closure]) is the
+        held-out slot of each closure slot, -1 for a pair that is not held out; order (int64 [m]) the held-out slot of
+        edges[i]; xcum (int32, one per extra interval) the closure slots of an apex before each of its extra intervals,
+        None for a Hierarchy.  Raises ValueError for an endpoint outside [0, n), a pair that is not a closure edge or a
+        repeated pair."""
+        pos_ptr, slot_of_edge = self.rank_slots()
+        e = np.asarray(edges, dtype=np.int64).reshape(-1, 2)
+        if len(e) and (e.min() < 0 or e.max() >= self.n):
+            raise ValueError("held-out edge endpoint outside [0, %d)" % self.n)
+        keys = _edge_keys(e, self.n)
+        if len(np.unique(keys)) != len(keys):
+            raise ValueError("a held-out edge is given twice")
+        ck = _edge_keys(self.closure_edges(), self.n) if len(slot_of_edge) else np.zeros(0, dtype=np.int64)
+        if not np.all(_in_sorted(keys, ck)):
+            raise ValueError("a held-out pair is not a closure edge")
+        cslot = slot_of_edge[np.searchsorted(ck, keys)] if len(keys) else np.zeros(0, dtype=np.int64)
+        held = np.zeros(len(slot_of_edge), dtype=bool)
+        held[cslot] = True
+        before = np.r_[0, np.cumsum(held)].astype(np.int64)   # held-out slots before each closure slot
+        slot_map = np.where(held, before[:-1], -1).astype(np.int32)
+        return before[pos_ptr], slot_map, before[cslot], self._rank_xcum
 
     def negative_adjacency(self):
         """Dense bool matrix of the reference (ones - closure - diagonal); only sensible for small n."""
@@ -298,6 +325,32 @@ class DagHierarchy(_Closure):
     def closure_edges(self):
         """All (ancestor, descendant) pairs, sorted like Hierarchy.closure_edges."""
         return self._edges.copy()
+
+
+def split_edges(h, val=0.05, test=0.05, train_nonbasic=1.0, seed=0):
+    """Link-prediction split of the closure of h (the protocol of create_splits, order_embeddings.py:397-497): the
+    basic edges -- the transitive reduction, pairs (u, v) with no w such that u > w > v; a Hierarchy's parent edges --
+    always train; of the n_nb other closure edges int(val n_nb) go to "val", int(test n_nb) to "test" and
+    int(train_nonbasic n_nb) of the rest to "train".  The draw is np.random.default_rng(seed)'s (not the reference's
+    random.sample order).  Returns {"train", "val", "test"}, each int64 [m, 2] (ancestor, descendant), sorted."""
+    e = h.closure_edges() if h.rank_slots()[0][-1] else np.zeros((0, 2), dtype=np.int64)
+    n = h.n
+    keys = _edge_keys(e, n)
+    nonbasic = _in_sorted(keys, np.unique(_compose(e, e, n))) if len(e) else np.zeros(0, dtype=bool)
+    basic, nb = keys[~nonbasic], keys[nonbasic]
+    n_nb = len(nb)
+    n_val, n_test = int(val * n_nb), int(test * n_nb)
+    if n_val + n_test > n_nb:
+        raise ValueError("val + test exceed the %d non-basic edges" % n_nb)
+    perm = np.random.default_rng(seed).permutation(n_nb)
+    n_train = min(int(train_nonbasic * n_nb), n_nb - n_val - n_test)
+    parts = {"train": np.r_[basic, nb[perm[n_val + n_test:n_val + n_test + n_train]]],
+             "val": nb[perm[:n_val]], "test": nb[perm[n_val:n_val + n_test]]}
+    out = {}
+    for name, k in parts.items():
+        k = np.sort(k)
+        out[name] = np.stack([k // n, k % n], axis=1).astype(np.int64)
+    return out
 
 
 def ethec():

@@ -41,6 +41,61 @@ def best_f1_sweep(e_pos, e_neg):
 RECON_OPEN_BINS = 128   # default coarse bins recounted per round of reconstruction_f1 (about 1 MB of workspace each)
 
 
+def _eval_rows(rows, hierarchy, D, what, need_pairs=False):
+    """(rows, D) of an all-pairs evaluation of `hierarchy`: checked, and copied to a plain [n, D] table unless the
+    kernels can read them as they are (16-byte aligned, unit column stride, row stride D or a multiple of 4)"""
+    N.require_cuda(rows)
+    if rows.dim() != 2 or rows.dtype != torch.float32:
+        raise N.LecError("%s: rows must be a float32 [n, ld] tensor" % what)
+    n = rows.shape[0]
+    D = rows.shape[1] if D is None else int(D)
+    if n != hierarchy.n:
+        raise ValueError("%s: %d rows for a hierarchy of %d nodes" % (what, n, hierarchy.n))
+    if need_pairs and n < 2:
+        raise ValueError("%s: no pairs" % what)
+    if D > rows.shape[1]:
+        raise ValueError("%s: D = %d exceeds the row width %d" % (what, D, rows.shape[1]))
+    rows = rows.detach()
+    if rows.stride(1) != 1 or (rows.stride(0) != D and rows.stride(0) % 4 != 0) or rows.data_ptr() % 16 != 0:
+        rows = rows[:, :D].contiguous()
+    return rows, D
+
+
+class _Cover:
+    """The interval cover of a hierarchy on the device: tin, tout and, for a DagHierarchy with extra intervals, the
+    LecReconExtra `x` (None otherwise) with the tensors it points into."""
+
+    def __init__(self, hierarchy, dev):
+        self.tin = torch.as_tensor(np.asarray(hierarchy.tin), dtype=torch.int32).to(dev)
+        self.tout = torch.as_tensor(np.asarray(hierarchy.tout), dtype=torch.int32).to(dev)
+        self.n_extra = int(hierarchy.extra_ptr[-1]) if hasattr(hierarchy, "extra_ptr") else 0
+        self.x = None
+        if self.n_extra:
+            self.xs = [torch.as_tensor(np.asarray(a), dtype=torch.int32).to(dev)
+                       for a in (hierarchy.extra_ptr, hierarchy.extra_lo, hierarchy.extra_hi)]
+            self.x = N.LecReconExtra(self.xs[0].data_ptr(), self.xs[1].data_ptr(), self.xs[2].data_ptr(), self.n_extra)
+
+
+class _Heldout:
+    """hierarchy.heldout_slots(edges) on the device: the LecHeldout `h`, the held-out layout eval_ptr (host and
+    device), the held-out slot of each edge (`order`) and the closure layout's size."""
+
+    def __init__(self, hierarchy, edges, dev):
+        closure_ptr, _ = hierarchy.rank_slots()
+        eval_ptr, slot_map, self.order, xcum = hierarchy.heldout_slots(edges)
+        self.eval_ptr_h = eval_ptr
+        self.n_closure = int(closure_ptr[-1])
+        # one spare entry: a closure without edges still passes a non-NULL slot map
+        self.keep = [torch.as_tensor(a).to(dev) for a in (closure_ptr, np.r_[slot_map, np.int32(-1)])]
+        self.eval_ptr = torch.as_tensor(eval_ptr).to(dev)
+        xc = None
+        if xcum is not None and len(xcum):
+            xc = torch.as_tensor(xcum).to(dev)
+            self.keep.append(xc)
+        self.h = N.LecHeldout(self.keep[0].data_ptr(), self.keep[1].data_ptr(), 0 if xc is None else xc.data_ptr(),
+                              self.n_closure)
+
+
 def recon_args(rows, tin, tout, geom, K, D, u_begin, u_end, workspace):
     """lec_recon_t for device rows [n, >= D] (fp32, unit column stride), device int32 Euler intervals tin / tout [n]
     and a device workspace tensor; apex rows [u_begin, u_end)."""
@@ -67,29 +122,17 @@ def reconstruction_f1(rows, hierarchy, geom, K, D=None, group=None, workspace_by
     workspace_bytes: device workspace, lec_recon_workspace_bytes(RECON_OPEN_BINS) by default; a smaller one costs
     rounds, not exactness.  stats: a dict that receives the rounds run, the open coarse bins, the numbers of positive
     and negative pairs, the workspace size and the number of extra intervals (0 for a forest)."""
-    N.require_cuda(rows)
-    if rows.dim() != 2 or rows.dtype != torch.float32:
-        raise N.LecError("reconstruction_f1: rows must be a float32 [n, ld] tensor")
+    rows, D = _eval_rows(rows, hierarchy, D, "reconstruction_f1", need_pairs=True)
+    return _recon_rounds(rows, hierarchy, geom, K, D, group, workspace_bytes, stats)
+
+
+def _recon_rounds(rows, hierarchy, geom, K, D, group, workspace_bytes, stats, held=None, threshold=None):
+    """the rounds of reconstruction_f1 (held: a _Heldout, threshold: lec_recon_finish_at's t)"""
     n = rows.shape[0]
-    D = rows.shape[1] if D is None else int(D)
-    if n != hierarchy.n:
-        raise ValueError("reconstruction_f1: %d rows for a hierarchy of %d nodes" % (n, hierarchy.n))
-    if n < 2:
-        raise ValueError("reconstruction_f1: no pairs")
-    if D > rows.shape[1]:
-        raise ValueError("reconstruction_f1: D = %d exceeds the row width %d" % (D, rows.shape[1]))
-    rows = rows.detach()
-    if rows.stride(1) != 1 or (rows.stride(0) != D and rows.stride(0) % 4 != 0) or rows.data_ptr() % 16 != 0:
-        rows = rows[:, :D].contiguous()
     dev = rows.device
     lib = N.lib()
-    tin = torch.as_tensor(np.asarray(hierarchy.tin), dtype=torch.int32).to(dev)
-    tout = torch.as_tensor(np.asarray(hierarchy.tout), dtype=torch.int32).to(dev)
-    n_extra = int(hierarchy.extra_ptr[-1]) if hasattr(hierarchy, "extra_ptr") else 0
-    if n_extra:
-        xptr, xlo, xhi = (torch.as_tensor(np.asarray(a), dtype=torch.int32).to(dev)
-                          for a in (hierarchy.extra_ptr, hierarchy.extra_lo, hierarchy.extra_hi))
-        x = N.LecReconExtra(xptr.data_ptr(), xlo.data_ptr(), xhi.data_ptr(), n_extra)
+    cov = _Cover(hierarchy, dev)
+    n_extra = cov.n_extra
     nb = int(lib.lec_recon_workspace_bytes(RECON_OPEN_BINS)) if workspace_bytes is None else int(workspace_bytes)
     cb = int(lib.lec_recon_counter_bytes(nb))
     if cb < 0:
@@ -99,20 +142,27 @@ def reconstruction_f1(rows, hierarchy, geom, K, D=None, group=None, workspace_by
     if group is not None:
         import torch.distributed as dist
         rank, world = dist.get_rank(group), dist.get_world_size(group)
-    r = recon_args(rows, tin, tout, geom, K, D, n * rank // world, n * (rank + 1) // world, ws)
+    r = recon_args(rows, cov.tin, cov.tout, geom, K, D, n * rank // world, n * (rank + 1) // world, ws)
     out = torch.empty(7, device=dev, dtype=torch.float64)
     status = torch.zeros(4, device=dev, dtype=torch.int64)
     stream = N.stream_ptr(dev)
     rounds = 0
     while True:
-        if n_extra:
-            N.check(lib.lec_recon_pass_dag(ctypes.byref(r), ctypes.byref(x), stream), "lec_recon_pass_dag")
+        if held is not None:
+            N.check(lib.lec_recon_pass_heldout(ctypes.byref(r), None if cov.x is None else ctypes.byref(cov.x),
+                                               ctypes.byref(held.h), stream), "lec_recon_pass_heldout")
+        elif n_extra:
+            N.check(lib.lec_recon_pass_dag(ctypes.byref(r), ctypes.byref(cov.x), stream), "lec_recon_pass_dag")
         else:
             N.check(lib.lec_recon_pass(ctypes.byref(r), stream), "lec_recon_pass")
         rounds += 1
         if group is not None:
             dist.all_reduce(ws[:cb].view(torch.int64), group=group)
-        N.check(lib.lec_recon_finish(ctypes.byref(r), N._p(out), N._p(status), stream), "lec_recon_finish")
+        if threshold is None:
+            N.check(lib.lec_recon_finish(ctypes.byref(r), N._p(out), N._p(status), stream), "lec_recon_finish")
+        else:
+            N.check(lib.lec_recon_finish_at(ctypes.byref(r), float(threshold), N._p(out), N._p(status), stream),
+                    "lec_recon_finish_at")
         more, open_bins, n_pos, n_neg = (int(v) for v in status.cpu())
         if not more:
             break
@@ -165,33 +215,22 @@ def reconstruction_ranks(rows, hierarchy, geom, K, D=None, group=None, return_ra
     (optimistic, pessimistic) in hierarchy.closure_edges() order.  Without edges the three means are NaN.
     stats: a dict that receives the workspace size, the negatives at or below their apex's largest positive key (the
     ones that reach the count) and, with time_stages (which synchronises after each call), the four stage times in ms."""
-    N.require_cuda(rows)
-    if rows.dim() != 2 or rows.dtype != torch.float32:
-        raise N.LecError("reconstruction_ranks: rows must be a float32 [n, ld] tensor")
+    rows, D = _eval_rows(rows, hierarchy, D, "reconstruction_ranks")
+    pos_ptr_h, slot_of_edge = hierarchy.rank_slots()
+    return _rank_run(rows, hierarchy, geom, K, D, group, return_ranks, stats, time_stages, pos_ptr_h, slot_of_edge)
+
+
+def _rank_run(rows, hierarchy, geom, K, D, group, return_ranks, stats, time_stages, pos_ptr_h, slot_of, held=None):
+    """lec_rank_run(_heldout) of reconstruction_ranks over the layout pos_ptr_h; slot_of: the slot of each returned
+    rank's edge"""
     n = rows.shape[0]
-    D = rows.shape[1] if D is None else int(D)
-    if n != hierarchy.n:
-        raise ValueError("reconstruction_ranks: %d rows for a hierarchy of %d nodes" % (n, hierarchy.n))
-    if D > rows.shape[1]:
-        raise ValueError("reconstruction_ranks: D = %d exceeds the row width %d" % (D, rows.shape[1]))
-    rows = rows.detach()
-    if rows.stride(1) != 1 or (rows.stride(0) != D and rows.stride(0) % 4 != 0) or rows.data_ptr() % 16 != 0:
-        rows = rows[:, :D].contiguous()
     dev = rows.device
     lib = N.lib()
-    pos_ptr_h, slot_of_edge = hierarchy.rank_slots()
     n_edges = int(pos_ptr_h[-1])
     has = np.diff(pos_ptr_h) > 0
     n_apexes = int(has.sum())
-    tin = torch.as_tensor(np.asarray(hierarchy.tin), dtype=torch.int32).to(dev)
-    tout = torch.as_tensor(np.asarray(hierarchy.tout), dtype=torch.int32).to(dev)
+    cov = _Cover(hierarchy, dev)
     pos_ptr = torch.as_tensor(pos_ptr_h, dtype=torch.int64).to(dev)
-    n_extra = int(hierarchy.extra_ptr[-1]) if hasattr(hierarchy, "extra_ptr") else 0
-    x = None
-    if n_extra:
-        xptr, xlo, xhi = (torch.as_tensor(np.asarray(a), dtype=torch.int32).to(dev)
-                          for a in (hierarchy.extra_ptr, hierarchy.extra_lo, hierarchy.extra_hi))
-        x = N.LecReconExtra(xptr.data_ptr(), xlo.data_ptr(), xhi.data_ptr(), n_extra)
     nb = int(lib.lec_rank_workspace_bytes(n, n_edges))
     if nb < 0:
         N.check(int(nb), "lec_rank_workspace_bytes")
@@ -201,12 +240,16 @@ def reconstruction_ranks(rows, hierarchy, geom, K, D=None, group=None, return_ra
         import torch.distributed as dist
         rank, world = dist.get_rank(group), dist.get_world_size(group)
     stage_ms = (ctypes.c_float * 4)() if time_stages else None
-    r = rank_args(rows, tin, tout, x, pos_ptr, n_edges, geom, K, D, n * rank // world, n * (rank + 1) // world, ws,
-                  stage_ms)
+    r = rank_args(rows, cov.tin, cov.tout, cov.x, pos_ptr, n_edges, geom, K, D, n * rank // world,
+                  n * (rank + 1) // world, ws, stage_ms)
     sums = torch.zeros(3, device=dev, dtype=torch.int64)
     ap = torch.zeros(n, device=dev, dtype=torch.float64)
     ranks = torch.zeros((n_edges, 2), device=dev, dtype=torch.int32) if return_ranks else None
-    N.check(lib.lec_rank_run(ctypes.byref(r), N._p(sums), N._p(ap), N._p(ranks), N.stream_ptr(dev)), "lec_rank_run")
+    if held is None:
+        N.check(lib.lec_rank_run(ctypes.byref(r), N._p(sums), N._p(ap), N._p(ranks), N.stream_ptr(dev)), "lec_rank_run")
+    else:
+        N.check(lib.lec_rank_run_heldout(ctypes.byref(r), ctypes.byref(held.h), N._p(sums), N._p(ap), N._p(ranks),
+                                         N.stream_ptr(dev)), "lec_rank_run_heldout")
     if group is not None:
         for t in (sums, ap) if ranks is None else (sums, ap, ranks):
             dist.all_reduce(t, group=group)
@@ -220,11 +263,45 @@ def reconstruction_ranks(rows, hierarchy, geom, K, D=None, group=None, return_ra
         out = {"mean_rank": math.nan, "mean_rank_optimistic": math.nan, "map": math.nan}
     out.update(n_edges=n_edges, n_apexes=n_apexes, ap=ap)
     if ranks is not None:
-        out["ranks"] = ranks[torch.as_tensor(slot_of_edge, device=dev)]
+        out["ranks"] = ranks[torch.as_tensor(slot_of, device=dev)]
     if stats is not None:
         stats.update(workspace_bytes=nb, counted_negatives=counted)
         if time_stages:
             stats["stage_ms"] = dict(zip(("keys", "sort", "count", "finish"), (float(v) for v in stage_ms)))
+    return out
+
+
+def link_prediction_ranks(rows, hierarchy, edges, geom, K, D=None, group=None, return_ranks=False, stats=None,
+                          time_stages=False):
+    """Mean rank and MAP of link prediction on the held-out closure edges `edges` [m, 2] (Nickel & Kiela's "link
+    prediction" column; hierarchy.split_edges makes a split): reconstruction_ranks with the held-out pairs as the
+    positives, every ordered pair u != w with w not below u in the full closure as the negatives, and the other closure
+    pairs (the training pairs) skipped; same keys, ties and energies, without materialising them (lec_rank_run_heldout).
+    With edges = hierarchy.closure_edges() the result is reconstruction_ranks', bit for bit.
+    Returns reconstruction_ranks' dict: n_edges = m, n_apexes = the apexes with a held-out edge, ap NaN at every other
+    node, and with return_ranks the ranks in `edges` order."""
+    rows, D = _eval_rows(rows, hierarchy, D, "link_prediction_ranks")
+    held = _Heldout(hierarchy, edges, rows.device)
+    return _rank_run(rows, hierarchy, geom, K, D, group, return_ranks, stats, time_stages, held.eval_ptr_h, held.order,
+                     held)
+
+
+def link_prediction_f1(rows, hierarchy, edges, geom, K, D=None, threshold=None, group=None, workspace_bytes=None,
+                       stats=None):
+    """F1 of link prediction on the held-out closure edges `edges` [m, 2] (Ganea et al.'s transitive closure
+    completion) over the pairs of link_prediction_ranks: positives the held-out pairs, negatives every ordered pair
+    u != w with w not below u in the full closure, training pairs skipped (lec_recon_pass_heldout).
+    Without threshold: reconstruction_f1's best-F1 row over those pairs ('val' phase).  With threshold=t: the row of
+    EmbeddingMetrics(..., t, 'test').calculate_metrics() over them (lec_recon_finish_at: E <= t is a predicted
+    positive, a NaN energy never is; t is compared in fp32 like the reference's float32 energies), with t itself in
+    slot 1 -- pick t on a "val" split, report it on "test".  stats as reconstruction_f1's, plus skipped_pairs."""
+    rows, D = _eval_rows(rows, hierarchy, D, "link_prediction_f1", need_pairs=True)
+    held = _Heldout(hierarchy, edges, rows.device)
+    out = _recon_rounds(rows, hierarchy, geom, K, D, group, workspace_bytes, stats, held, threshold)
+    if threshold is not None:
+        out[1] = threshold
+    if stats is not None:
+        stats["skipped_pairs"] = held.n_closure - int(held.eval_ptr_h[-1])
     return out
 
 
