@@ -38,6 +38,11 @@ extern "C" {
 #define LEC_GEOM_EUC 0 /* EucConesLoss.E_operator, order_embeddings.py:954-969 = oe.py:721-739 (cos-space) */
 #define LEC_GEOM_HYP 1 /* hyperbolic EucConesLoss.E_operator, order_embeddings_h.py:1097-1120 = oe_h.py:811-833 */
 #define LEC_GEOM_OE  2 /* OrderEmbeddingLoss.E_operator, order_embeddings.py:818-824 */
+/* Poincare distance of Nickel & Kiela 2017 (the baseline the cones are compared with, and what Ganea et al. initialise
+ * them from): d(x, y) = arcosh(1 + 2|x-y|^2 / ((1-|x|^2)(1-|y|^2))), symmetric, d = 0 for x == y.  Trained by
+ * lec_pairs_poincare / lec_cone_step, scored by lec_score_topk(_ex) (LEC_PREC_F32) and the lec_recon_* / lec_rank_*
+ * passes; lec_pairs_flat, lec_pairs_grouped, lec_energy_dense(_bwd) and the tensor-core scoring return LEC_E_ENUM. */
+#define LEC_GEOM_POINCARE 4
 
 /* per-row transform applied to the raw parameter rows (Embedder.forward / FeatNet tail) */
 #define LEC_ROWS_NONE          0 /* plain nn.Embedding lookup (order embeddings) */
@@ -150,6 +155,23 @@ int lec_pairs_grouped(int geom, int precision, const float* rows, const double* 
                       float alpha, float* E_pos, float* E_neg, double* loss_out, float* grad_rows,
                       int grad_replicas, void* stream);
 
+/* Nickel & Kiela's softmax loss on the Poincare distance d (LEC_GEOM_POINCARE) for B positives (u_i, v_i), each with
+ * the N negatives v'_ij = neg_to[i, j] (their candidate set {v' : v' != u, v' not below u} is the sampler's "corrupt the
+ * child of u" draw; a repeated negative counts once per draw):
+ *     L_i = d(u_i, v_i) + log sum_{w in {v_i, v'_i1 .. v'_iN}} exp(-d(u_i, w))     (max-subtracted log-sum-exp)
+ *   rows       [n_rows, ld] raw points inside the unit ball (no row transform, no aux terms)
+ *   E_pos [B], E_neg [B, N]   d of every pair (fp32)
+ *   loss_out   optional double[1], sum_i L_i is ADDED to it
+ *   grad_rows  optional [grad_replicas, n_rows, ld], d loss / d rows ADDED as in lec_pairs_grouped (block b -> b % R)
+ * Only LEC_PREC_F64CORE: |x|^2, |y|^2, |x-y|^2 (summed from the differences), <x,y> and the scalar factors in fp64 from
+ * the fp32 rows.  One team per positive (the team sizing of the other pair kernels); u's gradient is accumulated in
+ * registers over its 1 + N pairs.  An id outside [0, n_rows) is counted (lec_index_errors) and read as row 0: a bad u_i
+ * or v_i gives the whole group NaN energies and neither loss nor gradient, a bad negative gets NaN and is left out of
+ * the sum. */
+int lec_pairs_poincare(int precision, const float* rows, int64_t n_rows, int D, int ld, const void* pos_from,
+                       const void* pos_to, const void* neg_to, int idx_bytes, int64_t B, int N, float* E_pos,
+                       float* E_neg, double* loss_out, float* grad_rows, int grad_replicas, void* stream);
+
 /* Dense operands (no gather): E_operator(x, y) on arbitrary [P, D] tensors, as the reference calls
  * it from check_graph_embedding (order_embeddings.py:550-551) and the scoring loops. */
 int lec_energy_dense(int geom, int precision, const float* x, const float* y, int64_t P, int D, float K,
@@ -182,6 +204,10 @@ int lec_rsgd_update(float* table, const float* grad, int grad_replicas, int64_t 
  *        LEC_UPD_SGD   torch.optim.SGD(lr, momentum)   order_embeddings.py:563, oe.py:1712
  *        LEC_UPD_ADAM  torch.optim.Adam(lr)            order_embeddings.py:565, oe.py:1714, oe_h.py:1520-1523
  *        LEC_UPD_NONE  table left alone (grad_out receives d loss / d table)
+ *        LEC_UPD_RSGD_RETRACT  Nickel & Kiela's update (eq. 5-7): w <- proj(w - lr (1 - |w|^2)^2 / 4 g), |w|^2 in fp64,
+ *                      proj rescales a row with |w| >= 1 - 1e-5 to norm 1 - 1e-5 (no inner radius, none of LEC_UPD_RSGD's
+ *                      +1e-15 / +1e-6 offsets); grad_out receives the rescaled gradient.  row_mode must be
+ *                      LEC_ROWS_NONE (LEC_E_ENUM otherwise); rows_out is then the updated row, padded
  *      hyp_rescale != 0 multiplies the gradient by ((1 - |w|) / 2)^2 first (oe_h.py:1766, :1770) and
  *      project_shell != 0 projects the updated row into [r_in, 1 - 1e-5] afterwards (soft_clip, oe_h.py:1771) --
  *      together with LEC_UPD_ADAM that is the reference's default joint hyperbolic update.  RSGD includes both.
@@ -200,6 +226,7 @@ int lec_rsgd_update(float* table, const float* grad, int grad_replicas, int64_t 
 #define LEC_UPD_RSGD 1
 #define LEC_UPD_SGD  2
 #define LEC_UPD_ADAM 3
+#define LEC_UPD_RSGD_RETRACT 4
 typedef struct lec_update {
     int rule, row_mode, geom, lambda_mode /* RSGD: 0 reference 2/(1-|x|) (SURVEY F4), 1 textbook 2/(1-|x|^2) */;
     int hyp_rescale, project_shell;
@@ -263,6 +290,9 @@ int lec_update_rows(const lec_update_t* u, const lec_exchange_t* x /* NULL or wo
  * The pair kernel adds into *upd.loss_acc; the update leaves this rank's loss of the step in *upd.loss_step.
  * Table geometry (n, D, ld, K), rows (upd.rows_out), aux (upd.aux_out) and the gradient replicas are taken from `upd`.
  * ev_pairs_start/stop: optional cudaEvent_t recorded around the pair kernel (for the roofline timing).
+ * geom == LEC_GEOM_POINCARE: the pair kernel is lec_pairs_poincare (precision LEC_PREC_F64CORE, upd.row_mode
+ * LEC_ROWS_NONE, upd.aux_out NULL, w_pos = w_neg = NULL, else LEC_E_ENUM), E_neg is [B, N], alpha and upd.K
+ * are ignored and neg_from is not read (with lec_host_pipe_submit's Philox draw it is drawn and ignored).
  */
 typedef struct lec_step {
     int geom, precision, fused;
@@ -316,7 +346,9 @@ int lec_score_topk(int geom, int precision, const float* labels, int64_t L, cons
  *   LEC_SCORES_LABEL_MAJOR  scores[l * N + i]   the kernel's threads own images, so this is the layout
  *                           whose stores coalesce (128 B per warp); the host wrapper returns it as the
  *                           transposed view, i.e. still indexed scores[i, l].
- * level ranges must be ascending and disjoint. */
+ * level ranges must be ascending and disjoint.
+ * LEC_GEOM_POINCARE: LEC_PREC_F32 and D <= 64 only (LEC_E_ENUM / LEC_E_DIM otherwise); E = d(label, image) evaluated
+ * in fp32 from <x,y> and the row norms (|x-y|^2 = max(|x|^2 + |y|^2 - 2<x,y>, 0)), K ignored. */
 #define LEC_SCORES_IMAGE_MAJOR 0
 #define LEC_SCORES_LABEL_MAJOR 1
 int lec_score_topk_ex(int geom, int precision, const float* labels, int64_t L, const float* images,

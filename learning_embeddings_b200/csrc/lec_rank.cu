@@ -231,6 +231,7 @@ int rank_launch(int geom, FastArgs& a, cudaStream_t st) {
     switch (geom) {
         case LEC_GEOM_EUC: return rank_launch_geom<LEC_GEOM_EUC, EPI>(a, st);
         case LEC_GEOM_HYP: return rank_launch_geom<LEC_GEOM_HYP, EPI>(a, st);
+        case LEC_GEOM_POINCARE: return rank_launch_geom<LEC_GEOM_POINCARE, EPI>(a, st);
         default: return rank_launch_geom<LEC_GEOM_OE, EPI>(a, st);
     }
 }
@@ -239,7 +240,8 @@ int rank_launch(int geom, FastArgs& a, cudaStream_t st) {
 int validate(const lec_rank_t* r, const int64_t* rank_sums, const double* ap, int64_t n_slots) {
     if (!r || !r->rows || !r->tin || !r->tout || !r->pos_ptr || !r->workspace || !rank_sums || !ap) return LEC_E_NULL;
     if (r->D < 1 || r->D > 64 || r->ld < r->D || (r->ld != r->D && r->ld % 4 != 0)) return LEC_E_DIM;
-    if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE) return LEC_E_ENUM;
+    if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE && r->geom != LEC_GEOM_POINCARE)
+        return LEC_E_ENUM;
     if (r->n < 0 || r->n > 0x7fffffffLL || r->n_pos < 0 || r->n_pos > 0x7fffffffLL || r->u_begin < 0 ||
         r->u_end < r->u_begin || r->u_end > r->n)
         return LEC_E_SIZE;

@@ -365,7 +365,8 @@ int recon_launch_geom(FastArgs& a, cudaStream_t st) {
 int validate(const lec_recon_t* r) {
     if (!r || !r->rows || !r->tin || !r->tout || !r->workspace) return LEC_E_NULL;
     if (r->D < 1 || r->D > 64 || r->ld < r->D || (r->ld != r->D && r->ld % 4 != 0)) return LEC_E_DIM;
-    if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE) return LEC_E_ENUM;
+    if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE && r->geom != LEC_GEOM_POINCARE)
+        return LEC_E_ENUM;
     if (r->n < 0 || r->n > 0x7fffffffLL || r->u_begin < 0 || r->u_end < r->u_begin || r->u_end > r->n) return LEC_E_SIZE;
     if (batch_of(r->workspace_bytes) < 1) return LEC_E_SIZE;
     if ((reinterpret_cast<uintptr_t>(r->rows) & 15) || (reinterpret_cast<uintptr_t>(r->workspace) & 15)) return LEC_E_ALIGN;
@@ -416,12 +417,14 @@ extern "C" int lec_recon_pass_heldout(const lec_recon_t* r, const lec_recon_extr
             switch (r->geom) {
                 case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 6>(a, st);
                 case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 6>(a, st);
+                case LEC_GEOM_POINCARE: return recon_launch_geom<LEC_GEOM_POINCARE, 6>(a, st);
                 default: return recon_launch_geom<LEC_GEOM_OE, 6>(a, st);
             }
         }
         switch (r->geom) {
             case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 5>(a, st);
             case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 5>(a, st);
+            case LEC_GEOM_POINCARE: return recon_launch_geom<LEC_GEOM_POINCARE, 5>(a, st);
             default: return recon_launch_geom<LEC_GEOM_OE, 5>(a, st);
         }
     }
@@ -430,12 +433,14 @@ extern "C" int lec_recon_pass_heldout(const lec_recon_t* r, const lec_recon_extr
         switch (r->geom) {
             case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 2>(a, st);
             case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 2>(a, st);
+            case LEC_GEOM_POINCARE: return recon_launch_geom<LEC_GEOM_POINCARE, 2>(a, st);
             default: return recon_launch_geom<LEC_GEOM_OE, 2>(a, st);
         }
     }
     switch (r->geom) {
         case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 1>(a, st);
         case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 1>(a, st);
+        case LEC_GEOM_POINCARE: return recon_launch_geom<LEC_GEOM_POINCARE, 1>(a, st);
         default: return recon_launch_geom<LEC_GEOM_OE, 1>(a, st);
     }
 }

@@ -17,6 +17,8 @@
 //   E = max(0, acos(clamp(g)) - psi),  acos(x) = sqrt(1-|x|) P7(|x|), reflected for x < 0
 // (9 packed FMA-pipe ops + 2 MUFU + an 8-term polynomial; checked against the reference's fp64 run in
 // tests/test_gpu_parity.py -- its error is below the reference's own fp32 error on the golden vectors).
+// Poincare distance (LEC_GEOM_POINCARE, Nickel & Kiela): s = max(A + B - 2p, 0), delta = 2s / ((1-A)(1-B)),
+//   E = log1p(delta + sqrt(delta (delta + 2))) = arcosh(1 + delta), 2/(1-A) and 1/(1-B) formed in fp64 per row.
 //
 // Top-k: a thread cannot afford a sorted insertion per score (lanes diverge), so candidates that beat the
 // current k-th best are appended, predicated and branch-free, to a small per-thread ring in shared
@@ -148,16 +150,23 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         const float* s0 = a.images + (i0 < a.N ? i0 : 0) * (EPI ? a.ld : (int64_t)D);
         const float* s1 = a.images + (i1 < a.N ? i1 : 0) * (EPI ? a.ld : (int64_t)D);
         float b0 = 0.f, b1 = 0.f;
+        double e0 = 0.0, e1 = 0.0;  // Poincare: |y|^2 in fp64, as the labels' A
 #pragma unroll
         for (int d = 0; d < 4 * DQ; ++d) {
             const float v0 = (d < D) ? __ldg(s0 + d) : 0.f;
             const float v1 = (d < D) ? __ldg(s1 + d) : 0.f;
             b0 = fmaf(v0, v0, b0);
             b1 = fmaf(v1, v1, b1);
+            if (GEOM == LEC_GEOM_POINCARE) { e0 += (double)v0 * (double)v0; e1 += (double)v1 * (double)v1; }
             y[j][d] = (GEOM == LEC_GEOM_OE) ? pack2(-v0, -v1) : pack2(v0, v1);
         }
-        B2[j] = pack2(b0, b1);
-        C2[j] = pack2(-1.f - b0, -1.f - b1);
+        if (GEOM == LEC_GEOM_POINCARE) {  // B, 1 / (1 - B)
+            B2[j] = pack2((float)e0, (float)e1);
+            C2[j] = pack2((float)(1.0 / (1.0 - e0)), (float)(1.0 / (1.0 - e1)));
+        } else {
+            B2[j] = pack2(b0, b1);
+            C2[j] = pack2(-1.f - b0, -1.f - b1);
+        }
     }
 
     // ---- top-k state: thresholds in registers, sorted lists and the candidate ring in shared memory
@@ -430,6 +439,18 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 E[2 * j] = max_nan(z0, 0.f);
                 E[2 * j + 1] = max_nan(z1, 0.f);
             }
+        } else if (GEOM == LEC_GEOM_POINCARE) {
+            // cst = {A, 2 / (1 - A)};  s = max(A + B - 2p, 0);  delta = s 2/(1-A) 1/(1-B);  d = log1p(delta + sqrt(delta (delta + 2)))
+            const u64 A2 = pack2(cst.x, cst.x), M2 = pack2(-2.f, -2.f), IA2 = pack2(cst.y, cst.y);
+#pragma unroll
+            for (int j = 0; j < NP; ++j) {
+                float s0, s1, i0, i1;
+                unpack2(ffma2(M2, acc[j], fadd2(A2, B2[j])), s0, s1);
+                unpack2(fmul2(IA2, C2[j]), i0, i1);
+                const float d0 = max_nan(s0, 0.f) * i0, d1 = max_nan(s1, 0.f) * i1;
+                E[2 * j] = log1pf(d0 + sqrtf(d0 * (d0 + 2.f)));
+                E[2 * j + 1] = log1pf(d1 + sqrtf(d1 * (d1 + 2.f)));
+            }
         } else {
             const float Af = cst.x, t0 = cst.y;
             const u64 A2 = pack2(Af, Af);
@@ -655,7 +676,9 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 for (int d = 0; d < D; ++d) { const double v = (double)__ldg(src + d); A += v * v; }
                 const Aux<double> x = row_aux<double>(GEOM, A, a.K);
                 float4 c, c2 = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (GEOM == LEC_GEOM_HYP) {
+                if (GEOM == LEC_GEOM_POINCARE) {
+                    c = make_float4((float)A, (float)(2.0 / (1.0 - A)), 0.f, 0.f);
+                } else if (GEOM == LEC_GEOM_HYP) {
                     c = make_float4((float)A, (float)(1.0 + A), (float)(A * A), (float)(-x.t0));
                     const double sp = sin(x.t0);  // = the clamped asin argument
                     c2 = make_float4((float)sqrt(fmax(0.0, 1.0 - sp * sp)), (float)sp, 0.f, 0.f);

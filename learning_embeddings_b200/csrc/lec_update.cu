@@ -10,7 +10,7 @@
 //      carry this step's tag and adds them in rank order (identical bits on every rank)
 //   3. vector-Jacobian product of the row transform (Embedder.forward): d loss / d table
 //   4. the update rule on the raw row: Riemannian SGD (order_embeddings_h.py:764-775), SGD with momentum or Adam
-//      (torch.optim, order_embeddings.py:563-565), optionally preceded by the conformal rescale ((1-|w|)/2)^2 and followed
+//      (torch.optim, order_embeddings.py:563-565), Nickel & Kiela's rescaled step + retraction (Poincare embeddings), optionally preceded by the conformal rescale ((1-|w|)/2)^2 and followed
 //      by the shell projection of the joint hyperbolic trainer (oe_h.py:1765-1771)
 //   5. the row transform of the UPDATED row -- the Embedder.forward the next iteration starts with -- and its per-row
 //      aperture terms (aux), so the next pair kernel can start right away
@@ -268,7 +268,7 @@ __device__ __forceinline__ float sumsq32(const float (&x)[4 * V]) {
 
 // ---- steps 3 + 4 for one row held by a team: VJP of the row transform, update rule; e becomes the new raw row (and is
 //      stored to the table when valid), the optimizer state is advanced ------------------------------------------------
-template <int TT, int V>
+template <int TT, int V, int RULE_T>
 __device__ __forceinline__ void row_rule(const UpdArgs& a, const int rule, const int row_mode, float (&g)[4 * V], float (&e)[4 * V],
                                          float (&mb)[4 * V], float (&vb)[4 * V], const int64_t row, const int64_t rc,
                                          const bool valid, const int lane) {
@@ -308,7 +308,31 @@ __device__ __forceinline__ void row_rule(const UpdArgs& a, const int rule, const
         }
     }
     // ---- 4. update rule ------------------------------------------------------------------------------------------
-    if (rule == LEC_UPD_RSGD) {
+    if (RULE_T == LEC_UPD_RSGD_RETRACT) {
+        // Nickel & Kiela (eq. 5-7): w <- proj(w - lr (1 - |w|^2)^2 / 4 g), proj: |w| >= 1 - 1e-5 -> norm 1 - 1e-5.  Only
+        // this compile-time specialisation holds the rule (the generic kernels never see it; row_mode is NONE)
+        double uu = 0.0;
+#pragma unroll
+        for (int i = 0; i < 4 * V; ++i) uu = fma((double)e[i], (double)e[i], uu);
+        uu = team_sum<TT, double>(uu);
+        const double om = 1.0 - uu;
+        const float gs = (float)(0.25 * om * om);
+#pragma unroll
+        for (int i = 0; i < 4 * V; ++i) g[i] *= gs;                       // the Riemannian gradient
+        if (valid && a.grad_out) store_raw<TT, V>(a.grad_out + row * (int64_t)D, g, D, lane, a.tv);
+#pragma unroll
+        for (int i = 0; i < 4 * V; ++i) e[i] = fmaf(-a.lr, g[i], e[i]);
+        double nn = 0.0;
+#pragma unroll
+        for (int i = 0; i < 4 * V; ++i) nn = fma((double)e[i], (double)e[i], nn);
+        const double nrm = sqrt(team_sum<TT, double>(nn));
+        constexpr double kMaxNorm = 1.0 - 1e-5;
+        if (nrm >= kMaxNorm) {
+            const float sc = (float)(kMaxNorm / nrm);
+#pragma unroll
+            for (int i = 0; i < 4 * V; ++i) e[i] *= sc;
+        }
+    } else if (rule == LEC_UPD_RSGD) {
         // One pass gives the five row sums every later quantity is an algebraic function of (v = -lr gs g + 1e-15,
         // t = th v/|v| + 1e-6, the Moebius sums <w,t>, |t|^2 and the norm of the result), carried in fp64:
         double uu = 0.0, gg = 0.0, eg = 0.0, se = 0.0, sg = 0.0;
@@ -550,7 +574,7 @@ __global__ void __launch_bounds__(kThreads, (V <= 4 && !XCHG && RULE_T >= 0) ? L
             if (__any_sync(0xffffffffu, !ok)) valid = false;
             if (lane == 0) LEC_TRACE_MAX(a.trace, 5);
         }
-        row_rule<TT, V>(a, rule, row_mode, g, e, mb, vb, row, rc, valid, lane);
+        row_rule<TT, V, RULE_T>(a, rule, row_mode, g, e, mb, vb, row, rc, valid, lane);
         row_forward<TT, V>(a, row_mode, e, row, valid, lane);
     }
     if (threadIdx.x == 0) LEC_TRACE_MAX(a.trace, 6);
@@ -718,7 +742,7 @@ __global__ void __launch_bounds__(kThreads, V <= 4 ? 2 : 1) update_owner_kernel(
 #pragma unroll
             for (int j = 0; j < V; ++j) { g[4 * j] = acc[j].x; g[4 * j + 1] = acc[j].y; g[4 * j + 2] = acc[j].z; g[4 * j + 3] = acc[j].w; }
         }
-        row_rule<TT, V>(a, rule, row_mode, g, e, mb, vb, row, rc, valid, lane);
+        row_rule<TT, V, RULE_T>(a, rule, row_mode, g, e, mb, vb, row, rc, valid, lane);
         // the tile's updated raw rows (pad columns zero) are staged in shared memory as the slab they form in every peer's
         // staging area ...
         {
@@ -837,6 +861,7 @@ static int two_shot_go(UpdArgs& a, cudaStream_t st) {
     a.tiles_per_rank = (int)((per + tpb - 1) / tpb);
     a.rows_per_rank = (int64_t)a.tiles_per_rank * tpb;
     if (a.rule == LEC_UPD_RSGD && a.row_mode == LEC_ROWS_HYP_SHELL) return two_shot_go2<TT, V, LEC_UPD_RSGD, LEC_ROWS_HYP_SHELL>(a, st);
+    if (a.rule == LEC_UPD_RSGD_RETRACT) return two_shot_go2<TT, V, LEC_UPD_RSGD_RETRACT, LEC_ROWS_NONE>(a, st);
     return two_shot_go2<TT, V, -1, -1>(a, st);
 }
 
@@ -854,6 +879,7 @@ template <int TT, int V>
 static int update_go(const UpdArgs& a, cudaStream_t st) {
     // the two training configurations of the benchmarks get specialised kernels; everything else the generic one
     if (a.rule == LEC_UPD_RSGD && a.row_mode == LEC_ROWS_HYP_SHELL) return update_go2<TT, V, LEC_UPD_RSGD, LEC_ROWS_HYP_SHELL>(a, st);
+    if (a.rule == LEC_UPD_RSGD_RETRACT) return update_go2<TT, V, LEC_UPD_RSGD_RETRACT, LEC_ROWS_NONE>(a, st);   // row_mode NONE (checked)
     if (a.rule == LEC_UPD_ADAM && a.row_mode == LEC_ROWS_EUC_SOFTCLIP && !a.hyp_rescale && !a.project_shell)
         return update_go2<TT, V, LEC_UPD_ADAM, LEC_ROWS_EUC_SOFTCLIP>(a, st);
     return update_go2<TT, V, -1, -1>(a, st);

@@ -44,14 +44,19 @@ def pack_index_block(pos_from, pos_to, neg_to, neg_from, pin=True, dtype=np.int3
     return blk.pin_memory() if (pin and torch.cuda.is_available()) else blk
 
 
-RULES = {"none": N.UPD_NONE, "rsgd": N.UPD_RSGD, "sgd": N.UPD_SGD, "adam": N.UPD_ADAM}
+RULES = {"none": N.UPD_NONE, "rsgd": N.UPD_RSGD, "sgd": N.UPD_SGD, "adam": N.UPD_ADAM, "rsgd_retract": N.UPD_RSGD_RETRACT}
 
 
 class ConeStep:
     """update: "rsgd" (order_embeddings_h.py:764-775), "sgd" / "adam" (torch.optim semantics, order_embeddings.py:563-565),
     "none" (gradient only, left in grad_table), "auto" = rsgd for hyperbolic cones, sgd otherwise.  hyp_rescale /
     project_shell: the joint hyperbolic trainer's gradient rescale and table projection around sgd / adam
-    (oe_h.py:1765-1771).  Every rule runs inside the library's fused update kernel (lec_update_rows)."""
+    (oe_h.py:1765-1771).  Every rule runs inside the library's fused update kernel (lec_update_rows).
+
+    geom="poincare": Nickel & Kiela's Poincare embeddings -- the softmax loss over each positive and its n_neg
+    negatives (lec_pairs_poincare; neg_from is not read, E_neg is [max_groups, n_neg]) and update "rsgd_retract" (the
+    default: w <- proj(w - lr (1 - |w|^2)^2 / 4 g)) or "none".  The table is used as it is (no row transform, no aux
+    terms); K, alpha and pair weights do not apply."""
 
     def __init__(self, table, geom, n_neg, max_groups, K=None, alpha=1.0, lr=1e-3, row_mode=None, update="auto",
                  precision=ops.PREC_F64CORE, process_group=None, replicas=None, comm="auto", momentum=0.0,
@@ -64,14 +69,22 @@ class ConeStep:
         self.n, self.D = table.shape
         self.ld = ops.padded_dim(self.D)
         self.n_neg = int(n_neg)
-        self.K = {"euc": 3.0, "hyp": 0.1, "oe": 0.0}[geom] if K is None else float(K)
+        poincare = geom == "poincare"
+        self.K = {"euc": 3.0, "hyp": 0.1, "oe": 0.0, "poincare": 0.0}[geom] if K is None else float(K)
         self.alpha = float(alpha)
         self.lr = float(lr)
-        self.row_mode = {"euc": N.ROWS_EUC_SOFTCLIP, "hyp": N.ROWS_HYP_SHELL, "oe": N.ROWS_NONE}[geom] \
+        self.row_mode = {"euc": N.ROWS_EUC_SOFTCLIP, "hyp": N.ROWS_HYP_SHELL, "oe": N.ROWS_NONE, "poincare": N.ROWS_NONE}[geom] \
             if row_mode is None else int(row_mode)
-        self.update = ("rsgd" if geom == "hyp" else "sgd") if update == "auto" else update
+        if update == "auto":
+            update = {"hyp": "rsgd", "poincare": "rsgd_retract"}.get(geom, "sgd")
+        self.update = update
         if self.update not in RULES:
             raise N.LecError("unknown update rule %r" % (self.update,))
+        if poincare and (self.update not in ("rsgd_retract", "none") or self.row_mode != N.ROWS_NONE):
+            raise N.LecError("ConeStep(geom='poincare'): update must be 'rsgd_retract' or 'none' on untransformed rows, "
+                             "got update=%r, row_mode=%d" % (self.update, self.row_mode))
+        if self.update == "rsgd_retract" and not poincare:
+            raise N.LecError("update 'rsgd_retract' is the Poincare embeddings' rule (geom='poincare')")
         self.momentum, self.betas, self.eps = float(momentum), (float(betas[0]), float(betas[1])), float(eps)
         self.hyp_rescale, self.project_shell = bool(hyp_rescale), bool(project_shell)
         self.r_in = float(inner_radius(self.K)) if geom == "hyp" else 0.0
@@ -81,11 +94,11 @@ class ConeStep:
         dev = table.device
         self.replicas = ops.default_replicas(self.n, self.ld) if replicas is None else int(replicas)
         self.rows = torch.empty((self.n, self.ld), device=dev, dtype=torch.float32)
-        self.aux = torch.empty((self.n, 4), device=dev, dtype=torch.float64)
+        self.aux = None if poincare else torch.empty((self.n, 4), device=dev, dtype=torch.float64)
         self.grad_rows = torch.empty((self.replicas, self.n, self.ld), device=dev, dtype=torch.float32)
         self.grad_table = torch.empty((self.n, self.D), device=dev, dtype=torch.float32)
         self.E_pos = torch.empty(self.max_groups, device=dev, dtype=torch.float32)
-        self.E_neg = torch.empty((self.max_groups, 2 * self.n_neg), device=dev, dtype=torch.float32)
+        self.E_neg = torch.empty((self.max_groups, (1 if poincare else 2) * self.n_neg), device=dev, dtype=torch.float32)
         # the pair kernel adds into loss_acc; the update kernel moves it to `loss` (this rank's loss of the latest step)
         self.loss = torch.zeros(1, device=dev, dtype=torch.float64)
         self._loss_ptr = self.loss.data_ptr()
@@ -165,7 +178,7 @@ class ConeStep:
         u.grad_replicas = self.replicas if replicas is None else replicas
         u.state_m = self.opt_m.data_ptr() if self.opt_m is not None else None
         u.state_v = self.opt_v.data_ptr() if self.opt_v is not None else None
-        u.rows_out, u.aux_out = self.rows.data_ptr(), self.aux.data_ptr()
+        u.rows_out, u.aux_out = self.rows.data_ptr(), self.aux.data_ptr() if self.aux is not None else None
         u.grad_out = self.grad_table.data_ptr() if self.write_grad_table else None
         u.loss_acc, u.loss_step = self.loss_acc.data_ptr(), self.loss.data_ptr()
         if grad_rows is None:
@@ -190,12 +203,20 @@ class ConeStep:
         ev = self.kernel_events
         if ev is not None:
             ev[0].record()
-        N.check(lib.lec_pairs_grouped(
-            N.GEOM[self.geom], self.precision, N._p(self.rows), N._p(self.aux), self.n, self.D, self.ld,
-            N._p(pos_from), N._p(pos_to),
-            N._p(neg_to), N._p(neg_from), pos_from.element_size(), B, self.n_neg, N._p(w_pos), N._p(w_neg), self.K,
-            self.alpha, N._p(self.E_pos), N._p(self.E_neg), N._p(self.loss_acc), N._p(self.grad_rows), self.replicas, st),
-            "lec_pairs_grouped")
+        if self.geom == "poincare":
+            if w_pos is not None or w_neg is not None:
+                raise N.LecError("the Poincare loss takes no pair weights")
+            N.check(lib.lec_pairs_poincare(
+                self.precision, N._p(self.rows), self.n, self.D, self.ld, N._p(pos_from), N._p(pos_to), N._p(neg_to),
+                pos_from.element_size(), B, self.n_neg, N._p(self.E_pos), N._p(self.E_neg), N._p(self.loss_acc),
+                N._p(self.grad_rows), self.replicas, st), "lec_pairs_poincare")
+        else:
+            N.check(lib.lec_pairs_grouped(
+                N.GEOM[self.geom], self.precision, N._p(self.rows), N._p(self.aux), self.n, self.D, self.ld,
+                N._p(pos_from), N._p(pos_to),
+                N._p(neg_to), N._p(neg_from), pos_from.element_size(), B, self.n_neg, N._p(w_pos), N._p(w_neg), self.K,
+                self.alpha, N._p(self.E_pos), N._p(self.E_neg), N._p(self.loss_acc), N._p(self.grad_rows), self.replicas,
+                st), "lec_pairs_grouped")
         if ev is not None:
             ev[1].record()
         return B

@@ -183,6 +183,56 @@ def grouped_pair_loss(rows, aux, D, pos_from, pos_to, neg_to, neg_from, n_neg, g
                                  precision)
 
 
+class PoincareLoss(torch.autograd.Function):
+    """loss, E_pos[B], E_neg[B, N] of Nickel & Kiela's softmax loss on the Poincare distance (lec_pairs_poincare)."""
+
+    @staticmethod
+    def forward(ctx, rows, D, pos_from, pos_to, neg_to):
+        N.require_cuda(rows)
+        dev = rows.device
+        n, width = rows.shape
+        if width < D:
+            raise N.LecError("poincare_loss: rows have %d columns, D = %d" % (width, D))
+        ld = padded_dim(D)
+        padded = torch.zeros((n, ld), device=dev, dtype=torch.float32)
+        padded[:, :D] = rows.detach()[:, :D]
+        pos_from, pos_to, neg_to = _idx(pos_from, dev), _idx(pos_to, dev), _idx(neg_to, dev)
+        if not (pos_from.dtype == pos_to.dtype == neg_to.dtype):
+            pos_from, pos_to, neg_to = (t.to(torch.int64) for t in (pos_from, pos_to, neg_to))
+        B = int(pos_from.numel())
+        n_neg = int(neg_to.numel()) // max(B, 1)
+        E_pos = torch.empty(B, device=dev, dtype=torch.float32)
+        E_neg = torch.empty((B, n_neg), device=dev, dtype=torch.float32)
+        loss64 = torch.zeros(1, device=dev, dtype=torch.float64)
+        grad_rows = None
+        if ctx.needs_input_grad[0]:
+            grad_rows = torch.zeros((default_replicas(n, ld), n, ld), device=dev)
+        N.check(N.lib().lec_pairs_poincare(
+            PREC_F64CORE, N._p(padded), n, int(D), ld, N._p(pos_from), N._p(pos_to), N._p(neg_to),
+            pos_from.element_size(), B, n_neg, N._p(E_pos), N._p(E_neg), N._p(loss64), N._p(grad_rows),
+            1 if grad_rows is None else grad_rows.shape[0], N.stream_ptr(dev)), "lec_pairs_poincare")
+        grad = None
+        if grad_rows is not None:
+            grad = torch.zeros_like(rows, dtype=torch.float32)
+            grad[:, :D] = reduce_replicas(grad_rows)[:, :D]
+        ctx.save_for_backward(grad)
+        ctx.mark_non_differentiable(E_pos, E_neg)
+        return loss64[0], E_pos, E_neg
+
+    @staticmethod
+    def backward(ctx, g_loss, _gp, _gn):
+        (grad,) = ctx.saved_tensors
+        return (grad * g_loss.float(),) + (None,) * 4
+
+
+def poincare_loss(rows, D, pos_from, pos_to, neg_to):
+    """Nickel & Kiela's loss sum_i [d(u_i, v_i) + log sum_{w in {v_i} + neg_to[i]} exp(-d(u_i, w))] on the Poincare
+    distance, for use outside the step engine.  rows [n, >= D] are points inside the unit ball (fp32 CUDA); pos_from,
+    pos_to [B] and neg_to [B, N] are row ids.  Returns (loss as a float64 scalar, E_pos [B], E_neg [B, N]); the loss is
+    differentiable with respect to rows (fp64 pair algebra, gradient computed in the forward launch)."""
+    return PoincareLoss.apply(rows, D, pos_from, pos_to, neg_to)
+
+
 def pairs_flat_raw(geom, rows, aux, D, from_idx, to_idx, K, alpha, w=None, is_pos=None, grad_rows=None, loss_out=None,
                    precision=PREC_F64CORE, E_out=None):
     dev = rows.device
