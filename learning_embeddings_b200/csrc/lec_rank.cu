@@ -1,16 +1,16 @@
 // Reconstruction mean rank and MAP over all ordered node pairs without materialising the energies (the ranking
 // evaluation of Nickel & Kiela's Poincaré embeddings, over the pairs and energies of lec_recon.cu).  One call, four
 // stages, no host round trip:
-//   keys     score_fast_kernel<EPI = 3>: the rank key of every positive pair into its slot pos_ptr[u] + slot(u, v)
+//   keys     score_fast_kernel<Pass::RankKeys>: the rank key of every positive pair into its slot pos_ptr[u] + slot(u, v)
 //            (same <GEOM, DH, RI> as lec_recon_pass, so the same energy bits as the SIMT matrix)
 //   sort     cub::DeviceSegmentedRadixSort of each apex's keys (31 key bits), carrying the slot ids.  Not
 //            DeviceSegmentedSort: above 500 segments it copies its partition sizes to the host and synchronises.
-//   count    score_fast_kernel<EPI = 4>: a negative at or below its apex's largest positive key adds 1 to cnt[b] and,
+//   count    score_fast_kernel<Pass::RankCounts>: a negative at or below its apex's largest positive key adds 1 to cnt[b] and,
 //            when it equals sorted[b], to eq[b], where b is its lower bound among the apex's sorted keys
 //   finish   per apex: rank_pess = 1 + prefix(cnt) at the slot, rank_opt = rank_pess - eq[first slot of its tie group],
 //            AP_u in fp64 in a fixed order
-// On a held-out set (lec_rank_run_heldout) pos_ptr is the held-out layout and the key pass is EPI = 7: it finds each
-// positive's closure slot as EPI = 3 does and writes the key to the held-out slot the slot map gives, or nowhere.  Sort,
+// On a held-out set (lec_rank_run_heldout) pos_ptr is the held-out layout and the key pass is Pass::RankKeysHeld: it
+// finds each positive's closure slot as RankKeys does and writes the key to the held-out slot the slot map gives, or nowhere.  Sort,
 // count and finish run unchanged: the count already leaves out every closure pair, held out or not.
 //
 // Workspace (caller-owned, needs no initialisation; each region 256-byte aligned):
@@ -29,11 +29,6 @@ constexpr int kRankPrepThreads = 1024;
 constexpr int kRankFinishThreads = 256;
 constexpr int kRankFinishBlocks = 148 * 8;
 constexpr int kRankKeyBits = 31;  // keys are <= 0x7fc00000
-constexpr int kRankTarget = 148 * 16;
-constexpr int64_t kRankMaxChunk = 4096;
-
-template <int DH>
-constexpr int rank_threads() { return DH > 16 ? 256 : 512; }  // lec_recon_pass's blocks (energy bits do not depend on it)
 
 size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 
@@ -186,72 +181,17 @@ __global__ void __launch_bounds__(kRankFinishThreads) rank_finish_kernel(
     }
 }
 
-template <int GEOM, int DH, int RI, int EPI>
-int rank_launch_dh(FastArgs& a, cudaStream_t st) {
-    constexpr int NT = rank_threads<DH>();
-    constexpr int LS = 4 * ((DH + 1) / 2) + 8;
-    const size_t smem = (size_t)kTileLabels * LS * sizeof(float) + (size_t)kTileLabels * (sizeof(int4) + sizeof(int2) + 2 * sizeof(int)) +
-                        4 * sizeof(int) + (EPI == 4 ? (size_t)kRankShared * sizeof(unsigned) : 0);
-    static bool configured = false;
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(score_fast_kernel<GEOM, DH, RI, NT, 1, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-        configured = true;
-    }
-    a.groups = (a.N + (int64_t)NT * RI - 1) / ((int64_t)NT * RI);
-    const int64_t rows = a.u_end;  // an upper bound on the apex list; blocks past its end return at once
-    int64_t chunks = (kRankTarget + a.groups - 1) / a.groups;
-    int64_t chunk = (rows + chunks - 1) / chunks;
-    if (chunk < 32) chunk = 32;
-    if (chunk > kRankMaxChunk) chunk = kRankMaxChunk;
-    a.chunk = chunk;
-    chunks = (rows + chunk - 1) / chunk;
-    const int64_t blocks = a.groups * chunks;
-    if (blocks > 0x7fffffffLL) return LEC_E_SIZE;
-    score_fast_kernel<GEOM, DH, RI, NT, 1, EPI><<<(unsigned)blocks, NT, smem, st>>>(a);
-    ++g_launches;
-    return (int)cudaGetLastError();
-}
-
-template <int GEOM, int EPI>
-int rank_launch_geom(FastArgs& a, cudaStream_t st) {
-    const int dh = (a.D + 1) / 2;  // the scoring kernel's instantiations (fast_launch_geom)
-    if (dh <= 1) return rank_launch_dh<GEOM, 1, 4, EPI>(a, st);
-    if (dh <= 2) return rank_launch_dh<GEOM, 2, 4, EPI>(a, st);
-    if (dh <= 5) return rank_launch_dh<GEOM, 5, 4, EPI>(a, st);
-    if (dh <= 8) return rank_launch_dh<GEOM, 8, 4, EPI>(a, st);
-    if (dh <= 16) return rank_launch_dh<GEOM, 16, 2, EPI>(a, st);
-    if (dh <= 25) return rank_launch_dh<GEOM, 25, 2, EPI>(a, st);
-    if (dh <= 32) return rank_launch_dh<GEOM, 32, 2, EPI>(a, st);
-    return LEC_E_DIM;
-}
-
-template <int EPI>
-int rank_launch(int geom, FastArgs& a, cudaStream_t st) {
-    switch (geom) {
-        case LEC_GEOM_EUC: return rank_launch_geom<LEC_GEOM_EUC, EPI>(a, st);
-        case LEC_GEOM_HYP: return rank_launch_geom<LEC_GEOM_HYP, EPI>(a, st);
-        case LEC_GEOM_POINCARE: return rank_launch_geom<LEC_GEOM_POINCARE, EPI>(a, st);
-        default: return rank_launch_geom<LEC_GEOM_OE, EPI>(a, st);
-    }
-}
-
 // n_slots: the positives an extra interval may hold (n_pos, or the closure's on a held-out set)
 int validate(const lec_rank_t* r, const int64_t* rank_sums, const double* ap, int64_t n_slots) {
-    if (!r || !r->rows || !r->tin || !r->tout || !r->pos_ptr || !r->workspace || !rank_sums || !ap) return LEC_E_NULL;
-    if (r->D < 1 || r->D > 64 || r->ld < r->D || (r->ld != r->D && r->ld % 4 != 0)) return LEC_E_DIM;
-    if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE && r->geom != LEC_GEOM_POINCARE)
-        return LEC_E_ENUM;
-    if (r->n < 0 || r->n > 0x7fffffffLL || r->n_pos < 0 || r->n_pos > 0x7fffffffLL || r->u_begin < 0 ||
-        r->u_end < r->u_begin || r->u_end > r->n)
-        return LEC_E_SIZE;
-    const lec_recon_extra_t* x = r->extra;
-    if (x && x->count != 0) {
-        if (x->count < 0 || x->count > n_slots) return LEC_E_SIZE;  // an extra interval holds at least one positive
-        if (!x->ptr || !x->lo || !x->hi) return LEC_E_NULL;
-    }
-    if ((reinterpret_cast<uintptr_t>(r->rows) & 15) || (reinterpret_cast<uintptr_t>(r->workspace) & 15)) return LEC_E_ALIGN;
-    return 0;
+    return eval_validate(r, r && r->pos_ptr && rank_sums && ap, [&] {
+        if (r->n_pos < 0 || r->n_pos > 0x7fffffffLL) return LEC_E_SIZE;
+        const lec_recon_extra_t* x = r->extra;
+        if (x && x->count != 0) {
+            if (x->count < 0 || x->count > n_slots) return LEC_E_SIZE;  // an extra interval holds at least one positive
+            if (!x->ptr || !x->lo || !x->hi) return LEC_E_NULL;
+        }
+        return 0;
+    });
 }
 
 }  // namespace
@@ -315,7 +255,7 @@ extern "C" int lec_rank_run_heldout(const lec_rank_t* r, const lec_heldout_t* h,
         a.rapex = l.apex; a.rnapex = l.napex; a.rpos = r->pos_ptr; a.rxcum = h ? h->xcum : l.xcum;
         a.rkey = l.key_in; a.rval = l.val_in; a.rsorted = l.key_out; a.rcnt = l.cnt; a.req = l.eq;
         if (h) { a.hptr = h->closure_ptr; a.hmap = h->slot_map; }
-        rc = h ? rank_launch<7>(r->geom, a, st) : rank_launch<3>(r->geom, a, st);
+        rc = h ? eval_launch<Pass::RankKeysHeld>(r->geom, a, st) : eval_launch<Pass::RankKeys>(r->geom, a, st);
         if (rc) return rc;
         mark(1);
         size_t tb = temp;
@@ -324,7 +264,7 @@ extern "C" int lec_rank_run_heldout(const lec_rank_t* r, const lec_heldout_t* h,
                                                      kRankKeyBits, st);
         if (e != cudaSuccess) return (int)e;
         mark(2);
-        rc = rank_launch<4>(r->geom, a, st);
+        rc = eval_launch<Pass::RankCounts>(r->geom, a, st);
         if (rc) return rc;
         mark(3);
         rank_finish_kernel<<<kRankFinishBlocks, kRankFinishThreads, 0, st>>>(

@@ -2,10 +2,10 @@
 // order_embeddings.py:512-559 = oe.py:1923-1990: the energy of every closure edge against that of every other ordered
 // pair u != v, then EmbeddingMetrics.calculate_metrics('val')).
 //
-// The energies are the SIMT scoring kernel's (score_fast_kernel with EPI = 1: same per-pair instructions, so the same
-// bits as the lec_score_topk_ex matrix), classified by the Euler intervals and counted, never stored (EPI = 2,
-// lec_recon_pass_dag: a DAG's interval cover, the Euler-like primary interval plus each apex's extra intervals; EPI = 5, 6,
-// lec_recon_pass_heldout: positives only where the closure slot is held out, other closure pairs skipped):
+// The energies are the SIMT scoring kernel's (score_fast_kernel's Pass::F1: same per-pair instructions, so the same bits
+// as the lec_score_topk_ex matrix), classified by the Euler intervals and counted, never stored (Pass::F1Dag: a DAG's
+// interval cover, the Euler-like primary interval plus each apex's extra intervals; Pass::F1Held, F1HeldDag: positives
+// only where the closure slot is held out, other closure pairs skipped):
 //   round 0      every pair's key (fp32 bits; energies are >= 0 or NaN) into 2 x 32 768 coarse bins (key >> 16)
 //   select       exact F1 at each coarse bin's largest value gives a lower bound LB on the best F1; a bin can
 //                only hold a better threshold if 2 CP_b / (n_pos + CP_b + FP_{b-1}) >= LB (1 - 1e-12) -- the slack
@@ -29,12 +29,6 @@ namespace lec {
 namespace {
 
 typedef unsigned long long u64c;
-// one block per SM (128 KB of shared counters): 16 warps where the image rows fit 128 registers, else 8 (D > 32 spills
-// at 512 threads)
-template <int DH>
-constexpr int recon_threads() { return DH > 16 ? 256 : 512; }
-constexpr int kReconTarget = 148 * 16;  // blocks per pass to aim for (16 waves: the chunks balance)
-constexpr int64_t kReconMaxChunk = 4096;  // apex rows per block: its 32-bit shared counters cannot overflow
 constexpr int kSelThreads = 1024;
 constexpr int64_t kMaxBatch = 16383;  // fine tags (slot, key, sign) fit an int
 
@@ -71,7 +65,8 @@ Layout layout(void* ws, int64_t ws_bytes) {
     return l;
 }
 
-// exclusive prefix sum over the block (NT threads, NT / 32 <= 32 warps)
+// exclusive prefix sum over the block (NT threads, NT / 32 <= 32 warps).  Not cub::BlockScan: cub's headers add device
+// globals to this file, which would move the constant-bank slots the evaluation passes read their math tables from.
 template <typename T, int NT>
 __device__ T block_exclusive_scan(T x, T& total) {
     __shared__ T warp_sum[NT / 32];
@@ -98,6 +93,22 @@ __device__ T block_exclusive_scan(T x, T& total) {
     total = warp_sum[NT / 32 - 1];
     const T before = w > 0 ? warp_sum[w - 1] : T(0);
     return before + inc - x;
+}
+
+// the block's best candidate (f1_better: the higher F1, the lower key on a tie), in every thread
+__device__ ReconBest block_best(ReconBest b) {
+    __shared__ ReconBest sh[kSelThreads];
+    const int tid = threadIdx.x;
+    sh[tid] = b;
+    __syncthreads();
+    for (int w = kSelThreads / 2; w > 0; w >>= 1) {
+        if (tid < w) {
+            const ReconBest c = sh[tid + w], a = sh[tid];
+            if (c.has && (!a.has || f1_better(c.f1, c.key, a.f1, a.key))) sh[tid] = c;
+        }
+        __syncthreads();
+    }
+    return sh[0];
 }
 
 __device__ void write_row(const ReconState& s, float t, u64c cp, u64c cn, double* out7) {
@@ -203,17 +214,8 @@ __global__ void __launch_bounds__(kSelThreads) recon_fine_kernel(const u64c* __r
         const double f1 = row[0] == row[0] ? row[0] : -1.0;   // NaN never wins
         if (!b.has || f1 > b.f1) b = ReconBest{f1, cp, neg_fin - fp, key, 1};
     }
-    __shared__ ReconBest sh[kSelThreads];
-    sh[tid] = b;
-    __syncthreads();
-    for (int w = kSelThreads / 2; w > 0; w >>= 1) {
-        if (tid < w) {
-            const ReconBest c = sh[tid + w], a = sh[tid];
-            if (c.has && (!a.has || f1_better(c.f1, c.key, a.f1, a.key))) sh[tid] = c;
-        }
-        __syncthreads();
-    }
-    if (tid == 0) best[blockIdx.x] = sh[0];
+    b = block_best(b);
+    if (tid == 0) best[blockIdx.x] = b;
 }
 
 // end of a fine round: merge the batch into the carried best (earlier batches hold lower keys: they win ties)
@@ -230,18 +232,8 @@ __global__ void __launch_bounds__(kSelThreads) recon_merge_kernel(ReconState* __
         const ReconBest c = best[i];
         if (c.has && (!b.has || f1_better(c.f1, c.key, b.f1, b.key))) b = c;
     }
-    __shared__ ReconBest sh[kSelThreads];
-    sh[tid] = b;
-    __syncthreads();
-    for (int w = kSelThreads / 2; w > 0; w >>= 1) {
-        if (tid < w) {
-            const ReconBest c = sh[tid + w], a = sh[tid];
-            if (c.has && (!a.has || f1_better(c.f1, c.key, a.f1, a.key))) sh[tid] = c;
-        }
-        __syncthreads();
-    }
+    const ReconBest c = block_best(b);
     if (tid == 0) {
-        const ReconBest c = sh[0];
         if (c.has && (!s->has_best || c.f1 > s->best_f1)) {
             s->best_f1 = c.f1; s->best_cp = c.cp; s->best_cn = c.cn; s->best_key = c.key; s->has_best = 1;
         }
@@ -322,55 +314,8 @@ __global__ void __launch_bounds__(kSelThreads) recon_at_fine_kernel(const u64c* 
     }
 }
 
-template <int GEOM, int DH, int RI, int EPI>
-int recon_launch_dh(FastArgs& a, cudaStream_t st) {
-    constexpr int NT = recon_threads<DH>();
-    constexpr int LS = 4 * ((DH + 1) / 2) + 8;
-    const size_t smem = (size_t)kTileLabels * LS * sizeof(float) + (size_t)kReconBins * sizeof(unsigned) +
-                        (EPI == 2 || EPI == 6 ? (size_t)kTileLabels * sizeof(int2) : 0);
-    static bool configured = false;
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(score_fast_kernel<GEOM, DH, RI, NT, 1, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-        configured = true;
-    }
-    a.groups = (a.N + (int64_t)NT * RI - 1) / ((int64_t)NT * RI);
-    const int64_t rows = a.u_end - a.u_begin;
-    int64_t chunks = (kReconTarget + a.groups - 1) / a.groups;
-    int64_t chunk = (rows + chunks - 1) / chunks;
-    if (chunk < 32) chunk = 32;
-    if (chunk > kReconMaxChunk) chunk = kReconMaxChunk;
-    a.chunk = chunk;
-    chunks = (rows + chunk - 1) / chunk;
-    const int64_t blocks = a.groups * chunks;
-    if (blocks > 0x7fffffffLL) return LEC_E_SIZE;
-    score_fast_kernel<GEOM, DH, RI, NT, 1, EPI><<<(unsigned)blocks, NT, smem, st>>>(a);
-    ++g_launches;
-    return (int)cudaGetLastError();
-}
-
-template <int GEOM, int EPI>
-int recon_launch_geom(FastArgs& a, cudaStream_t st) {
-    const int dh = (a.D + 1) / 2;   // the scoring kernel's instantiations (fast_launch_geom)
-    if (dh <= 1) return recon_launch_dh<GEOM, 1, 4, EPI>(a, st);
-    if (dh <= 2) return recon_launch_dh<GEOM, 2, 4, EPI>(a, st);
-    if (dh <= 5) return recon_launch_dh<GEOM, 5, 4, EPI>(a, st);
-    if (dh <= 8) return recon_launch_dh<GEOM, 8, 4, EPI>(a, st);
-    if (dh <= 16) return recon_launch_dh<GEOM, 16, 2, EPI>(a, st);
-    if (dh <= 25) return recon_launch_dh<GEOM, 25, 2, EPI>(a, st);
-    if (dh <= 32) return recon_launch_dh<GEOM, 32, 2, EPI>(a, st);
-    return LEC_E_DIM;
-}
-
 int validate(const lec_recon_t* r) {
-    if (!r || !r->rows || !r->tin || !r->tout || !r->workspace) return LEC_E_NULL;
-    if (r->D < 1 || r->D > 64 || r->ld < r->D || (r->ld != r->D && r->ld % 4 != 0)) return LEC_E_DIM;
-    if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE && r->geom != LEC_GEOM_POINCARE)
-        return LEC_E_ENUM;
-    if (r->n < 0 || r->n > 0x7fffffffLL || r->u_begin < 0 || r->u_end < r->u_begin || r->u_end > r->n) return LEC_E_SIZE;
-    if (batch_of(r->workspace_bytes) < 1) return LEC_E_SIZE;
-    if ((reinterpret_cast<uintptr_t>(r->rows) & 15) || (reinterpret_cast<uintptr_t>(r->workspace) & 15)) return LEC_E_ALIGN;
-    return 0;
+    return eval_validate(r, true, [&] { return batch_of(r->workspace_bytes) < 1 ? LEC_E_SIZE : 0; });
 }
 
 }  // namespace
@@ -409,40 +354,13 @@ extern "C" int lec_recon_pass_heldout(const lec_recon_t* r, const lec_recon_extr
     a.ld = r->ld; a.u_begin = r->u_begin; a.u_end = r->u_end;
     a.tin = r->tin; a.tout = r->tout;
     a.rstate = l.state; a.ropen = l.open; a.rhdr = l.hdr; a.rhist = l.hist;
+    if (dag) { a.xptr = x->ptr; a.xlo = x->lo; a.xhi = x->hi; }
+    if (h) { a.hptr = h->closure_ptr; a.hmap = h->slot_map; a.rxcum = h->xcum; }
     cudaStream_t st = (cudaStream_t)stream;
-    if (h) {  // only pairs below their apex look up the slot map
-        a.hptr = h->closure_ptr; a.hmap = h->slot_map;
-        if (dag) {
-            a.xptr = x->ptr; a.xlo = x->lo; a.xhi = x->hi; a.rxcum = h->xcum;
-            switch (r->geom) {
-                case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 6>(a, st);
-                case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 6>(a, st);
-                case LEC_GEOM_POINCARE: return recon_launch_geom<LEC_GEOM_POINCARE, 6>(a, st);
-                default: return recon_launch_geom<LEC_GEOM_OE, 6>(a, st);
-            }
-        }
-        switch (r->geom) {
-            case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 5>(a, st);
-            case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 5>(a, st);
-            case LEC_GEOM_POINCARE: return recon_launch_geom<LEC_GEOM_POINCARE, 5>(a, st);
-            default: return recon_launch_geom<LEC_GEOM_OE, 5>(a, st);
-        }
-    }
-    if (dag) {  // only apexes with extra intervals leave the forest kernel's instructions
-        a.xptr = x->ptr; a.xlo = x->lo; a.xhi = x->hi;
-        switch (r->geom) {
-            case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 2>(a, st);
-            case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 2>(a, st);
-            case LEC_GEOM_POINCARE: return recon_launch_geom<LEC_GEOM_POINCARE, 2>(a, st);
-            default: return recon_launch_geom<LEC_GEOM_OE, 2>(a, st);
-        }
-    }
-    switch (r->geom) {
-        case LEC_GEOM_EUC: return recon_launch_geom<LEC_GEOM_EUC, 1>(a, st);
-        case LEC_GEOM_HYP: return recon_launch_geom<LEC_GEOM_HYP, 1>(a, st);
-        case LEC_GEOM_POINCARE: return recon_launch_geom<LEC_GEOM_POINCARE, 1>(a, st);
-        default: return recon_launch_geom<LEC_GEOM_OE, 1>(a, st);
-    }
+    // only apexes with extra intervals leave the forest pass's instructions; only pairs below their apex look up the
+    // slot map
+    if (h) return dag ? eval_launch<Pass::F1HeldDag>(r->geom, a, st) : eval_launch<Pass::F1Held>(r->geom, a, st);
+    return dag ? eval_launch<Pass::F1Dag>(r->geom, a, st) : eval_launch<Pass::F1>(r->geom, a, st);
 }
 
 extern "C" int lec_recon_pass_dag(const lec_recon_t* r, const lec_recon_extra_t* x, void* stream) {

@@ -50,24 +50,46 @@ struct FastArgs {
     int32_t* topk_idx; float* topk_val;
     int64_t groups;  // image groups of NT*RI images
     int ring;        // candidate ring entries per thread (> RI)
-    // reconstruction pass (EPI = 1, lec_recon.cu): labels = images = rows, row stride ld; a block evaluates the
-    // apex rows [u_begin + c*chunk, ...) of chunk c against its image group
+    // evaluation passes (Pass below): labels = images = rows, row stride ld; a block evaluates the apex rows
+    // [u_begin + c*chunk, ...) of chunk c against its image group
     int64_t ld, u_begin, u_end, chunk;
     const int32_t* tin; const int32_t* tout;
     const struct ReconState* rstate; const struct ReconOpen* ropen;
     unsigned long long* rhdr; unsigned long long* rhist;
-    // DAG reconstruction pass (EPI = 2): apex u's extra preorder intervals [xlo[i], xhi[i]], i in [xptr[u], xptr[u+1])
+    // extra intervals (DAG): apex u's extra preorder intervals [xlo[i], xhi[i]], i in [xptr[u], xptr[u+1])
     const int32_t* xptr; const int32_t* xlo; const int32_t* xhi;
-    // reconstruction ranks (EPI = 3 positive keys, EPI = 4 negative counts, lec_rank.cu): block chunks index the apex
-    // list rapex[0, *rnapex); apex u's positives own slots [rpos[u], rpos[u+1]); rxcum[i] = slots of u's primary interval
-    // and of its extra intervals before i
+    // rank passes (lec_rank.cu): block chunks index the apex list rapex[0, *rnapex); apex u's positives own slots
+    // [rpos[u], rpos[u+1]); rxcum[i] = slots of u's primary interval and of its extra intervals before i
     const int32_t* rapex; const int* rnapex; const int64_t* rpos; const int32_t* rxcum;
     unsigned* rkey; int32_t* rval; const unsigned* rsorted; unsigned* rcnt; unsigned* req;
-    // held-out evaluation (EPI = 5, 6 F1 pass, EPI = 7 rank keys): apex u's closure pairs own the closure slots
-    // [hptr[u], hptr[u+1]) (the layout of rpos for every closure edge, extra intervals offset by rxcum); hmap[j] is the
-    // held-out slot of closure slot j, -1 for a pair that is neither positive nor negative
+    // held-out passes: apex u's closure pairs own the closure slots [hptr[u], hptr[u+1]) (the layout of rpos for every
+    // closure edge, extra intervals offset by rxcum); hmap[j] is the held-out slot of closure slot j, -1 for a pair that
+    // is neither positive nor negative
     const int64_t* hptr; const int32_t* hmap;
 };
+
+// What a score_fast_kernel instantiation computes.  Score is the scoring kernel (top-k and / or the score matrix); the
+// others are the all-pairs evaluation passes over the same energies, counted instead of stored.  The values appear in
+// the kernels' mangled names.
+//   F1            reconstruction F1 (lec_recon.cu): every pair's energy into the round's histograms
+//   F1Dag         F1 on a DAG: a pair is also positive when tin[v] lies in one of the apex's extra intervals
+//   RankKeys      reconstruction ranks (lec_rank.cu): the rank key of every positive pair into its slot (forest or DAG)
+//   RankCounts    every negative pair at or below its apex's largest positive key into the bucket of its lower bound
+//                 among the apex's sorted positive keys
+//   F1Held, F1HeldDag  F1, F1Dag on a held-out set: a pair below its apex is positive only when its closure slot is
+//                 held out and is skipped otherwise (only those pairs look the slot up); negatives are F1's
+//   RankKeysHeld  RankKeys on a held-out set: the key of a held-out pair into its held-out slot hmap[closure slot]
+enum class Pass : int { Score = 0, F1, F1Dag, RankKeys, RankCounts, F1Held, F1HeldDag, RankKeysHeld };
+__host__ __device__ constexpr bool is_eval(Pass p) { return p != Pass::Score; }
+__host__ __device__ constexpr bool is_rank(Pass p) {
+    return p == Pass::RankKeys || p == Pass::RankCounts || p == Pass::RankKeysHeld;
+}
+__host__ __device__ constexpr bool is_f1(Pass p) { return is_eval(p) && !is_rank(p); }
+// F1 passes with the extra-interval test compiled in (the rank passes test at run time: xptr may be NULL)
+__host__ __device__ constexpr bool has_extra(Pass p) { return p == Pass::F1Dag || p == Pass::F1HeldDag; }
+__host__ __device__ constexpr bool is_held(Pass p) {
+    return p == Pass::F1Held || p == Pass::F1HeldDag || p == Pass::RankKeysHeld;
+}
 
 // Reconstruction check (lec_recon.cu).  Key of an energy = its fp32 bit pattern (energies are >= 0 or NaN, -0 is
 // counted as 0); the coarse round histograms key >> kReconShift, a fine round counts every key of the open coarse bins.
@@ -92,6 +114,21 @@ __device__ __forceinline__ unsigned rank_key(float e) {
     return e != e ? 0x7fc00000u : (k == 0x80000000u ? 0u : k);
 }
 
+// per image: how many of an apex's extra intervals (xlo[xe.x, xe.x + xe.y), sorted starts, xe.y > 0) start at or before
+// tin_v (binary lifting over the starts, the same ceil(log2(count + 1)) steps in every lane)
+template <int RI>
+__device__ __forceinline__ void extra_below(const int32_t* xlo, int2 xe, const int (&tin_v)[RI], int (&below)[RI]) {
+#pragma unroll
+    for (int r = 0; r < RI; ++r) below[r] = 0;
+    for (int s = 1 << (31 - __clz(xe.y)); s > 0; s >>= 1) {
+#pragma unroll
+        for (int r = 0; r < RI; ++r) {
+            const int i = below[r] + s;
+            if (i <= xe.y && __ldg(xlo + xe.x + i - 1) <= tin_v[r]) below[r] = i;
+        }
+    }
+}
+
 // Shared-memory layout of one staged label: DQ float4 chunks of the row (zero padded), then one float4
 // of constants.   hyp: {A, 1+A, A^2, -psi} {cos psi, sin psi, 0, 0}   euc: {A, t0, 0, 0}   oe: unused
 // Label values enter the packed FMAs as scalar-broadcast operands (FFMA2 takes a .F32 operand that
@@ -103,19 +140,11 @@ struct IntC {
     static constexpr int value = V;
 };
 
-// EPI = 1: the reconstruction pass -- the same energies, counted into the lec_recon.cu histograms instead of stored
-// EPI = 2: the same pass on a DAG: a pair is also positive when tin[v] lies in one of the apex's extra intervals
-// EPI = 3: reconstruction ranks, the rank key of every positive pair into its slot (forest or DAG)
-// EPI = 4: reconstruction ranks, every negative pair at or below its apex's largest positive key into the bucket of its
-//          lower bound among the apex's sorted positive keys
-// EPI = 5, 6: EPI = 1, 2 on a held-out set: a pair below its apex is positive only when its closure slot is held out
-//          and is skipped otherwise (only those pairs look the slot up); negatives are those of EPI = 1, 2
-// EPI = 7: EPI = 3 on a held-out set: the key of a held-out pair into its held-out slot hmap[closure slot]
-template <int GEOM, int DH, int RI, int NT, int MINB, int EPI = 0>
+template <int GEOM, int DH, int RI, int NT, int MINB, Pass PASS = Pass::Score>
 __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) {
     static_assert(RI % 2 == 0, "images are packed in pairs");
-    constexpr bool RANK = EPI == 3 || EPI == 4 || EPI == 7;  // rank passes (lec_rank.cu); other EPI > 0: F1 passes
-    constexpr bool XDAG = EPI == 2 || EPI == 6;              // F1 pass with extra intervals
+    constexpr bool EVAL = is_eval(PASS), RANK = is_rank(PASS), F1 = is_f1(PASS), XDAG = has_extra(PASS);
+    constexpr bool HELD = is_held(PASS);
     constexpr int DQ = (DH + 1) / 2;     // float4 chunks per row
     constexpr int LS = 4 * DQ + 8;       // floats per staged label: row chunks + two float4 of constants
     constexpr int NP = RI / 2;           // packed image pairs per thread
@@ -129,13 +158,13 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     const int tid = threadIdx.x;
     const int seg = (int)(blockIdx.x / a.groups);
     const int64_t group = blockIdx.x % a.groups;
-    const int l_begin = EPI ? (int)(a.u_begin + (int64_t)seg * a.chunk) : a.seg_start[seg];
-    const int l_end = EPI ? (int)min(RANK ? (int64_t)*a.rnapex : a.u_end, a.u_begin + (int64_t)(seg + 1) * a.chunk)
+    const int l_begin = EVAL ? (int)(a.u_begin + (int64_t)seg * a.chunk) : a.seg_start[seg];
+    const int l_end = EVAL ? (int)min(RANK ? (int64_t)*a.rnapex : a.u_end, a.u_begin + (int64_t)(seg + 1) * a.chunk)
                           : a.seg_stop[seg];
     if (RANK && l_begin >= l_end) return;  // the grid is sized for every apex row, the list holds those with P_u >= 1
     // row of staged label l: the apex list indexes the rows in the rank passes
     auto label_row = [&](int l) -> int64_t { return RANK ? (int64_t)a.rapex[l] : (int64_t)l; };
-    const int level = EPI ? -1 : a.seg_level[seg];
+    const int level = EVAL ? -1 : a.seg_level[seg];
     const bool want_topk = (level >= 0) && (a.topk_idx != nullptr);
     const int k = a.k;
     const int D = a.D;
@@ -147,8 +176,8 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
 #pragma unroll
     for (int j = 0; j < NP; ++j) {
         const int64_t i0 = img0 + (2 * j) * NT, i1 = img0 + (2 * j + 1) * NT;
-        const float* s0 = a.images + (i0 < a.N ? i0 : 0) * (EPI ? a.ld : (int64_t)D);
-        const float* s1 = a.images + (i1 < a.N ? i1 : 0) * (EPI ? a.ld : (int64_t)D);
+        const float* s0 = a.images + (i0 < a.N ? i0 : 0) * (EVAL ? a.ld : (int64_t)D);
+        const float* s1 = a.images + (i1 < a.N ? i1 : 0) * (EVAL ? a.ld : (int64_t)D);
         float b0 = 0.f, b1 = 0.f;
         double e0 = 0.0, e1 = 0.0;  // Poincare: |y|^2 in fp64, as the labels' A
 #pragma unroll
@@ -185,7 +214,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     // fraction of a percent of the pairs, go straight to global memory); fine rounds = the batch slot of every coarse
     // bin (or -1) in the same shared array.  Zeros, NaNs and the pair counts stay in registers until the block ends.
     unsigned* rsh = reinterpret_cast<unsigned*>(smem + kTileLabels * LS);
-    int2* xsh = reinterpret_cast<int2*>(rsh + kReconBins);  // EPI = 2, 6: [kTileLabels] {first extra interval, count}
+    int2* xsh = reinterpret_cast<int2*>(rsh + kReconBins);  // has_extra: [kTileLabels] {first extra interval, count}
     int rphase = 0;
     int tin_v[RI];
     unsigned c_np = 0, c_nn = 0, c_nanp = 0, c_nann = 0, c_zp = 0, c_zn = 0;
@@ -197,23 +226,20 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     int* rpre = rso + kTileLabels;
     int* rused = rpre + kTileLabels;
     unsigned* rbk = reinterpret_cast<unsigned*>(rused + 4);
-    if (RANK) {
-#pragma unroll
-        for (int r = 0; r < RI; ++r) {
-            const int64_t v = img0 + r * NT;
-            tin_v[r] = v < a.N ? a.tin[v] : 0;
-        }
-        if (EPI == 4)
-            for (int b = tid; b < kRankShared; b += NT) rbk[b] = 0u;
-    }
-    if (EPI && !RANK) {
+    if (F1) {
         rphase = a.rstate->phase;
         if (rphase == 2) return;
+    }
+    if (EVAL) {
 #pragma unroll
         for (int r = 0; r < RI; ++r) {
             const int64_t v = img0 + r * NT;
             tin_v[r] = v < a.N ? a.tin[v] : 0;
         }
+    }
+    if (PASS == Pass::RankCounts)
+        for (int b = tid; b < kRankShared; b += NT) rbk[b] = 0u;
+    if (F1) {
         for (int b = tid; b < kReconBins; b += NT) rsh[b] = rphase == 0 ? 0u : ~0u;
         if (rphase == 1) {
             __syncthreads();
@@ -472,8 +498,8 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         }
     };
 
-    // STORE: 0 no matrix, 1 label-major and every image of the group exists, 2 generic strides / partial group,
-    // 3 reconstruction counts, 4 reconstruction counts with extra intervals (DAG), 5 rank keys, 6 rank counts
+    // STORE (Pass::Score): 0 no matrix, 1 label-major and every image of the group exists, 2 generic strides / partial
+    // group; an evaluation pass counts instead (STORE 0)
     auto tile_loop = [&](int l0, int tl, auto store_c, auto topk_c) {
         constexpr int STORE = decltype(store_c)::value;
         constexpr bool TOPK = decltype(topk_c)::value != 0;
@@ -496,7 +522,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                     const int64_t i = img0 + r * NT;
                     if (i < a.N) row[i * a.s_img] = E[r];
                 }
-            } else if (STORE == 3) {
+            } else if (F1 && !XDAG) {
                 const int u = l0 + t;
                 const int* ue = reinterpret_cast<const int*>(lab + t * LS + 4 * DQ + 6);  // Euler interval of u
                 const int tin_u = ue[0], tout_u = ue[1];
@@ -507,35 +533,26 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                     const bool pos = tin_u < tin_v[r] && tin_v[r] <= tout_u;
                     // held out: a pair below u loads the held-out slot of its closure slot (ue[-1]: u's first one); a
                     // training pair is skipped
-                    if (EPI == 5 && valid && pos && __ldg(a.hmap + ue[-1] + tin_v[r] - tin_u - 1) < 0) valid = false;
+                    if (HELD && valid && pos && __ldg(a.hmap + ue[-1] + tin_v[r] - tin_u - 1) < 0) valid = false;
                     recon_count(E[r], valid, pos);
                 }
-            } else if (STORE == 4) {
+            } else if (XDAG) {
                 const int u = l0 + t;
                 const int* ue = reinterpret_cast<const int*>(lab + t * LS + 4 * DQ + 6);
                 const int tin_u = ue[0], tout_u = ue[1];
                 bool pos[RI];
-                int cs[RI];  // EPI = 6: closure slot of a pair below u
+                int cs[RI];  // held out: closure slot of a pair below u
 #pragma unroll
                 for (int r = 0; r < RI; ++r) {
                     pos[r] = tin_u < tin_v[r] && tin_v[r] <= tout_u;
-                    if (EPI == 6) cs[r] = ue[-1] + tin_v[r] - tin_u - 1;
+                    if (HELD) cs[r] = ue[-1] + tin_v[r] - tin_u - 1;
                 }
                 const int2 xe = xsh[t];
                 if (xe.y > 0) {  // block-uniform: every thread is on apex u
-                    // per image: how many of u's extra intervals start at or before tin_v (binary lifting over the
-                    // sorted starts, the same ceil(log2(count + 1)) steps in every lane), then the end of the last one
+                    // the last extra interval starting at or before tin_v, then its end
                     int below[RI];
-#pragma unroll
-                    for (int r = 0; r < RI; ++r) below[r] = 0;
-                    for (int s = 1 << (31 - __clz(xe.y)); s > 0; s >>= 1) {
-#pragma unroll
-                        for (int r = 0; r < RI; ++r) {
-                            const int i = below[r] + s;
-                            if (i <= xe.y && __ldg(a.xlo + xe.x + i - 1) <= tin_v[r]) below[r] = i;
-                        }
-                    }
-                    if (EPI == 6) {
+                    extra_below(a.xlo, xe, tin_v, below);
+                    if (HELD) {
 #pragma unroll
                         for (int r = 0; r < RI; ++r) {
                             const int i = xe.x + below[r] - 1;
@@ -554,10 +571,11 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 for (int r = 0; r < RI; ++r) {
                     const int64_t v = img0 + r * NT;
                     bool valid = v < a.N && v != u;
-                    if (EPI == 6 && valid && pos[r] && __ldg(a.hmap + cs[r]) < 0) valid = false;  // as EPI = 5
+                    if (HELD && valid && pos[r] && __ldg(a.hmap + cs[r]) < 0) valid = false;  // as F1Held
                     recon_count(E[r], valid, pos[r]);
                 }
-            } else if (STORE == 5 || STORE == 6) {
+            } else if (RANK) {
+                constexpr bool KEYS = PASS != Pass::RankCounts;
                 const int* ue = reinterpret_cast<const int*>(lab + t * LS + 4 * DQ + 6);
                 const int tin_u = ue[0], tout_u = ue[1];
                 const int4 rk = rsk[t];  // {first slot, P_u, smallest key, largest key}
@@ -569,32 +587,24 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                     slot[r] = tin_v[r] - tin_u - 1;
                 }
                 const int2 xe = rxs[t];
-                if (xe.y > 0) {  // block-uniform: EPI = 2's search of the apex's extra intervals
+                if (xe.y > 0) {  // block-uniform: F1Dag's search of the apex's extra intervals
                     int below[RI];
-#pragma unroll
-                    for (int r = 0; r < RI; ++r) below[r] = 0;
-                    for (int s = 1 << (31 - __clz(xe.y)); s > 0; s >>= 1) {
-#pragma unroll
-                        for (int r = 0; r < RI; ++r) {
-                            const int i = below[r] + s;
-                            if (i <= xe.y && __ldg(a.xlo + xe.x + i - 1) <= tin_v[r]) below[r] = i;
-                        }
-                    }
+                    extra_below(a.xlo, xe, tin_v, below);
 #pragma unroll
                     for (int r = 0; r < RI; ++r) {
                         const int i = xe.x + below[r] - 1;
                         if (img0 + r * NT < a.N && below[r] > 0 && tin_v[r] <= __ldg(a.xhi + i)) {
                             pos[r] = true;
-                            if (STORE == 5) slot[r] = __ldg(a.rxcum + i) + tin_v[r] - __ldg(a.xlo + i);
+                            if (KEYS) slot[r] = __ldg(a.rxcum + i) + tin_v[r] - __ldg(a.xlo + i);
                         }
                     }
                 }
-                if (STORE == 5) {
+                if (KEYS) {
 #pragma unroll
                     for (int r = 0; r < RI; ++r) {
                         if (pos[r] && slot[r] < rk.y) {  // a slot past P_u would mean pos_ptr disagrees with the cover
-                            const int j = EPI == 7 ? __ldg(a.hmap + rk.x + slot[r]) : rk.x + slot[r];
-                            if (EPI == 7 && j < 0) continue;  // a training pair
+                            const int j = HELD ? __ldg(a.hmap + rk.x + slot[r]) : rk.x + slot[r];
+                            if (HELD && j < 0) continue;  // a training pair
                             a.rkey[j] = rank_key(E[r]);
                             a.rval[j] = j;
                         }
@@ -666,12 +676,12 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         // ---- stage the tile: rows zero-padded to whole float4 chunks
         for (int i = tid; i < tl * 4 * DQ; i += NT) {
             const int t = i / (4 * DQ), d = i - t * (4 * DQ);
-            lab[t * LS + d] = (d < D) ? __ldg(a.labels + label_row(l0 + t) * (EPI ? a.ld : (int64_t)D) + d) : 0.f;
+            lab[t * LS + d] = (d < D) ? __ldg(a.labels + label_row(l0 + t) * (EVAL ? a.ld : (int64_t)D) + d) : 0.f;
         }
         // ---- per-label constants in fp64 (same terms as lec_rows_fwd's aux)
         if (GEOM != LEC_GEOM_OE) {
             for (int t = tid; t < tl; t += NT) {
-                const float* src = a.labels + label_row(l0 + t) * (EPI ? a.ld : (int64_t)D);
+                const float* src = a.labels + label_row(l0 + t) * (EVAL ? a.ld : (int64_t)D);
                 double A = 0.0;
                 for (int d = 0; d < D; ++d) { const double v = (double)__ldg(src + d); A += v * v; }
                 const Aux<double> x = row_aux<double>(GEOM, A, a.K);
@@ -689,33 +699,30 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 *reinterpret_cast<float4*>(lab + t * LS + 4 * DQ + 4) = c2;
             }
         }
-        if (EPI) {  // the apex's Euler interval in the last two constant slots (after the stores above, same thread)
+        if (EVAL) {  // the apex's Euler interval in the last two constant slots (after the stores above, same thread)
             for (int t = tid; t < tl; t += NT) {
                 int* ue = reinterpret_cast<int*>(lab + t * LS + 4 * DQ + 6);
-                if (!RANK) {
-                    ue[0] = a.tin[l0 + t];
-                    ue[1] = a.tout[l0 + t];
-                }
-                if (EPI == 5 || EPI == 6) ue[-1] = (int)a.hptr[l0 + t];  // the deferred top-k's sin(psi) slot
+                const int64_t u = label_row(l0 + t);
+                ue[0] = a.tin[u];
+                ue[1] = a.tout[u];
+                if (F1 && HELD) ue[-1] = (int)a.hptr[u];  // the deferred top-k's sin(psi) slot
                 if (XDAG) {
-                    const int x0 = a.xptr[l0 + t];
-                    xsh[t] = make_int2(x0, a.xptr[l0 + t + 1] - x0);
+                    const int x0 = a.xptr[u];
+                    xsh[t] = make_int2(x0, a.xptr[u + 1] - x0);
                 }
                 if (RANK) {
-                    const int64_t u = label_row(l0 + t);
-                    ue[0] = a.tin[u];
-                    ue[1] = a.tout[u];
                     const int x0 = a.xptr ? a.xptr[u] : 0;
                     rxs[t] = make_int2(x0, a.xptr ? a.xptr[u + 1] - x0 : 0);
-                    const int64_t* sp = EPI == 7 ? a.hptr : a.rpos;  // EPI = 7 walks the closure slots
-                    const int base = (int)sp[u], P = (int)(sp[u + 1] - base);
-                    rsk[t] = EPI == 4 ? make_int4(base, P, (int)a.rsorted[base], (int)a.rsorted[base + P - 1])
-                                      : make_int4(base, P, 0, 0);
+                    const int64_t* sp = HELD ? a.hptr : a.rpos;  // RankKeysHeld walks the closure slots
+                    const int base = (int)sp[u], n = (int)(sp[u + 1] - base);
+                    rsk[t] = PASS == Pass::RankCounts
+                                 ? make_int4(base, n, (int)a.rsorted[base], (int)a.rsorted[base + n - 1])
+                                 : make_int4(base, n, 0, 0);
                 }
             }
         }
         __syncthreads();
-        if (EPI == 4) {
+        if (PASS == Pass::RankCounts) {
             // shared buckets for the tile's apexes in order while their P_u sum stays within kRankShared; an apex
             // larger than that, and every apex after the budget is spent, counts in global memory
             if (tid < 32) {
@@ -724,8 +731,8 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
 #pragma unroll
                 for (int j = 0; j < 3; ++j) {
                     const int t = 3 * tid + j;
-                    const int P = t < tl ? rsk[t].y : 0;
-                    s[j] = P <= kRankShared ? P : 0;
+                    const int n = t < tl ? rsk[t].y : 0;
+                    s[j] = n <= kRankShared ? n : 0;
                     loc += s[j];
                 }
                 int inc = loc;
@@ -761,8 +768,8 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
             refresh_filter();
         }
         if (RANK) {
-            tile_loop(l0, tl, IntC<EPI == 4 ? 6 : 5>(), IntC<0>());
-            if (EPI == 4) {  // flush the tile's non-zero buckets and clear them for the next tile
+            tile_loop(l0, tl, IntC<0>(), IntC<0>());
+            if (PASS == Pass::RankCounts) {  // flush the tile's non-zero buckets and clear them for the next tile
                 __syncthreads();
                 const int used = *rused;
                 for (int i = tid; i < used; i += NT) {
@@ -780,8 +787,8 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                     if (c >> 16) atomicAdd(a.req + g, c >> 16);
                 }
             }
-        } else if (EPI) {
-            tile_loop(l0, tl, IntC<XDAG ? 4 : 3>(), IntC<0>());
+        } else if (F1) {
+            tile_loop(l0, tl, IntC<0>(), IntC<0>());
         } else if (want_topk) {
             if (store == 0 && GEOM == LEC_GEOM_HYP) tile_loop_deferred(l0, tl);
             else if (store == 0) tile_loop(l0, tl, IntC<0>(), IntC<1>());
@@ -794,7 +801,7 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     }
 
     if (RANK) return;
-    if (EPI) {
+    if (F1) {
         // register counters: one global add per warp; then the block's coarse negatives
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
@@ -849,13 +856,20 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
     }
 }
 
-// arguments of a held-out set (lec_rank_run_heldout, lec_recon_pass_heldout); xcum is needed with extra intervals.
-// closure_ptr[n] == n_closure is the caller's to keep, like pos_ptr's agreement with the cover: reading it would
-// synchronise.
-inline int heldout_validate(const lec_heldout_t* h, bool dag) {
-    if (!h->closure_ptr || !h->slot_map || (dag && !h->xcum)) return LEC_E_NULL;
-    if (h->n_closure < 0 || h->n_closure > 0x7fffffffLL) return LEC_E_SIZE;
-    return 0;
+// The <DH, RI> instantiation for a row width D, f(IntC<DH>(), IntC<RI>()): the scoring kernel and every evaluation pass
+// share it, because the energy bits depend on RI (through the accumulator split of dots), and so every evaluation pass
+// equals the SIMT score matrix bit for bit.
+template <typename F>
+static int dispatch_width(int D, F&& f) {
+    const int dh = (D + 1) / 2;
+    if (dh <= 1) return f(IntC<1>(), IntC<4>());
+    if (dh <= 2) return f(IntC<2>(), IntC<4>());
+    if (dh <= 5) return f(IntC<5>(), IntC<4>());
+    if (dh <= 8) return f(IntC<8>(), IntC<4>());
+    if (dh <= 16) return f(IntC<16>(), IntC<2>());
+    if (dh <= 25) return f(IntC<25>(), IntC<2>());
+    if (dh <= 32) return f(IntC<32>(), IntC<2>());
+    return LEC_E_DIM;
 }
 
 // 128-thread blocks whose register allocation need only allow one resident block per SM; a thread holds RI images.
@@ -884,15 +898,91 @@ static int fast_launch_dh(FastArgs& a, cudaStream_t st) {
 
 template <int GEOM>
 static int fast_launch_geom(FastArgs& a, cudaStream_t st) {
-    const int dh = (a.D + 1) / 2;
-    if (dh <= 1) return fast_launch_dh<GEOM, 1, 4>(a, st);
-    if (dh <= 2) return fast_launch_dh<GEOM, 2, 4>(a, st);
-    if (dh <= 5) return fast_launch_dh<GEOM, 5, 4>(a, st);
-    if (dh <= 8) return fast_launch_dh<GEOM, 8, 4>(a, st);
-    if (dh <= 16) return fast_launch_dh<GEOM, 16, 2>(a, st);
-    if (dh <= 25) return fast_launch_dh<GEOM, 25, 2>(a, st);
-    if (dh <= 32) return fast_launch_dh<GEOM, 32, 2>(a, st);
-    return LEC_E_DIM;
+    return dispatch_width(a.D, [&](auto dh, auto ri) {
+        return fast_launch_dh<GEOM, decltype(dh)::value, decltype(ri)::value>(a, st);
+    });
+}
+
+// Evaluation passes: one block per SM (128 KB of shared counters in the F1 passes), 16 warps where the image rows fit
+// 128 registers, else 8 (D > 32 spills at 512 threads).  The block size does not change the energy bits.
+constexpr int eval_threads(int dh) { return dh > 16 ? 256 : 512; }
+constexpr int kEvalTarget = 148 * 16;    // blocks per pass to aim for (16 waves: the chunks balance)
+constexpr int64_t kEvalMaxChunk = 4096;  // apex rows per block: the F1 passes' 32-bit shared counters cannot overflow
+
+// dynamic shared memory of an evaluation pass: the staged tile, then the F1 passes' coarse counters (and the extra
+// intervals of the staged apexes) or the rank passes' per-apex table (and the count's buckets)
+constexpr size_t eval_smem_bytes(Pass p, int dh) {
+    return (size_t)kTileLabels * (4 * ((dh + 1) / 2) + 8) * sizeof(float) +
+           (is_rank(p) ? (size_t)kTileLabels * (sizeof(int4) + sizeof(int2) + 2 * sizeof(int)) + 4 * sizeof(int) +
+                             (p == Pass::RankCounts ? (size_t)kRankShared * sizeof(unsigned) : 0)
+                       : (size_t)kReconBins * sizeof(unsigned) + (has_extra(p) ? (size_t)kTileLabels * sizeof(int2) : 0));
+}
+
+// one pass over the apex rows [u_begin, u_end) (the rank passes: entries of the apex list, u_begin = 0)
+template <int GEOM, int DH, int RI, Pass P>
+static int eval_launch_dh(FastArgs& a, cudaStream_t st) {
+    constexpr int NT = eval_threads(DH);
+    constexpr size_t smem = eval_smem_bytes(P, DH);
+    static bool configured = false;
+    if (!configured) {
+        cudaError_t e = cudaFuncSetAttribute(score_fast_kernel<GEOM, DH, RI, NT, 1, P>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return (int)e;
+        configured = true;
+    }
+    a.groups = (a.N + (int64_t)NT * RI - 1) / ((int64_t)NT * RI);
+    const int64_t rows = a.u_end - a.u_begin;  // rank passes: an upper bound on the apex list; blocks past its end return
+    int64_t chunks = (kEvalTarget + a.groups - 1) / a.groups;
+    int64_t chunk = (rows + chunks - 1) / chunks;
+    if (chunk < 32) chunk = 32;
+    if (chunk > kEvalMaxChunk) chunk = kEvalMaxChunk;
+    a.chunk = chunk;
+    chunks = (rows + chunk - 1) / chunk;
+    const int64_t blocks = a.groups * chunks;
+    if (blocks > 0x7fffffffLL) return LEC_E_SIZE;
+    score_fast_kernel<GEOM, DH, RI, NT, 1, P><<<(unsigned)blocks, NT, smem, st>>>(a);
+    ++g_launches;
+    return (int)cudaGetLastError();
+}
+
+template <int GEOM, Pass P>
+static int eval_launch_geom(FastArgs& a, cudaStream_t st) {
+    return dispatch_width(a.D, [&](auto dh, auto ri) {
+        return eval_launch_dh<GEOM, decltype(dh)::value, decltype(ri)::value, P>(a, st);
+    });
+}
+
+// evaluation pass P for a geometry the caller has validated
+template <Pass P>
+static int eval_launch(int geom, FastArgs& a, cudaStream_t st) {
+    switch (geom) {
+        case LEC_GEOM_EUC: return eval_launch_geom<LEC_GEOM_EUC, P>(a, st);
+        case LEC_GEOM_HYP: return eval_launch_geom<LEC_GEOM_HYP, P>(a, st);
+        case LEC_GEOM_POINCARE: return eval_launch_geom<LEC_GEOM_POINCARE, P>(a, st);
+        default: return eval_launch_geom<LEC_GEOM_OE, P>(a, st);
+    }
+}
+
+// Checks of the fields lec_recon_t and lec_rank_t share, in the order their entry points apply them: NULL (`set`: the
+// caller's own pointers are set), DIM, ENUM, SIZE, then the caller's own checks `more()`, then ALIGN.
+template <typename T, typename F>
+static int eval_validate(const T* r, bool set, F&& more) {
+    if (!r || !r->rows || !r->tin || !r->tout || !r->workspace || !set) return LEC_E_NULL;
+    if (r->D < 1 || r->D > 64 || r->ld < r->D || (r->ld != r->D && r->ld % 4 != 0)) return LEC_E_DIM;
+    if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE && r->geom != LEC_GEOM_POINCARE)
+        return LEC_E_ENUM;
+    if (r->n < 0 || r->n > 0x7fffffffLL || r->u_begin < 0 || r->u_end < r->u_begin || r->u_end > r->n) return LEC_E_SIZE;
+    if (const int e = more()) return e;
+    if ((reinterpret_cast<uintptr_t>(r->rows) & 15) || (reinterpret_cast<uintptr_t>(r->workspace) & 15)) return LEC_E_ALIGN;
+    return 0;
+}
+
+// arguments of a held-out set (lec_rank_run_heldout, lec_recon_pass_heldout); xcum is needed with extra intervals.
+// closure_ptr[n] == n_closure is the caller's to keep, like pos_ptr's agreement with the cover: reading it would
+// synchronise.
+inline int heldout_validate(const lec_heldout_t* h, bool dag) {
+    if (!h->closure_ptr || !h->slot_map || (dag && !h->xcum)) return LEC_E_NULL;
+    if (h->n_closure < 0 || h->n_closure > 0x7fffffffLL) return LEC_E_SIZE;
+    return 0;
 }
 
 }  // namespace lec

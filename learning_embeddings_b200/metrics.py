@@ -146,15 +146,11 @@ def _recon_rounds(rows, hierarchy, geom, K, D, group, workspace_bytes, stats, he
     out = torch.empty(7, device=dev, dtype=torch.float64)
     status = torch.zeros(4, device=dev, dtype=torch.int64)
     stream = N.stream_ptr(dev)
+    x = None if cov.x is None else ctypes.byref(cov.x)
+    h = None if held is None else ctypes.byref(held.h)
     rounds = 0
     while True:
-        if held is not None:
-            N.check(lib.lec_recon_pass_heldout(ctypes.byref(r), None if cov.x is None else ctypes.byref(cov.x),
-                                               ctypes.byref(held.h), stream), "lec_recon_pass_heldout")
-        elif n_extra:
-            N.check(lib.lec_recon_pass_dag(ctypes.byref(r), ctypes.byref(cov.x), stream), "lec_recon_pass_dag")
-        else:
-            N.check(lib.lec_recon_pass(ctypes.byref(r), stream), "lec_recon_pass")
+        N.check(lib.lec_recon_pass_heldout(ctypes.byref(r), x, h, stream), "lec_recon_pass_heldout")
         rounds += 1
         if group is not None:
             dist.all_reduce(ws[:cb].view(torch.int64), group=group)
@@ -245,11 +241,8 @@ def _rank_run(rows, hierarchy, geom, K, D, group, return_ranks, stats, time_stag
     sums = torch.zeros(3, device=dev, dtype=torch.int64)
     ap = torch.zeros(n, device=dev, dtype=torch.float64)
     ranks = torch.zeros((n_edges, 2), device=dev, dtype=torch.int32) if return_ranks else None
-    if held is None:
-        N.check(lib.lec_rank_run(ctypes.byref(r), N._p(sums), N._p(ap), N._p(ranks), N.stream_ptr(dev)), "lec_rank_run")
-    else:
-        N.check(lib.lec_rank_run_heldout(ctypes.byref(r), ctypes.byref(held.h), N._p(sums), N._p(ap), N._p(ranks),
-                                         N.stream_ptr(dev)), "lec_rank_run_heldout")
+    N.check(lib.lec_rank_run_heldout(ctypes.byref(r), None if held is None else ctypes.byref(held.h), N._p(sums),
+                                     N._p(ap), N._p(ranks), N.stream_ptr(dev)), "lec_rank_run_heldout")
     if group is not None:
         for t in (sums, ap) if ranks is None else (sums, ap, ranks):
             dist.all_reduce(t, group=group)

@@ -36,15 +36,15 @@ def gpu_info():
     return {"gpu": name, "power_limit": power, "max_sm_clock": clock}
 
 
-def pass_kernel_sass(DH, NT, EPI=1):
-    """Static instructions of the tile loop of score_fast_kernel<HYP, DH, ., NT, 1, EPI> (unrolled twice: 2 labels x RI
-    images per trip) from cuobjdump -sass of the built object.  With EPI = 2 the loop holds, per label, the
-    block-uniform branch of apexes with extra intervals and its binary-search loop, summarised separately."""
+def pass_kernel_sass(DH, NT, PASS=1):
+    """Static instructions of the tile loop of score_fast_kernel<HYP, DH, ., NT, 1, Pass(PASS)> (PASS = 1: Pass::F1,
+    2: Pass::F1Dag; unrolled twice: 2 labels x RI images per trip) from cuobjdump -sass of the built object.  With
+    Pass::F1Dag the loop holds, per label, the block-uniform branch of apexes with extra intervals and its binary-search loop, summarised separately."""
     obj = os.path.join(ROOT, "learning_embeddings_b200", "csrc", "build", "lec_recon.o")
     sass = subprocess.run(["cuobjdump", "-sass", obj], capture_output=True, text=True).stdout
     sym = "_ZN3lec17score_fast_kernelILi1ELi%dELi" % DH
     blocks = sass.split("Function : ")
-    body = next(b for b in blocks if b.startswith(sym) and b.split("\n", 1)[0].endswith("ELi%dELi1ELi%dEEEvNS_8FastArgsE" % (NT, EPI)))
+    body = next(b for b in blocks if b.startswith(sym) and b.split("\n", 1)[0].endswith("ELi%dELi1ELNS_4PassE%dEEEvNS_8FastArgsE" % (NT, PASS)))
     ins = []
     for line in body.splitlines():
         m = re.match(r"\s+/\*([0-9a-f]{4,})\*/\s+(.*?);", line)
@@ -57,14 +57,14 @@ def pass_kernel_sass(DH, NT, EPI=1):
         if m and int(m.group(1), 16) < a and int(m.group(1), 16) in addr:
             loops.append((addr[int(m.group(1), 16)], i))
     ffma2 = lambda se: sum("FFMA2" in ins[k][1] for k in range(se[0], se[1] + 1))  # noqa: E731
-    # innermost among the loops that do arithmetic (EPI = 2's search loops hold no FFMA2 and sit inside the tile loop)
+    # innermost among the loops that do arithmetic (F1Dag's search loops hold no FFMA2 and sit inside the tile loop)
     inner = [(s, e) for s, e in loops
              if not any(s <= s2 and e2 <= e and (s2, e2) != (s, e) and ffma2((s2, e2)) for s2, e2 in loops)]
     s, e = max(inner, key=ffma2)
     body = [t for _, t in ins[s:e + 1]]
     rec = {"loop_instructions": len(body), "ffma2": sum("FFMA2" in t for t in body),
            "mufu": sum("MUFU" in t for t in body), "atomics": sum(("ATOM" in t or "RED" in t) for t in body)}
-    if EPI == 2:
+    if PASS == 2:
         search = [(s2, e2) for s2, e2 in loops if s <= s2 and e2 <= e and (s2, e2) != (s, e)]
         rec["search_loops"] = len(search)
         rec["search_loop_instructions"] = [e2 - s2 + 1 for s2, e2 in search]
@@ -182,7 +182,7 @@ def main():
     h = H.random_dag(82115, 1.0831, 0.02)
     rows, D = trained(h, 50, args.cfg4_steps)
     lines.append(workload("cfg4dag002_hyp_D50_trained%d" % args.cfg4_steps, h, rows, D, args, info,
-                          pass_kernel_sass(25, 256, EPI=2)))
+                          pass_kernel_sass(25, 256, PASS=2)))
     lines[-1]["pair_evals_per_s_vs_cfg4_tree"] = lines[-1]["pair_evals_per_s"] / lines[-2]["pair_evals_per_s"]
     out = open(args.out, "w") if args.out else None
     for rec in lines:
