@@ -43,6 +43,15 @@ extern "C" {
  * lec_pairs_poincare / lec_cone_step, scored by lec_score_topk(_ex) (LEC_PREC_F32) and the lec_recon_* / lec_rank_*
  * passes; lec_pairs_flat, lec_pairs_grouped, lec_energy_dense(_bwd) and the tensor-core scoring return LEC_E_ENUM. */
 #define LEC_GEOM_POINCARE 4
+/* Lorentz (hyperboloid) distance of Nickel & Kiela 2018, the same hyperbolic space as LEC_GEOM_POINCARE in the chart
+ * that stays accurate far from the origin.  A table row is the SPATIAL part x in R^D of the hyperboloid point
+ * (x0, x), x0 = sqrt(1 + |x|^2) implied and formed in fp64; every row is a valid point.  With A = |x|^2, B = |y|^2,
+ * s = |x-y|^2 (summed from the differences):
+ *     w = -<X,Y>_L - 1 = (s - (A - B)^2 / (x0 + y0)^2) / 2  (clamped at 0),   d = arcosh(1 + w)
+ * symmetric, d = 0 for x == y; d equals the Poincare distance of x / (1 + x0).  Trained by lec_pairs_lorentz /
+ * lec_cone_step, scored by lec_score_topk(_ex) (LEC_PREC_F32) and the lec_recon_* / lec_rank_* passes;
+ * lec_pairs_flat, lec_pairs_grouped, lec_energy_dense(_bwd) and the tensor-core scoring return LEC_E_ENUM. */
+#define LEC_GEOM_LORENTZ 5
 
 /* per-row transform applied to the raw parameter rows (Embedder.forward / FeatNet tail) */
 #define LEC_ROWS_NONE          0 /* plain nn.Embedding lookup (order embeddings) */
@@ -172,6 +181,16 @@ int lec_pairs_poincare(int precision, const float* rows, int64_t n_rows, int D, 
                        const void* pos_to, const void* neg_to, int idx_bytes, int64_t B, int N, float* E_pos,
                        float* E_neg, double* loss_out, float* grad_rows, int grad_replicas, void* stream);
 
+/* The same softmax loss on the Lorentz distance (LEC_GEOM_LORENTZ, Nickel & Kiela 2018), with the parameters, outputs,
+ * team sizing and index checks of lec_pairs_poincare.  rows [n_rows, ld] are spatial parts of hyperboloid points (any
+ * vector is one).  Only LEC_PREC_F64CORE: A, B, s, A - B = <x - y, x + y>, x0 = sqrt(1 + A), y0 and w in fp64 from
+ * the fp32 rows (the difference form of w above: x0 y0 - 1 - <x,y> loses every digit for nearby points far from the
+ * origin; with A - B summed from the differences |dw| <= (3D + 12) 2^-53 s), and
+ *     dd/dx = (y0 / x0 x - y) / r,  dd/dy = (x0 / y0 y - x) / r,  r = sqrt(w (w + 2)),  both 0 where w = 0. */
+int lec_pairs_lorentz(int precision, const float* rows, int64_t n_rows, int D, int ld, const void* pos_from,
+                      const void* pos_to, const void* neg_to, int idx_bytes, int64_t B, int N, float* E_pos,
+                      float* E_neg, double* loss_out, float* grad_rows, int grad_replicas, void* stream);
+
 /* Dense operands (no gather): E_operator(x, y) on arbitrary [P, D] tensors, as the reference calls
  * it from check_graph_embedding (order_embeddings.py:550-551) and the scoring loops. */
 int lec_energy_dense(int geom, int precision, const float* x, const float* y, int64_t P, int D, float K,
@@ -208,6 +227,12 @@ int lec_rsgd_update(float* table, const float* grad, int grad_replicas, int64_t 
  *                      proj rescales a row with |w| >= 1 - 1e-5 to norm 1 - 1e-5 (no inner radius, none of LEC_UPD_RSGD's
  *                      +1e-15 / +1e-6 offsets); grad_out receives the rescaled gradient.  row_mode must be
  *                      LEC_ROWS_NONE (LEC_E_ENUM otherwise); rows_out is then the updated row, padded
+ *        LEC_UPD_RSGD_LORENTZ  Nickel & Kiela 2018's Riemannian SGD on the hyperboloid (exponential map), in the
+ *                      spatial chart of LEC_GEOM_LORENTZ: with g the row's summed gradient and c = <x,g>,
+ *                      r = g + c x,  nu = sqrt(|g|^2 + c^2) (the Lorentz norm of the tangent vector),  t = lr nu,
+ *                      x <- cosh(t) x - lr (sinh(t) / t) r  (row unchanged where nu = 0).  Scalars and the new row in
+ *                      fp64, no clipping of t; grad_out receives r.  geom must be LEC_GEOM_LORENTZ, row_mode
+ *                      LEC_ROWS_NONE and aux_out NULL (LEC_E_ENUM otherwise); rows_out is then the updated row, padded
  *      hyp_rescale != 0 multiplies the gradient by ((1 - |w|) / 2)^2 first (oe_h.py:1766, :1770) and
  *      project_shell != 0 projects the updated row into [r_in, 1 - 1e-5] afterwards (soft_clip, oe_h.py:1771) --
  *      together with LEC_UPD_ADAM that is the reference's default joint hyperbolic update.  RSGD includes both.
@@ -227,6 +252,7 @@ int lec_rsgd_update(float* table, const float* grad, int grad_replicas, int64_t 
 #define LEC_UPD_SGD  2
 #define LEC_UPD_ADAM 3
 #define LEC_UPD_RSGD_RETRACT 4
+#define LEC_UPD_RSGD_LORENTZ 5
 typedef struct lec_update {
     int rule, row_mode, geom, lambda_mode /* RSGD: 0 reference 2/(1-|x|) (SURVEY F4), 1 textbook 2/(1-|x|^2) */;
     int hyp_rescale, project_shell;
@@ -293,6 +319,7 @@ int lec_update_rows(const lec_update_t* u, const lec_exchange_t* x /* NULL or wo
  * geom == LEC_GEOM_POINCARE: the pair kernel is lec_pairs_poincare (precision LEC_PREC_F64CORE, upd.row_mode
  * LEC_ROWS_NONE, upd.aux_out NULL, w_pos = w_neg = NULL, else LEC_E_ENUM), E_neg is [B, N], alpha and upd.K
  * are ignored and neg_from is not read (with lec_host_pipe_submit's Philox draw it is drawn and ignored).
+ * geom == LEC_GEOM_LORENTZ: the same with lec_pairs_lorentz as the pair kernel.
  */
 typedef struct lec_step {
     int geom, precision, fused;
@@ -348,7 +375,11 @@ int lec_score_topk(int geom, int precision, const float* labels, int64_t L, cons
  *                           transposed view, i.e. still indexed scores[i, l].
  * level ranges must be ascending and disjoint.
  * LEC_GEOM_POINCARE: LEC_PREC_F32 and D <= 64 only (LEC_E_ENUM / LEC_E_DIM otherwise); E = d(label, image) evaluated
- * in fp32 from <x,y> and the row norms (|x-y|^2 = max(|x|^2 + |y|^2 - 2<x,y>, 0)), K ignored. */
+ * in fp32 from <x,y> and the row norms (|x-y|^2 = max(|x|^2 + |y|^2 - 2<x,y>, 0)), K ignored.
+ * LEC_GEOM_LORENTZ: the same restrictions; with e = x0 - 1 = A / (1 + x0) and x0 formed per row in fp64 and rounded
+ * to fp32, w = max(e_x y0 + (e_y - <x,y>), 0) in fp32 and E = log1p(w + sqrt(w (w + 2))), K ignored.  Its error
+ * against fp64 d is the rounding of w, |dw| <= (D + 8) 2^-24 (x0 y0 - 1 + |x||y|), mapped through arcosh(1 + w), plus
+ * a few ulp of the final functions (DESIGN.md); w must stay below ~1e19 (hyperbolic radii summing to ~45). */
 #define LEC_SCORES_IMAGE_MAJOR 0
 #define LEC_SCORES_LABEL_MAJOR 1
 int lec_score_topk_ex(int geom, int precision, const float* labels, int64_t L, const float* images,

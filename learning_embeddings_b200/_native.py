@@ -11,7 +11,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_lib", "liblec_b200.so")
 
-GEOM = {"euc": 0, "hyp": 1, "oe": 2, "poincare": 4}
+GEOM = {"euc": 0, "hyp": 1, "oe": 2, "poincare": 4, "lorentz": 5}
 ROWS_NONE, ROWS_EUC_SOFTCLIP, ROWS_HYP_SHELL, ROWS_HYP_TANH, ROWS_HYP_TANH_FEAT = 0, 1, 2, 3, 4
 PREC_F32, PREC_F64CORE = 0, 1
 ABI_VERSION = 14
@@ -19,7 +19,7 @@ ABI_VERSION = 14
 EXPORTS = (
     "lec_abi_version", "lec_error_string", "lec_launch_count", "lec_set_pdl", "lec_index_errors", "lec_rows_fwd", "lec_rows_bwd",
     "lec_featnet_supported", "lec_featnet_fwd", "lec_featnet_wgrad",
-    "lec_reduce_replicas", "lec_pairs_flat", "lec_pairs_grouped", "lec_pairs_poincare", "lec_energy_dense", "lec_energy_dense_bwd",
+    "lec_reduce_replicas", "lec_pairs_flat", "lec_pairs_grouped", "lec_pairs_poincare", "lec_pairs_lorentz", "lec_energy_dense", "lec_energy_dense_bwd",
     "lec_rsgd_update", "lec_exchange_packets", "lec_exchange_bytes", "lec_update_rows", "lec_cone_step", "lec_score_topk", "lec_score_topk_ex",
     "lec_score_tc_supported",
     "lec_score_workspace_bytes", "lec_score_topk_tc", "lec_mt_seed", "lec_mt_uint32", "lec_mt_randbelow",
@@ -116,7 +116,7 @@ class LecHeldout(ctypes.Structure):
                 ("n_closure", ctypes.c_int64)]
 
 
-UPD_NONE, UPD_RSGD, UPD_SGD, UPD_ADAM, UPD_RSGD_RETRACT = 0, 1, 2, 3, 4
+UPD_NONE, UPD_RSGD, UPD_SGD, UPD_ADAM, UPD_RSGD_RETRACT, UPD_RSGD_LORENTZ = 0, 1, 2, 3, 4, 5
 XCHG_ONE_SHOT, XCHG_TWO_SHOT = 0, 1
 
 _lib = None
@@ -153,6 +153,8 @@ def lib():
                                         c_vp, c_vp, c_f, c_f, c_vp, c_vp, c_vp, c_vp, c_i, c_vp]
         L.lec_pairs_poincare.argtypes = [c_i, c_vp, c_i64, c_i, c_i, c_vp, c_vp, c_vp, c_i, c_i64, c_i, c_vp, c_vp, c_vp,
                                          c_vp, c_i, c_vp]
+        L.lec_pairs_lorentz.argtypes = [c_i, c_vp, c_i64, c_i, c_i, c_vp, c_vp, c_vp, c_i, c_i64, c_i, c_vp, c_vp, c_vp,
+                                        c_vp, c_i, c_vp]
         L.lec_energy_dense.argtypes = [c_i, c_i, c_vp, c_vp, c_i64, c_i, c_f, c_vp, c_vp]
         L.lec_energy_dense_bwd.argtypes = [c_i, c_i, c_vp, c_vp, c_vp, c_i64, c_i, c_f, c_vp, c_vp, c_vp]
         L.lec_rsgd_update.argtypes = [c_vp, c_vp, c_i, c_i64, c_i, c_i, c_f, c_f, c_i, c_vp, c_vp]

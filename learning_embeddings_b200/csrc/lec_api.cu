@@ -164,9 +164,10 @@ int lec_pairs_flat(int geom, int precision, const float* rows, const double* aux
     }
 }
 
-int lec_pairs_poincare(int precision, const float* rows, int64_t n_rows, int D, int ld, const void* pos_from, const void* pos_to,
-                       const void* neg_to, int idx_bytes, int64_t B, int N, float* E_pos, float* E_neg, double* loss_out,
-                       float* grad_rows, int grad_replicas, void* stream) {
+// lec_pairs_poincare and lec_pairs_lorentz: the same checks, the same kernel with the distance as a policy
+static int pairs_softmax(int geom, int precision, const float* rows, int64_t n_rows, int D, int ld, const void* pos_from,
+                         const void* pos_to, const void* neg_to, int idx_bytes, int64_t B, int N, float* E_pos, float* E_neg,
+                         double* loss_out, float* grad_rows, int grad_replicas, void* stream) {
     if (precision != LEC_PREC_F64CORE || (idx_bytes != 2 && idx_bytes != 4 && idx_bytes != 8)) return LEC_E_ENUM;
     if (B < 0 || N < 0 || n_rows < 0) return LEC_E_SIZE;
     if (int e = check_rows(rows, D, ld)) return e;
@@ -175,9 +176,24 @@ int lec_pairs_poincare(int precision, const float* rows, int64_t n_rows, int D, 
     if (B == 0) return 0;
     if (!pos_from || !pos_to || !E_pos) return LEC_E_NULL;
     if (N > 0 && (!neg_to || !E_neg)) return LEC_E_NULL;
-    PoincareArgs a{rows, ld, pos_from, pos_to, neg_to, idx_bytes, B, N, E_pos, E_neg, loss_out, grad_rows, grad_replicas,
-                   n_rows * (int64_t)ld, n_rows, index_errors_ptr(), (D - (ld / 4 - 1) * 4) <= 2 ? 1 : 0};
-    return launch_pairs_poincare(a, (cudaStream_t)stream);
+    SoftmaxArgs a{rows, ld, pos_from, pos_to, neg_to, idx_bytes, B, N, E_pos, E_neg, loss_out, grad_rows, grad_replicas,
+                  n_rows * (int64_t)ld, n_rows, index_errors_ptr(), (D - (ld / 4 - 1) * 4) <= 2 ? 1 : 0};
+    return geom == LEC_GEOM_LORENTZ ? launch_pairs_lorentz(a, (cudaStream_t)stream)
+                                    : launch_pairs_poincare(a, (cudaStream_t)stream);
+}
+
+int lec_pairs_poincare(int precision, const float* rows, int64_t n_rows, int D, int ld, const void* pos_from, const void* pos_to,
+                       const void* neg_to, int idx_bytes, int64_t B, int N, float* E_pos, float* E_neg, double* loss_out,
+                       float* grad_rows, int grad_replicas, void* stream) {
+    return pairs_softmax(LEC_GEOM_POINCARE, precision, rows, n_rows, D, ld, pos_from, pos_to, neg_to, idx_bytes, B, N, E_pos,
+                         E_neg, loss_out, grad_rows, grad_replicas, stream);
+}
+
+int lec_pairs_lorentz(int precision, const float* rows, int64_t n_rows, int D, int ld, const void* pos_from, const void* pos_to,
+                      const void* neg_to, int idx_bytes, int64_t B, int N, float* E_pos, float* E_neg, double* loss_out,
+                      float* grad_rows, int grad_replicas, void* stream) {
+    return pairs_softmax(LEC_GEOM_LORENTZ, precision, rows, n_rows, D, ld, pos_from, pos_to, neg_to, idx_bytes, B, N, E_pos,
+                         E_neg, loss_out, grad_rows, grad_replicas, stream);
 }
 
 int lec_pairs_grouped(int geom, int precision, const float* rows, const double* aux, int64_t n_rows, int D, int ld, const void* pos_from,
@@ -248,9 +264,11 @@ int lec_rsgd_update(float* table, const float* grad, int grad_replicas, int64_t 
 
 static int check_update(const lec_update_t* u) {
     if (!u) return LEC_E_NULL;
-    if (u->rule < LEC_UPD_NONE || u->rule > LEC_UPD_RSGD_RETRACT) return LEC_E_ENUM;
+    if (u->rule < LEC_UPD_NONE || u->rule > LEC_UPD_RSGD_LORENTZ) return LEC_E_ENUM;
     if (u->row_mode < LEC_ROWS_NONE || u->row_mode > LEC_ROWS_HYP_TANH) return LEC_E_ENUM;   // table modes only
     if (u->rule == LEC_UPD_RSGD_RETRACT && u->row_mode != LEC_ROWS_NONE) return LEC_E_ENUM;
+    if (u->rule == LEC_UPD_RSGD_LORENTZ && (u->geom != LEC_GEOM_LORENTZ || u->row_mode != LEC_ROWS_NONE || u->aux_out))
+        return LEC_E_ENUM;
     if (u->lambda_mode != 0 && u->lambda_mode != 1) return LEC_E_ENUM;
     if (u->aux_out && (u->geom < LEC_GEOM_EUC || u->geom > LEC_GEOM_OE)) return LEC_E_ENUM;
     if (!u->table || !u->grad_rows) return LEC_E_NULL;
@@ -302,7 +320,8 @@ int lec_cone_step(const lec_step_t* s, void* stream) {
     if (int e = check_update(&u)) return e;
     if (int e = check_exchange(&s->xchg, u.n, u.ld)) return e;
     if (!u.rows_out || !u.loss_acc) return LEC_E_NULL;
-    const bool poincare = s->geom == LEC_GEOM_POINCARE;
+    // Nickel & Kiela's embeddings (Poincare ball or Lorentz model): the softmax pair kernel on untransformed rows
+    const bool poincare = s->geom == LEC_GEOM_POINCARE || s->geom == LEC_GEOM_LORENTZ;
     if (poincare && (s->precision != LEC_PREC_F64CORE || u.row_mode != LEC_ROWS_NONE || s->w_pos || s->w_neg))
         return LEC_E_ENUM;
     struct PdlScope {   // the kernels of this step are launched as programmatic dependents of one another
@@ -318,8 +337,8 @@ int lec_cone_step(const lec_step_t* s, void* stream) {
     }
     if (s->ev_pairs_start) cudaEventRecord((cudaEvent_t)s->ev_pairs_start, st);
     const int e = poincare
-        ? lec_pairs_poincare(s->precision, u.rows_out, u.n, u.D, u.ld, s->pos_from, s->pos_to, s->neg_to, s->idx_bytes, s->B,
-                             s->N, s->E_pos, s->E_neg, u.loss_acc, u.grad_rows, u.grad_replicas, stream)
+        ? pairs_softmax(s->geom, s->precision, u.rows_out, u.n, u.D, u.ld, s->pos_from, s->pos_to, s->neg_to, s->idx_bytes,
+                        s->B, s->N, s->E_pos, s->E_neg, u.loss_acc, u.grad_rows, u.grad_replicas, stream)
         : lec_pairs_grouped(s->geom, s->precision, u.rows_out, u.aux_out, u.n, u.D, u.ld, s->pos_from, s->pos_to,
                             s->neg_to, s->neg_from, s->idx_bytes, s->B, s->N, s->w_pos, s->w_neg, u.K, s->alpha,
                             s->E_pos, s->E_neg, u.loss_acc, u.grad_rows, u.grad_replicas, stream);
@@ -364,8 +383,8 @@ int lec_featnet_wgrad(const float* features, int64_t n_pool, int F, const void* 
 int lec_score_topk_ex(int geom, int precision, const float* labels, int64_t L, const float* images, int64_t N, int D,
                       float K, const int32_t* level_start, const int32_t* level_stop, int n_levels, int k, float* scores,
                       int scores_layout, int32_t* topk_idx, float* topk_val, void* stream) {
-    // the Poincare distance has the fp32 SIMT kernel only (D <= 64)
-    const bool poincare = geom == LEC_GEOM_POINCARE;
+    // the Poincare and Lorentz distances have the fp32 SIMT kernel only (D <= 64)
+    const bool poincare = geom == LEC_GEOM_POINCARE || geom == LEC_GEOM_LORENTZ;
     if (poincare ? precision != LEC_PREC_F32 : pick_core(geom, precision) < 0) return LEC_E_ENUM;
     if (poincare && (D < 1 || D > 64)) return LEC_E_DIM;
     if (scores_layout != LEC_SCORES_IMAGE_MAJOR && scores_layout != LEC_SCORES_LABEL_MAJOR) return LEC_E_ENUM;

@@ -40,8 +40,9 @@ struct GroupArgs {
     unsigned long long* trace;   // LEC_STEP_TRACE builds only
 };
 
-// Poincare softmax loss (lec_pairs_poincare.cu): B positives with N negatives each, neg_to only
-struct PoincareArgs {
+// Nickel & Kiela's softmax loss on the Poincare or Lorentz distance (lec_pairs_softmax.cu): B positives with N
+// negatives each, neg_to only
+struct SoftmaxArgs {
     const float* rows; int ld;
     const void* pos_from; const void* pos_to; const void* neg_to; int idx_bytes;
     int64_t B; int N;
@@ -49,7 +50,8 @@ struct PoincareArgs {
     int64_t n_rows; unsigned* index_errors;
     int narrow_tail;
 };
-int launch_pairs_poincare(const PoincareArgs& a, cudaStream_t st);
+int launch_pairs_poincare(const SoftmaxArgs& a, cudaStream_t st);
+int launch_pairs_lorentz(const SoftmaxArgs& a, cudaStream_t st);
 
 // Gradient reduction of chunk q of a row.  The L2 executes a vector reduction as one fp32 add per element and its add
 // rate is what bounds the Euclidean kernels (cfg0, D = 2: 2.3 M REDG.128 per step = 340 G adds/s on a 92 KB target), so

@@ -1,5 +1,5 @@
 // Host side of the fast scoring kernel: builds the work-unit table (label segments x image groups) and
-// dispatches to the per-geometry translation units (lec_score_fast_{hyp,euc,oe,poincare}.cu).
+// dispatches to the per-geometry translation units (lec_score_fast_{hyp,euc,oe,poincare,lorentz}.cu).
 #include "lec_score_fast_impl.cuh"
 
 namespace lec {
@@ -8,6 +8,7 @@ int score_fast_hyp(FastArgs& a, cudaStream_t st);
 int score_fast_euc(FastArgs& a, cudaStream_t st);
 int score_fast_oe(FastArgs& a, cudaStream_t st);
 int score_fast_poincare(FastArgs& a, cudaStream_t st);
+int score_fast_lorentz(FastArgs& a, cudaStream_t st);
 
 bool score_fast_supported(int geom, int precision, int D, int64_t L) {
     (void)geom;
@@ -50,6 +51,7 @@ int score_fast_launch(int geom, const float* labels, int64_t L, const float* ima
         case LEC_GEOM_HYP: return score_fast_hyp(a, st);
         case LEC_GEOM_OE: return score_fast_oe(a, st);
         case LEC_GEOM_POINCARE: return score_fast_poincare(a, st);
+        case LEC_GEOM_LORENTZ: return score_fast_lorentz(a, st);
     }
     return LEC_E_ENUM;
 }

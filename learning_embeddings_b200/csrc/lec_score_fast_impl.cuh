@@ -19,6 +19,11 @@
 // tests/test_gpu_parity.py -- its error is below the reference's own fp32 error on the golden vectors).
 // Poincare distance (LEC_GEOM_POINCARE, Nickel & Kiela): s = max(A + B - 2p, 0), delta = 2s / ((1-A)(1-B)),
 //   E = log1p(delta + sqrt(delta (delta + 2))) = arcosh(1 + delta), 2/(1-A) and 1/(1-B) formed in fp64 per row.
+// Lorentz distance (LEC_GEOM_LORENTZ, Nickel & Kiela 2018; rows are spatial parts, x0 = sqrt(1 + A)): per row, in fp64
+//   and rounded once, x0 and e = x0 - 1 = A / (1 + x0);  per pair w = max(e_x y0 + (e_y - p), 0) = -<X,Y>_L - 1 and
+//   E = log1p(w + sqrt(w (w + 2))).  Every term of w is a product of per-row constants or p itself, so its error is
+//   |dw| <= (D + 8) 2^-24 (x0 y0 - 1 + |x||y|) (the dot product's gamma_D plus five roundings), small against w for
+//   points apart at any radius; E then carries that error through arcosh(1 + w) plus a few ulp (DESIGN.md).
 //
 // Top-k: a thread cannot afford a sorted insertion per score (lanes diverge), so candidates that beat the
 // current k-th best are appended, predicated and branch-free, to a small per-thread ring in shared
@@ -179,19 +184,26 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
         const float* s0 = a.images + (i0 < a.N ? i0 : 0) * (EVAL ? a.ld : (int64_t)D);
         const float* s1 = a.images + (i1 < a.N ? i1 : 0) * (EVAL ? a.ld : (int64_t)D);
         float b0 = 0.f, b1 = 0.f;
-        double e0 = 0.0, e1 = 0.0;  // Poincare: |y|^2 in fp64, as the labels' A
+        double e0 = 0.0, e1 = 0.0;  // Poincare, Lorentz: |y|^2 in fp64, as the labels' A
 #pragma unroll
         for (int d = 0; d < 4 * DQ; ++d) {
             const float v0 = (d < D) ? __ldg(s0 + d) : 0.f;
             const float v1 = (d < D) ? __ldg(s1 + d) : 0.f;
             b0 = fmaf(v0, v0, b0);
             b1 = fmaf(v1, v1, b1);
-            if (GEOM == LEC_GEOM_POINCARE) { e0 += (double)v0 * (double)v0; e1 += (double)v1 * (double)v1; }
+            if (GEOM == LEC_GEOM_POINCARE || GEOM == LEC_GEOM_LORENTZ) {
+                e0 += (double)v0 * (double)v0;
+                e1 += (double)v1 * (double)v1;
+            }
             y[j][d] = (GEOM == LEC_GEOM_OE) ? pack2(-v0, -v1) : pack2(v0, v1);
         }
         if (GEOM == LEC_GEOM_POINCARE) {  // B, 1 / (1 - B)
             B2[j] = pack2((float)e0, (float)e1);
             C2[j] = pack2((float)(1.0 / (1.0 - e0)), (float)(1.0 / (1.0 - e1)));
+        } else if (GEOM == LEC_GEOM_LORENTZ) {  // y0, y0 - 1
+            const double h0 = sqrt(1.0 + e0), h1 = sqrt(1.0 + e1);
+            B2[j] = pack2((float)h0, (float)h1);
+            C2[j] = pack2((float)(e0 / (1.0 + h0)), (float)(e1 / (1.0 + h1)));
         } else {
             B2[j] = pack2(b0, b1);
             C2[j] = pack2(-1.f - b0, -1.f - b1);
@@ -477,6 +489,18 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 E[2 * j] = log1pf(d0 + sqrtf(d0 * (d0 + 2.f)));
                 E[2 * j + 1] = log1pf(d1 + sqrtf(d1 * (d1 + 2.f)));
             }
+        } else if (GEOM == LEC_GEOM_LORENTZ) {
+            // cst = {x0 - 1};  w = (x0 - 1) y0 + ((y0 - 1) - p);  d = log1p(w + sqrt(w (w + 2)))
+            const u64 EX2 = pack2(cst.x, cst.x), M1 = pack2(-1.f, -1.f);
+#pragma unroll
+            for (int j = 0; j < NP; ++j) {
+                float w0, w1;
+                unpack2(ffma2(EX2, B2[j], ffma2(M1, acc[j], C2[j])), w0, w1);
+                w0 = max_nan(w0, 0.f);
+                w1 = max_nan(w1, 0.f);
+                E[2 * j] = log1pf(w0 + sqrtf(w0 * (w0 + 2.f)));
+                E[2 * j + 1] = log1pf(w1 + sqrtf(w1 * (w1 + 2.f)));
+            }
         } else {
             const float Af = cst.x, t0 = cst.y;
             const u64 A2 = pack2(Af, Af);
@@ -688,6 +712,8 @@ __global__ void __launch_bounds__(NT, MINB) score_fast_kernel(const FastArgs a) 
                 float4 c, c2 = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (GEOM == LEC_GEOM_POINCARE) {
                     c = make_float4((float)A, (float)(2.0 / (1.0 - A)), 0.f, 0.f);
+                } else if (GEOM == LEC_GEOM_LORENTZ) {
+                    c = make_float4((float)(A / (1.0 + sqrt(1.0 + A))), 0.f, 0.f, 0.f);  // x0 - 1
                 } else if (GEOM == LEC_GEOM_HYP) {
                     c = make_float4((float)A, (float)(1.0 + A), (float)(A * A), (float)(-x.t0));
                     const double sp = sin(x.t0);  // = the clamped asin argument
@@ -958,6 +984,7 @@ static int eval_launch(int geom, FastArgs& a, cudaStream_t st) {
         case LEC_GEOM_EUC: return eval_launch_geom<LEC_GEOM_EUC, P>(a, st);
         case LEC_GEOM_HYP: return eval_launch_geom<LEC_GEOM_HYP, P>(a, st);
         case LEC_GEOM_POINCARE: return eval_launch_geom<LEC_GEOM_POINCARE, P>(a, st);
+        case LEC_GEOM_LORENTZ: return eval_launch_geom<LEC_GEOM_LORENTZ, P>(a, st);
         default: return eval_launch_geom<LEC_GEOM_OE, P>(a, st);
     }
 }
@@ -968,7 +995,8 @@ template <typename T, typename F>
 static int eval_validate(const T* r, bool set, F&& more) {
     if (!r || !r->rows || !r->tin || !r->tout || !r->workspace || !set) return LEC_E_NULL;
     if (r->D < 1 || r->D > 64 || r->ld < r->D || (r->ld != r->D && r->ld % 4 != 0)) return LEC_E_DIM;
-    if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE && r->geom != LEC_GEOM_POINCARE)
+    if (r->geom != LEC_GEOM_EUC && r->geom != LEC_GEOM_HYP && r->geom != LEC_GEOM_OE && r->geom != LEC_GEOM_POINCARE &&
+        r->geom != LEC_GEOM_LORENTZ)
         return LEC_E_ENUM;
     if (r->n < 0 || r->n > 0x7fffffffLL || r->u_begin < 0 || r->u_end < r->u_begin || r->u_end > r->n) return LEC_E_SIZE;
     if (const int e = more()) return e;

@@ -10,7 +10,8 @@
 //      carry this step's tag and adds them in rank order (identical bits on every rank)
 //   3. vector-Jacobian product of the row transform (Embedder.forward): d loss / d table
 //   4. the update rule on the raw row: Riemannian SGD (order_embeddings_h.py:764-775), SGD with momentum or Adam
-//      (torch.optim, order_embeddings.py:563-565), Nickel & Kiela's rescaled step + retraction (Poincare embeddings), optionally preceded by the conformal rescale ((1-|w|)/2)^2 and followed
+//      (torch.optim, order_embeddings.py:563-565), Nickel & Kiela's rescaled step + retraction (Poincare embeddings) or
+//      exponential map on the hyperboloid (Lorentz embeddings), optionally preceded by the conformal rescale ((1-|w|)/2)^2 and followed
 //      by the shell projection of the joint hyperbolic trainer (oe_h.py:1765-1771)
 //   5. the row transform of the UPDATED row -- the Embedder.forward the next iteration starts with -- and its per-row
 //      aperture terms (aux), so the next pair kernel can start right away
@@ -332,6 +333,36 @@ __device__ __forceinline__ void row_rule(const UpdArgs& a, const int rule, const
 #pragma unroll
             for (int i = 0; i < 4 * V; ++i) e[i] *= sc;
         }
+    } else if (RULE_T == LEC_UPD_RSGD_LORENTZ) {
+        // Nickel & Kiela 2018: the exponential map on the hyperboloid along -lr times the Riemannian gradient, in the
+        // spatial chart (include/lec_b200.h): c = <x,g>, r = g + c x, nu = sqrt(|g|^2 + c^2), t = lr nu,
+        // x <- cosh(t) x - lr sinh(t)/t r.  Only this compile-time specialisation holds the rule (row_mode is NONE)
+        double xg = 0.0, gg = 0.0;
+#pragma unroll
+        for (int i = 0; i < 4 * V; ++i) {
+            xg = fma((double)e[i], (double)g[i], xg);
+            gg = fma((double)g[i], (double)g[i], gg);
+        }
+        xg = team_sum<TT, double>(xg);
+        gg = team_sum<TT, double>(gg);
+        const double nu = sqrt(fma(xg, xg, gg));
+        const double t = (double)a.lr * nu;
+        // cosh(t) and sinh(t) from one expm1: E = e^t = 1 + m, cosh = 1 + m^2 / 2E, sinh = m (m + 2) / 2E (no cancellation
+        // as t -> 0, where sinh(t) / t -> 1)
+        const double m = expm1(t), ie = 0.5 / (1.0 + m);
+        const double ch = fma(m * m, ie, 1.0);
+        const double sh = t > 0.0 ? (double)a.lr * (m * (m + 2.0) * ie / t) : (double)a.lr;   // lr sinh(t) / t
+        if (valid && a.grad_out) {
+            float r[4 * V];
+#pragma unroll
+            for (int i = 0; i < 4 * V; ++i) r[i] = (float)fma(xg, (double)e[i], (double)g[i]);
+            store_raw<TT, V>(a.grad_out + row * (int64_t)D, r, D, lane, a.tv);
+        }
+        if (nu > 0.0) {
+            const double ce = fma(-sh, xg, ch);   // x <- (cosh(t) - lr sinh(t)/t c) x - lr sinh(t)/t g
+#pragma unroll
+            for (int i = 0; i < 4 * V; ++i) e[i] = (float)fma(ce, (double)e[i], -sh * (double)g[i]);
+        }
     } else if (rule == LEC_UPD_RSGD) {
         // One pass gives the five row sums every later quantity is an algebraic function of (v = -lr gs g + 1e-15,
         // t = th v/|v| + 1e-6, the Moebius sums <w,t>, |t|^2 and the norm of the result), carried in fp64:
@@ -485,9 +516,14 @@ __device__ __forceinline__ void row_forward(const UpdArgs& a, const int row_mode
 }
 
 // RULE_T / MODE_T >= 0 fix the update rule / row transform at compile time (the hot combinations get their own, much
-// smaller, instruction stream); -1 reads them from the arguments.
+// smaller, instruction stream); -1 reads them from the arguments.  The Lorentz rule's fp64 expm1 does not fit the
+// register cap of LEC_UPD_MINBLOCKS (28 bytes of spill at 80 registers with four chunks per lane): it gets two blocks.
+template <int V, bool XCHG, int RULE_T>
+constexpr int kUpdMinBlocks =
+    (V <= 4 && !XCHG && RULE_T >= 0) ? (RULE_T == LEC_UPD_RSGD_LORENTZ ? 2 : LEC_UPD_MINBLOCKS) : 1;
+
 template <int TT, int V, bool XCHG, int RULE_T, int MODE_T>
-__global__ void __launch_bounds__(kThreads, (V <= 4 && !XCHG && RULE_T >= 0) ? LEC_UPD_MINBLOCKS : 1) update_rows_kernel(const UpdArgs a) {
+__global__ void __launch_bounds__(kThreads, (kUpdMinBlocks<V, XCHG, RULE_T>)) update_rows_kernel(const UpdArgs a) {
     const int rule = RULE_T >= 0 ? RULE_T : a.rule;
     const int row_mode = MODE_T >= 0 ? MODE_T : a.row_mode;
     pdl_launch_dependents();
@@ -862,6 +898,7 @@ static int two_shot_go(UpdArgs& a, cudaStream_t st) {
     a.rows_per_rank = (int64_t)a.tiles_per_rank * tpb;
     if (a.rule == LEC_UPD_RSGD && a.row_mode == LEC_ROWS_HYP_SHELL) return two_shot_go2<TT, V, LEC_UPD_RSGD, LEC_ROWS_HYP_SHELL>(a, st);
     if (a.rule == LEC_UPD_RSGD_RETRACT) return two_shot_go2<TT, V, LEC_UPD_RSGD_RETRACT, LEC_ROWS_NONE>(a, st);
+    if (a.rule == LEC_UPD_RSGD_LORENTZ) return two_shot_go2<TT, V, LEC_UPD_RSGD_LORENTZ, LEC_ROWS_NONE>(a, st);
     return two_shot_go2<TT, V, -1, -1>(a, st);
 }
 
@@ -880,6 +917,7 @@ static int update_go(const UpdArgs& a, cudaStream_t st) {
     // the two training configurations of the benchmarks get specialised kernels; everything else the generic one
     if (a.rule == LEC_UPD_RSGD && a.row_mode == LEC_ROWS_HYP_SHELL) return update_go2<TT, V, LEC_UPD_RSGD, LEC_ROWS_HYP_SHELL>(a, st);
     if (a.rule == LEC_UPD_RSGD_RETRACT) return update_go2<TT, V, LEC_UPD_RSGD_RETRACT, LEC_ROWS_NONE>(a, st);   // row_mode NONE (checked)
+    if (a.rule == LEC_UPD_RSGD_LORENTZ) return update_go2<TT, V, LEC_UPD_RSGD_LORENTZ, LEC_ROWS_NONE>(a, st);   // row_mode NONE (checked)
     if (a.rule == LEC_UPD_ADAM && a.row_mode == LEC_ROWS_EUC_SOFTCLIP && !a.hyp_rescale && !a.project_shell)
         return update_go2<TT, V, LEC_UPD_ADAM, LEC_ROWS_EUC_SOFTCLIP>(a, st);
     return update_go2<TT, V, -1, -1>(a, st);

@@ -44,7 +44,10 @@ def pack_index_block(pos_from, pos_to, neg_to, neg_from, pin=True, dtype=np.int3
     return blk.pin_memory() if (pin and torch.cuda.is_available()) else blk
 
 
-RULES = {"none": N.UPD_NONE, "rsgd": N.UPD_RSGD, "sgd": N.UPD_SGD, "adam": N.UPD_ADAM, "rsgd_retract": N.UPD_RSGD_RETRACT}
+RULES = {"none": N.UPD_NONE, "rsgd": N.UPD_RSGD, "sgd": N.UPD_SGD, "adam": N.UPD_ADAM, "rsgd_retract": N.UPD_RSGD_RETRACT,
+         "rsgd_lorentz": N.UPD_RSGD_LORENTZ}
+# Nickel & Kiela's embeddings: geometry -> (pair kernel, its update rule)
+_NK = {"poincare": ("lec_pairs_poincare", "rsgd_retract"), "lorentz": ("lec_pairs_lorentz", "rsgd_lorentz")}
 
 
 class ConeStep:
@@ -56,7 +59,12 @@ class ConeStep:
     geom="poincare": Nickel & Kiela's Poincare embeddings -- the softmax loss over each positive and its n_neg
     negatives (lec_pairs_poincare; neg_from is not read, E_neg is [max_groups, n_neg]) and update "rsgd_retract" (the
     default: w <- proj(w - lr (1 - |w|^2)^2 / 4 g)) or "none".  The table is used as it is (no row transform, no aux
-    terms); K, alpha and pair weights do not apply."""
+    terms); K, alpha and pair weights do not apply.
+
+    geom="lorentz": Nickel & Kiela's Lorentz-model embeddings, the same loss on the hyperboloid distance
+    (lec_pairs_lorentz; each table row is the spatial part x of the point (sqrt(1 + |x|^2), x)) and update "rsgd_lorentz"
+    (the default: the exponential map x <- cosh(t) x - lr sinh(t)/t (g + <x,g> x), t = lr sqrt(|g|^2 + <x,g>^2)) or
+    "none", with the same restrictions as "poincare"."""
 
     def __init__(self, table, geom, n_neg, max_groups, K=None, alpha=1.0, lr=1e-3, row_mode=None, update="auto",
                  precision=ops.PREC_F64CORE, process_group=None, replicas=None, comm="auto", momentum=0.0,
@@ -69,22 +77,24 @@ class ConeStep:
         self.n, self.D = table.shape
         self.ld = ops.padded_dim(self.D)
         self.n_neg = int(n_neg)
-        poincare = geom == "poincare"
-        self.K = {"euc": 3.0, "hyp": 0.1, "oe": 0.0, "poincare": 0.0}[geom] if K is None else float(K)
+        nk = geom in _NK   # the softmax loss of Nickel & Kiela: no aux terms, E_neg [max_groups, n_neg]
+        self.K = {"euc": 3.0, "hyp": 0.1, "oe": 0.0, "poincare": 0.0, "lorentz": 0.0}[geom] if K is None else float(K)
         self.alpha = float(alpha)
         self.lr = float(lr)
-        self.row_mode = {"euc": N.ROWS_EUC_SOFTCLIP, "hyp": N.ROWS_HYP_SHELL, "oe": N.ROWS_NONE, "poincare": N.ROWS_NONE}[geom] \
-            if row_mode is None else int(row_mode)
+        self.row_mode = {"euc": N.ROWS_EUC_SOFTCLIP, "hyp": N.ROWS_HYP_SHELL, "oe": N.ROWS_NONE, "poincare": N.ROWS_NONE,
+                         "lorentz": N.ROWS_NONE}[geom] if row_mode is None else int(row_mode)
         if update == "auto":
-            update = {"hyp": "rsgd", "poincare": "rsgd_retract"}.get(geom, "sgd")
+            update = _NK[geom][1] if nk else ("rsgd" if geom == "hyp" else "sgd")
         self.update = update
         if self.update not in RULES:
             raise N.LecError("unknown update rule %r" % (self.update,))
-        if poincare and (self.update not in ("rsgd_retract", "none") or self.row_mode != N.ROWS_NONE):
-            raise N.LecError("ConeStep(geom='poincare'): update must be 'rsgd_retract' or 'none' on untransformed rows, "
-                             "got update=%r, row_mode=%d" % (self.update, self.row_mode))
-        if self.update == "rsgd_retract" and not poincare:
+        if nk and (self.update not in (_NK[geom][1], "none") or self.row_mode != N.ROWS_NONE):
+            raise N.LecError("ConeStep(geom=%r): update must be %r or 'none' on untransformed rows, got update=%r, "
+                             "row_mode=%d" % (geom, _NK[geom][1], self.update, self.row_mode))
+        if self.update == "rsgd_retract" and geom != "poincare":
             raise N.LecError("update 'rsgd_retract' is the Poincare embeddings' rule (geom='poincare')")
+        if self.update == "rsgd_lorentz" and geom != "lorentz":
+            raise N.LecError("update 'rsgd_lorentz' is the Lorentz embeddings' rule (geom='lorentz')")
         self.momentum, self.betas, self.eps = float(momentum), (float(betas[0]), float(betas[1])), float(eps)
         self.hyp_rescale, self.project_shell = bool(hyp_rescale), bool(project_shell)
         self.r_in = float(inner_radius(self.K)) if geom == "hyp" else 0.0
@@ -94,11 +104,11 @@ class ConeStep:
         dev = table.device
         self.replicas = ops.default_replicas(self.n, self.ld) if replicas is None else int(replicas)
         self.rows = torch.empty((self.n, self.ld), device=dev, dtype=torch.float32)
-        self.aux = None if poincare else torch.empty((self.n, 4), device=dev, dtype=torch.float64)
+        self.aux = None if nk else torch.empty((self.n, 4), device=dev, dtype=torch.float64)
         self.grad_rows = torch.empty((self.replicas, self.n, self.ld), device=dev, dtype=torch.float32)
         self.grad_table = torch.empty((self.n, self.D), device=dev, dtype=torch.float32)
         self.E_pos = torch.empty(self.max_groups, device=dev, dtype=torch.float32)
-        self.E_neg = torch.empty((self.max_groups, (1 if poincare else 2) * self.n_neg), device=dev, dtype=torch.float32)
+        self.E_neg = torch.empty((self.max_groups, (1 if nk else 2) * self.n_neg), device=dev, dtype=torch.float32)
         # the pair kernel adds into loss_acc; the update kernel moves it to `loss` (this rank's loss of the latest step)
         self.loss = torch.zeros(1, device=dev, dtype=torch.float64)
         self._loss_ptr = self.loss.data_ptr()
@@ -203,13 +213,14 @@ class ConeStep:
         ev = self.kernel_events
         if ev is not None:
             ev[0].record()
-        if self.geom == "poincare":
+        if self.geom in _NK:
             if w_pos is not None or w_neg is not None:
-                raise N.LecError("the Poincare loss takes no pair weights")
-            N.check(lib.lec_pairs_poincare(
+                raise N.LecError("the softmax loss of geom=%r takes no pair weights" % (self.geom,))
+            name = _NK[self.geom][0]
+            N.check(getattr(lib, name)(
                 self.precision, N._p(self.rows), self.n, self.D, self.ld, N._p(pos_from), N._p(pos_to), N._p(neg_to),
                 pos_from.element_size(), B, self.n_neg, N._p(self.E_pos), N._p(self.E_neg), N._p(self.loss_acc),
-                N._p(self.grad_rows), self.replicas, st), "lec_pairs_poincare")
+                N._p(self.grad_rows), self.replicas, st), name)
         else:
             N.check(lib.lec_pairs_grouped(
                 N.GEOM[self.geom], self.precision, N._p(self.rows), N._p(self.aux), self.n, self.D, self.ld,

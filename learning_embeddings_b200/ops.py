@@ -183,41 +183,59 @@ def grouped_pair_loss(rows, aux, D, pos_from, pos_to, neg_to, neg_from, n_neg, g
                                  precision)
 
 
+def _softmax_loss_forward(ctx, entry, rows, D, pos_from, pos_to, neg_to):
+    """forward of PoincareLoss / LorentzLoss: one launch of `entry` (lec_pairs_poincare or lec_pairs_lorentz)."""
+    N.require_cuda(rows)
+    dev = rows.device
+    n, width = rows.shape
+    if width < D:
+        raise N.LecError("%s_loss: rows have %d columns, D = %d" % (entry[len("lec_pairs_"):], width, D))
+    ld = padded_dim(D)
+    padded = torch.zeros((n, ld), device=dev, dtype=torch.float32)
+    padded[:, :D] = rows.detach()[:, :D]
+    pos_from, pos_to, neg_to = _idx(pos_from, dev), _idx(pos_to, dev), _idx(neg_to, dev)
+    if not (pos_from.dtype == pos_to.dtype == neg_to.dtype):
+        pos_from, pos_to, neg_to = (t.to(torch.int64) for t in (pos_from, pos_to, neg_to))
+    B = int(pos_from.numel())
+    n_neg = int(neg_to.numel()) // max(B, 1)
+    E_pos = torch.empty(B, device=dev, dtype=torch.float32)
+    E_neg = torch.empty((B, n_neg), device=dev, dtype=torch.float32)
+    loss64 = torch.zeros(1, device=dev, dtype=torch.float64)
+    grad_rows = None
+    if ctx.needs_input_grad[0]:
+        grad_rows = torch.zeros((default_replicas(n, ld), n, ld), device=dev)
+    N.check(getattr(N.lib(), entry)(
+        PREC_F64CORE, N._p(padded), n, int(D), ld, N._p(pos_from), N._p(pos_to), N._p(neg_to),
+        pos_from.element_size(), B, n_neg, N._p(E_pos), N._p(E_neg), N._p(loss64), N._p(grad_rows),
+        1 if grad_rows is None else grad_rows.shape[0], N.stream_ptr(dev)), entry)
+    grad = None
+    if grad_rows is not None:
+        grad = torch.zeros_like(rows, dtype=torch.float32)
+        grad[:, :D] = reduce_replicas(grad_rows)[:, :D]
+    ctx.save_for_backward(grad)
+    ctx.mark_non_differentiable(E_pos, E_neg)
+    return loss64[0], E_pos, E_neg
+
+
 class PoincareLoss(torch.autograd.Function):
     """loss, E_pos[B], E_neg[B, N] of Nickel & Kiela's softmax loss on the Poincare distance (lec_pairs_poincare)."""
 
     @staticmethod
     def forward(ctx, rows, D, pos_from, pos_to, neg_to):
-        N.require_cuda(rows)
-        dev = rows.device
-        n, width = rows.shape
-        if width < D:
-            raise N.LecError("poincare_loss: rows have %d columns, D = %d" % (width, D))
-        ld = padded_dim(D)
-        padded = torch.zeros((n, ld), device=dev, dtype=torch.float32)
-        padded[:, :D] = rows.detach()[:, :D]
-        pos_from, pos_to, neg_to = _idx(pos_from, dev), _idx(pos_to, dev), _idx(neg_to, dev)
-        if not (pos_from.dtype == pos_to.dtype == neg_to.dtype):
-            pos_from, pos_to, neg_to = (t.to(torch.int64) for t in (pos_from, pos_to, neg_to))
-        B = int(pos_from.numel())
-        n_neg = int(neg_to.numel()) // max(B, 1)
-        E_pos = torch.empty(B, device=dev, dtype=torch.float32)
-        E_neg = torch.empty((B, n_neg), device=dev, dtype=torch.float32)
-        loss64 = torch.zeros(1, device=dev, dtype=torch.float64)
-        grad_rows = None
-        if ctx.needs_input_grad[0]:
-            grad_rows = torch.zeros((default_replicas(n, ld), n, ld), device=dev)
-        N.check(N.lib().lec_pairs_poincare(
-            PREC_F64CORE, N._p(padded), n, int(D), ld, N._p(pos_from), N._p(pos_to), N._p(neg_to),
-            pos_from.element_size(), B, n_neg, N._p(E_pos), N._p(E_neg), N._p(loss64), N._p(grad_rows),
-            1 if grad_rows is None else grad_rows.shape[0], N.stream_ptr(dev)), "lec_pairs_poincare")
-        grad = None
-        if grad_rows is not None:
-            grad = torch.zeros_like(rows, dtype=torch.float32)
-            grad[:, :D] = reduce_replicas(grad_rows)[:, :D]
-        ctx.save_for_backward(grad)
-        ctx.mark_non_differentiable(E_pos, E_neg)
-        return loss64[0], E_pos, E_neg
+        return _softmax_loss_forward(ctx, "lec_pairs_poincare", rows, D, pos_from, pos_to, neg_to)
+
+    @staticmethod
+    def backward(ctx, g_loss, _gp, _gn):
+        (grad,) = ctx.saved_tensors
+        return (grad * g_loss.float(),) + (None,) * 4
+
+
+class LorentzLoss(torch.autograd.Function):
+    """loss, E_pos[B], E_neg[B, N] of Nickel & Kiela's softmax loss on the Lorentz distance (lec_pairs_lorentz)."""
+
+    @staticmethod
+    def forward(ctx, rows, D, pos_from, pos_to, neg_to):
+        return _softmax_loss_forward(ctx, "lec_pairs_lorentz", rows, D, pos_from, pos_to, neg_to)
 
     @staticmethod
     def backward(ctx, g_loss, _gp, _gn):
@@ -231,6 +249,28 @@ def poincare_loss(rows, D, pos_from, pos_to, neg_to):
     pos_to [B] and neg_to [B, N] are row ids.  Returns (loss as a float64 scalar, E_pos [B], E_neg [B, N]); the loss is
     differentiable with respect to rows (fp64 pair algebra, gradient computed in the forward launch)."""
     return PoincareLoss.apply(rows, D, pos_from, pos_to, neg_to)
+
+
+def lorentz_loss(rows, D, pos_from, pos_to, neg_to):
+    """The loss of poincare_loss on the Lorentz distance d = arcosh(1 + w), w = -<X,Y>_L - 1 (Nickel & Kiela 2018).
+    rows [n, >= D] are the spatial parts x of hyperboloid points (sqrt(1 + |x|^2), x) (fp32 CUDA, any values); the
+    other arguments and the results are those of poincare_loss."""
+    return LorentzLoss.apply(rows, D, pos_from, pos_to, neg_to)
+
+
+def lorentz_to_ball(W):
+    """Lorentz rows (spatial parts x) -> Poincare-ball points x / (1 + sqrt(1 + |x|^2)); the distance is kept
+    (d_L(x, y) = d_P of the images).  fp64 inside, fp32 out, on W's device."""
+    x = W.detach().to(torch.float64)
+    x0 = torch.sqrt(1.0 + (x * x).sum(-1, keepdim=True))
+    return (x / (1.0 + x0)).to(torch.float32)
+
+
+def ball_to_lorentz(P):
+    """Poincare-ball points p (|p| < 1) -> Lorentz rows 2p / (1 - |p|^2), the inverse of lorentz_to_ball.  fp64 inside,
+    fp32 out, on P's device."""
+    p = P.detach().to(torch.float64)
+    return (2.0 * p / (1.0 - (p * p).sum(-1, keepdim=True))).to(torch.float32)
 
 
 def pairs_flat_raw(geom, rows, aux, D, from_idx, to_idx, K, alpha, w=None, is_pos=None, grad_rows=None, loss_out=None,
